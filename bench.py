@@ -18,7 +18,9 @@ stereo_net(L, fl, fr, 'l').  Prints ONE JSON line on rank 0 (contract in the tas
   roofline / kernels    per-kernel event timings with an L2 flush before every launch; DRAM traffic from the committed ncu capture
   cpu_baseline          the reference modules (oracle/_ref) — or the oracle port where they are absent — on the host cores
 
-Every timed region runs for at least --min-seconds (default 2 s) AND at least the requested number of steps.
+Every timed region runs exactly its number of steps (--steps for `value` and `e2e`); with --min-seconds S > 0 a region instead
+grows until it lasts at least S seconds.  --dump-outputs DIR writes the outputs of the last step of the `value` region as
+DIR/<name>.npy (float32, '/' in a name becomes '_'): seeded inputs and weights make two builds comparable output for output.
 """
 import argparse
 import json
@@ -216,9 +218,18 @@ def time_kernel(fn, iters, flush, stream):
   return sum(ts) / len(ts), ts[len(ts) // 2]
 
 
+def dump_outputs(outputs, out_dir):
+  """outputs: the dict of device tensors the forward returns (KITTI size: ~4.5 MB in all) -> out_dir/<name>.npy, float32."""
+  import numpy as np
+  os.makedirs(out_dir, exist_ok=True)
+  for name, t in outputs.items():
+    np.save(os.path.join(out_dir, name.replace("/", "_") + ".npy"), t.detach().float().cpu().numpy())
+
+
 class Timer:
-  """Timed regions of at least `min_steps` steps AND `min_seconds`: a probe of a few steps sizes the region (the step count is
-  agreed over the ranks), then the region runs between a barrier + synchronize on both sides, CUDA events, max over ranks."""
+  """Timed regions of exactly `min_steps` steps, or with `min_seconds` > 0 of at least `min_steps` steps AND `min_seconds`: a probe of
+  a few steps sizes the region (the step count is agreed over the ranks).  The region runs between a barrier + synchronize on both
+  sides, CUDA events, max over ranks."""
 
   def __init__(self, dev, world, min_seconds):
     self.dev, self.world, self.min_seconds = dev, world, min_seconds
@@ -243,17 +254,19 @@ class Timer:
       step()
     if finish:
       finish()
-    self.barrier()
-    a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    a.record(self.stream)
-    for _ in range(5):
-      step()
-    if finish:
-      finish()
-    b.record(self.stream)
-    torch.cuda.synchronize()
-    probe_ms = self._max(a.elapsed_time(b) / 5)
-    steps = int(min(max_steps, max(min_steps, self.min_seconds * 1e3 / max(probe_ms, 1e-3) + 1)))
+    steps = min_steps
+    if self.min_seconds > 0:
+      self.barrier()
+      a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+      a.record(self.stream)
+      for _ in range(5):
+        step()
+      if finish:
+        finish()
+      b.record(self.stream)
+      torch.cuda.synchronize()
+      probe_ms = self._max(a.elapsed_time(b) / 5)
+      steps = int(min(max_steps, max(min_steps, self.min_seconds * 1e3 / max(probe_ms, 1e-3) + 1)))
     for attempt in range(3):
       self.barrier()
       a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -313,7 +326,13 @@ def gpu_arm(args):
     sampler.start()
 
   # ---- configs[1], device-resident throughput: inputs already in HBM, graph replays
-  steps_dev, ms_dev = tm.run(lambda: engine.run_static(shape, dev), args.steps, args.warmup)
+  last = {}
+
+  def step_dev():
+    last["out"] = engine.run_static(shape, dev)[0]
+  steps_dev, ms_dev = tm.run(step_dev, args.steps, args.warmup)
+  if args.dump_outputs and rank == 0:
+    dump_outputs(last["out"], args.dump_outputs)          # what the last timed step returned
 
   # ---- configs[1], end to end through the public engine API: pinned host images in, host disparity out, every step
   # (a) streaming API: H2D of frame i+1 / forward of frame i / D2H of frame i-1 overlap (throughput = the headline e2e);
@@ -567,7 +586,10 @@ def main():
   ap.add_argument("--steps", type=int, default=50)
   ap.add_argument("--warmup", type=int, default=5)
   ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
-  ap.add_argument("--min-seconds", type=float, default=2.0, help="every timed region runs at least this long (and at least --steps steps)")
+  ap.add_argument("--min-seconds", type=float, default=0.0,
+                  help="> 0: every timed region runs at least this long (and at least its number of steps); 0: exactly its number of steps")
+  ap.add_argument("--dump-outputs", metavar="DIR",
+                  help="after the timed steps, write the outputs of the last step of the `value` region as DIR/<name>.npy (float32)")
   ap.add_argument("--no-graph", action="store_true")
   ap.add_argument("--skip-cpu", action="store_true")
   ap.add_argument("--cpu-steps", type=int, default=12)
@@ -580,9 +602,11 @@ def main():
 
   rank = int(os.environ.get("RANK", "0"))
   if args.impl == "reference":
+    if args.dump_outputs:
+      ap.error("--dump-outputs applies to --impl b200 (the reference arm runs other seeded weights)")
     if rank != 0:
       return
-    c = cpu_reference(steps=args.steps, warmup=min(args.warmup, 2), budget_s=150.0)
+    c = cpu_reference(steps=args.steps, warmup=min(args.warmup, 2), budget_s=float("inf"))
     line = {"impl": "reference", "metric": METRIC, "value": c["value"], "unit": "pairs/s", "n_gpus": args.gpus, "steps": c["steps"],
             "warmup": min(args.warmup, 2), "ms_per_step": c["ms_per_step"], "higher_is_better": True, "scaling": "weak",
             "vs_baseline": None, "dtype": "f32", "data": "synthetic", "config": {"workload": WORKLOAD},

@@ -15,7 +15,8 @@ def _line(name):
 
 def test_round2_line_entries():
   """Round-2 additions: every timed region >= 2 s, >= 50 adaptation steps, the other BASELINE.json configurations as keyed entries,
-  the CPU baseline measured on the reference's own modules."""
+  the CPU baseline measured on the reference's own modules.  A committed r2 line is taken with `bench.py --min-seconds 2`
+  (profiles/README.md); with the default (0) every region runs exactly its number of steps."""
   import pytest
   if not os.path.exists(os.path.join(ROOT, "profiles", "r2_bench_n1.json")):
     pytest.skip("no round-2 bench line committed yet")

@@ -26,6 +26,28 @@ def test_vendored_files_are_the_reference_byte_for_byte(tmp_path):
     assert hashlib.sha256(open(os.path.join(make_ref.DST, rel), "rb").read()).hexdigest() == digest, rel
 
 
+def test_make_ref_recipe_copies_byte_for_byte_and_records_digests(tmp_path, monkeypatch):
+  """The recipe itself, on every host: make() on a stand-in checkout of seeded bytes (CR/LF and non-UTF-8 included) in tmp_path
+  copies each module byte for byte and writes both copies' SHA-256 into MANIFEST.json; a missing checkout writes nothing.  It
+  says nothing about the reference's contents (the test above does, where a reference checkout exists)."""
+  import random
+  sys.path.insert(0, os.path.join(ROOT, "oracle"))
+  import make_ref
+  ref, dst = tmp_path / "reference", tmp_path / "_ref"
+  monkeypatch.setattr(make_ref, "DST", str(dst))
+  assert not make_ref.make(str(tmp_path / "absent")) and not dst.exists()
+  rng = random.Random(0)
+  for rel in make_ref.FILES:
+    (ref / rel).parent.mkdir(parents=True, exist_ok=True)
+    (ref / rel).write_bytes(bytes(rng.randrange(256) for _ in range(rng.randrange(1000, 5000))) + b"\r\n\x00\xff")
+  assert make_ref.make(str(ref))
+  manifest = json.load(open(dst / "MANIFEST.json"))
+  assert sorted(manifest) == sorted(make_ref.FILES)
+  for rel, digest in manifest.items():
+    assert hashlib.sha256((ref / rel).read_bytes()).hexdigest() == digest, rel
+    assert hashlib.sha256((dst / rel).read_bytes()).hexdigest() == digest, rel
+
+
 @pytest.mark.skipif(not os.path.exists(os.path.join(ROOT, "oracle", "_ref", "adaptive_stereo", "models", "stereo_net.py")),
                     reason="oracle/_ref has not been made on this host")
 def test_reference_forward_equals_oracle_port():

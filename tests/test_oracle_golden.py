@@ -31,6 +31,23 @@ def summ(t):
   return np.array([t.sum().item(), t.abs().sum().item(), (t * t).sum().sqrt().item()])
 
 
+ADAM_LR = 5e-5
+
+
+def zero_grad_bias(n):
+  """Biases whose gradient in a train-mode step is mathematically zero: a convolution feeding a batch-statistics BatchNorm
+  (convbn / convbn_3d: '<...>.0.0.bias', the BN removes the batch mean), conv3d_alone.bias (under the softmax: shift invariant) and
+  conv_alone.bias (cancels in L - R).  What is computed for them is rounding noise whose value depends on the host CPU's
+  summation order (its oneDNN kernels), and Adam's first step turns that noise into a move of up to lr per element.  They are
+  held to zero up to rounding and to that lr bound instead of to the stored noise (as in tests/test_gpu_backward.py)."""
+  return n.endswith(".0.0.bias") or n in ("conv3d_alone.bias", "conv_alone.bias")
+
+
+def zero_up_to_rounding(grads, tag, n):
+  """|gradient| <= 1e-3 x the largest gradient entry of the same convolution's weight (the noise measures below 5e-5 x)."""
+  return grads[(tag, n)].abs().max().item() <= 1e-3 * grads[(tag, n[:-len("bias")] + "weight")].abs().max().item()
+
+
 @pytest.mark.parametrize("name", list(CASES))
 def test_inputs_regenerate(name):
   """Seeded weights/inputs must regenerate exactly, otherwise the fixtures do not apply."""
@@ -74,7 +91,7 @@ def test_adapt_step_matches_reference(name):
   ssd = O.make_stereo_state(seed=22, sharpen=cfg["sharpen"] * TRAIN_SHARPEN_RATIO)
   fsd, ssd = O.clone_state(fsd, True), O.clone_state(ssd, True)
   adam = {}
-  loss, outputs, grads = O.adapt_step(fsd, ssd, left, right, cfg["k"], adam, lr=5e-5, input_scale=cfg["s"])
+  loss, outputs, grads = O.adapt_step(fsd, ssd, left, right, cfg["k"], adam, lr=ADAM_LR, input_scale=cfg["s"])
   assert abs(loss.item() - float(g["train/loss"])) < 2e-6
   for key, v in outputs.items():
     np.testing.assert_allclose(v.detach().numpy(), g["train/" + key], rtol=0, atol=2e-3, err_msg=key)
@@ -87,7 +104,10 @@ def test_adapt_step_matches_reference(name):
       _, tag, n = key.split("/", 2)
       got = grads[(tag, n)] / (coef if tag == "s" else 1.0)
       ref = g[key]
-      assert abs(summ(got)[2] - ref[2]) <= 2e-3 * ref[2] + 1e-7, (key, summ(got), ref)
+      if zero_grad_bias(n):
+        assert zero_up_to_rounding(grads, tag, n), key
+      else:
+        assert abs(summ(got)[2] - ref[2]) <= 2e-3 * ref[2] + 1e-7, (key, summ(got), ref)
       checked += 1
     elif key.startswith("grad_none/"):
       _, tag, n = key.split("/", 2)
@@ -97,17 +117,23 @@ def test_adapt_step_matches_reference(name):
       got = (grads[(tag, n)] / (coef if tag == "s" else 1.0)).numpy()
       ref = g[key]
       scale = np.abs(ref).max() + 1e-12
-      assert np.abs(got - ref).max() <= 2e-3 * scale + 1e-7, key
+      assert zero_up_to_rounding(grads, tag, n) if zero_grad_bias(n) else np.abs(got - ref).max() <= 2e-3 * scale + 1e-7, key
   assert checked > 40
   for key in g.files:
     if key.startswith("post/"):
       _, tag, n = key.split("/", 2)
       sd = ssd if tag == "s" else fsd
-      np.testing.assert_allclose(sd[n].detach().numpy(), g[key], rtol=1e-4, atol=1e-6, err_msg=key)
+      if zero_grad_bias(n):
+        np.testing.assert_allclose(sd[n].detach().numpy(), g[key], rtol=0, atol=2 * ADAM_LR, err_msg=key)
+      else:
+        np.testing.assert_allclose(sd[n].detach().numpy(), g[key], rtol=1e-4, atol=1e-6, err_msg=key)
     elif key.startswith("post_sum/"):
       _, tag, n = key.split("/", 2)
       sd = ssd if tag == "s" else fsd
-      np.testing.assert_allclose(summ(sd[n]), g[key], rtol=1e-5, atol=1e-7, err_msg=key)
+      if zero_grad_bias(n):
+        np.testing.assert_allclose(summ(sd[n]), g[key], rtol=0, atol=2 * ADAM_LR * sd[n].numel(), err_msg=key)
+      else:
+        np.testing.assert_allclose(summ(sd[n]), g[key], rtol=1e-5, atol=1e-7, err_msg=key)
 
 
 # ---- round 2: the reference's own test / timing configurations at full size (oracle/gen_golden.py BIG_CASES) and rows f3 / f4
@@ -180,7 +206,7 @@ def test_rows_f3_f4_oracle_matches_reference():
   f2, s2 = O.clone_state(fsd, True), O.clone_state(ssd, True)
   l, r, _ = O.make_stereo_pair(1, H, W, seed=1000, max_disp_px=40.0)
   rl, rr, rgt = O.make_stereo_pair(1, H, W, seed=1001, max_disp_px=40.0)
-  loss, _, grads = O.adapt_step(f2, s2, l, r, k, {}, lr=5e-5, replay=(rl, rr, rgt))
+  loss, _, grads = O.adapt_step(f2, s2, l, r, k, {}, lr=ADAM_LR, replay=(rl, rr, rgt))
   assert abs(loss.item() - float(g["er/loss"])) < 2e-5
   for key in g.files:
     if key.startswith("er/post/") and ("running_" in key or "num_batches" in key):
@@ -188,4 +214,9 @@ def test_rows_f3_f4_oracle_matches_reference():
       np.testing.assert_allclose((s2 if tag == "s" else f2)[n].detach().numpy(), g[key], rtol=1e-4, atol=1e-6, err_msg=key)
     elif key.startswith("er/post_sum/"):
       _, _, tag, n = key.split("/", 3)
-      np.testing.assert_allclose(summ((s2 if tag == "s" else f2)[n]), g[key], rtol=1e-5, atol=1e-7, err_msg=key)
+      t = (s2 if tag == "s" else f2)[n]
+      if zero_grad_bias(n):
+        assert zero_up_to_rounding(grads, tag, n), key
+        np.testing.assert_allclose(summ(t), g[key], rtol=0, atol=2 * ADAM_LR * t.numel(), err_msg=key)
+      else:
+        np.testing.assert_allclose(summ(t), g[key], rtol=1e-5, atol=1e-7, err_msg=key)
