@@ -1,4 +1,7 @@
-"""Build libsnb200.so (sm_100a only) in-tree with nvcc.  Usage: python build.py [--force]"""
+"""Build libsnb200.so (sm_100a only) in-tree with nvcc.  Usage: python build.py [--force] [--example [OUT]]
+
+--example also builds examples/stereonet_infer.cpp (the torch-free whole-model host, include/snb200.h) with the same nvcc flags,
+linked against libsnb200.so; OUT defaults to build/stereonet_infer next to this file."""
 import glob
 import os
 import subprocess
@@ -52,5 +55,24 @@ def build(force=False, verbose=False):
   return OUT
 
 
+EXAMPLE = os.path.join(HERE, "..", "examples", "stereonet_infer.cpp")
+
+
+def build_example(out=None):
+  """examples/stereonet_infer.cpp -> `out` (default build/stereonet_infer), linked against (and with an rpath to) libsnb200.so."""
+  lib = build()
+  out = out or os.path.join(HERE, "build", "stereonet_infer")
+  os.makedirs(os.path.dirname(os.path.abspath(out)), exist_ok=True)
+  libdir = os.path.dirname(lib)
+  cmd = ([NVCC] + FLAGS + ["-I", os.path.join(HERE, "..", "include"), EXAMPLE, "-o", out,
+                           "-L" + libdir, "-lsnb200", "-Xlinker", "-rpath=" + libdir])
+  subprocess.check_call(cmd)
+  return out
+
+
 if __name__ == "__main__":
   print(build(force="--force" in sys.argv, verbose="-v" in sys.argv))
+  if "--example" in sys.argv:
+    i = sys.argv.index("--example")
+    nxt = sys.argv[i + 1] if i + 1 < len(sys.argv) and not sys.argv[i + 1].startswith("-") else None
+    print(build_example(nxt))

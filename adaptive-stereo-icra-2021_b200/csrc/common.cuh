@@ -53,6 +53,12 @@ __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;\
 
 static inline int snb_ceil_div(long long a, long long b) { return (int)((a + b - 1) / b); }
 
+// ---- one entry of the batched weight preparation with the table passed by value (conv_c32_tc.cu; used by the whole-model
+// prepare of model.cu).  cfg = nwin | mode << 8 | kind << 16 | a << 24 | b << 28 as in snb_prep_conv_weights_tc_batch, plus
+// kind 3 (C4 image), 4 (eval-mode BatchNorm fold: aux = {beta, running_mean, running_var}) and 5 (copy of `count` floats).
+struct snb_prep_item { const float* src; const float* aux[3]; float* out; int cfg; int count; };
+int snb_prep_param_launch(const snb_prep_item* items, int n, void* stream);
+
 // ---- small device helpers
 __device__ __forceinline__ float lrelu(float v) { return v > 0.f ? v : SNB_LRELU_SLOPE * v; }
 

@@ -421,14 +421,26 @@ __global__ void weight_scale_kernel(const float* __restrict__ w, int numel, floa
   pdl_wait();            // no early trigger: see WEIGHT-IMAGE WRITERS below
   weight_scale_block(w, numel, slot);
 }
+// Entry kinds of the batched preparation (config bits 16..23, see snb_prep_conv_weights_tc_batch):
+//   0, 1, 2  the tensor-core images described in snb200.h;
+//   3        the C4 image of the refinement's input layer from its [32][4][3][3] weight: the "ws" image of the [32][32][3][3] tensor
+//            W'[co][kw*4 + ch][kh][0] = w[co][ch][kh][kw] (zero elsewhere), nwin = 3, mode = SNB_CONV_WS (what ops.refine_in_weights_ws
+//            builds with torch layout ops);
+//   4        eval-mode BatchNorm fold: src = gamma, aux = {beta, running_mean, running_var}; out[0:32] = scale, out[64:96] = shift;
+//   5        plain copy of `count` floats.
+// Kinds 4 and 5 need the aux pointers / count of snb_prep_item, i.e. the by-value table of snb_prep_param_launch.
+__device__ __forceinline__ int weight_numel_of(int kind, int nwin) {
+  return kind == 0 ? 1024 * nwin * 3 : (kind == 3 ? 32 * 4 * 9 : 1024 * 25);
+}
+__device__ __forceinline__ void weight_scale_entry(const float* w, float* out, int cfg) {
+  if (((cfg >> 8) & (SNB_CONV_F16 | SNB_CONV_WS)) == 0) return;
+  const int nwin = cfg & 0xff, kind = (cfg >> 16) & 0xff;
+  weight_scale_block(w, weight_numel_of(kind, nwin), out + scale_slot_of(cfg >> 8, nwin));
+}
 __global__ void weight_scale_batch_kernel(const long long* __restrict__ table) {
   pdl_wait();            // no early trigger: see WEIGHT-IMAGE WRITERS below
   const long long* e = table + 4 * blockIdx.x;
-  const int cfg = (int)e[2];
-  if (((cfg >> 8) & (SNB_CONV_F16 | SNB_CONV_WS)) == 0) return;
-  const int nwin = cfg & 0xff, kind = (cfg >> 16) & 0xff;
-  weight_scale_block(reinterpret_cast<const float*>(e[0]), kind == 0 ? 1024 * nwin * 3 : 1024 * 25,
-                     reinterpret_cast<float*>(e[1]) + scale_slot_of(cfg >> 8, nwin));
+  weight_scale_entry(reinterpret_cast<const float*>(e[0]), reinterpret_cast<float*>(e[1]), (int)e[2]);
 }
 
 // w [32 cout][32 cin][kd*kh*kw taps] -> per (kd,kh) window: B_hi[n = kw*32 + cout][k = cin] then B_lo, each in the
@@ -459,20 +471,31 @@ __global__ void prep_weights_tc_kernel(const float* __restrict__ w, float* __res
   }
 }
 
-// Batched variant: blockIdx.y picks a table entry {w, out, config, 0} (see snb_prep_conv_weights_tc_batch in snb200.h).
-__global__ void prep_weights_tc_batch_kernel(const long long* __restrict__ table) {
-  pdl_wait();            // no early trigger: see WEIGHT-IMAGE WRITERS below
-  const long long* e = table + 4 * blockIdx.y;
-  const float* __restrict__ w = reinterpret_cast<const float*>(e[0]);
-  float* __restrict__ out = reinterpret_cast<float*>(e[1]);
-  const int cfg = (int)e[2];
+// One table entry (kinds above) over the flat index range first, first + step, ...
+__device__ __forceinline__ void prep_entry(const float* __restrict__ w, const float* const* aux, float* __restrict__ out, int cfg,
+                                           int count, int first, int step) {
   const int nwin = cfg & 0xff, mode = (cfg >> 8) & 0xf, kind = (cfg >> 16) & 0xff, pa = (cfg >> 24) & 0xf, pb = (cfg >> 28) & 0xf;
+  if (kind == 4) {
+    if (aux == nullptr) return;
+    // bit for bit what autograd.fused.bn_fold computes with torch ops, one rounding per op and no FMA contraction:
+    // scale = gamma * rsqrt(var + eps), shift = beta - mean * scale
+    for (int c = first; c < 32; c += step) {
+      const float sc = __fmul_rn(w[c], rsqrtf(__fadd_rn(aux[2][c], 1e-5f)));
+      out[c] = sc;
+      out[64 + c] = __fsub_rn(aux[0][c], __fmul_rn(aux[1][c], sc));
+    }
+    return;
+  }
+  if (kind == 5) {
+    for (int i = first; i < count; i += step) out[i] = w[i];
+    return;
+  }
   const bool f16 = ((cfg >> 8) & SNB_CONV_F16) != 0, ws = ((cfg >> 8) & SNB_CONV_WS) != 0;
   const float scale = (f16 || ws) ? 1.f / out[scale_slot_of(cfg >> 8, nwin)] : 1.f;
-  if (kind == 2) { store_p4_images(w, out, scale, blockIdx.x * blockDim.x + threadIdx.x, gridDim.x * blockDim.x); return; }
+  if (kind == 2) { store_p4_images(w, out, scale, first, step); return; }
   const int taps = nwin * 3;
   const int total = nwin * 96 * 32;
-  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < total; i += gridDim.x * blockDim.x) {
+  for (int i = first; i < total; i += step) {
     const int k = i & 31;
     const int n = (i >> 5) % 96;
     const int win = i / (96 * 32);
@@ -483,6 +506,8 @@ __global__ void prep_weights_tc_batch_kernel(const long long* __restrict__ table
     float v;
     if (kind == 0) {
       v = w[((size_t)oc * 32 + ic) * taps + tap];
+    } else if (kind == 3) {
+      v = (tap % 3 == 0 && ic < 12) ? w[((oc * 4 + (ic & 3)) * 3 + tap / 3) * 3 + (ic >> 2)] : 0.f;
     } else {
       const int y5 = 2 * (tap / 3) + pa, x5 = 2 * (tap % 3) + pb;
       v = (y5 < 5 && x5 < 5) ? w[((size_t)oc * 32 + ic) * 25 + y5 * 5 + x5] : 0.f;
@@ -494,6 +519,32 @@ __global__ void prep_weights_tc_batch_kernel(const long long* __restrict__ table
     out[o] = hi;
     out[o + B_BYTES / 4] = v - hi;
   }
+}
+
+// Batched variant: blockIdx.y picks a table entry {w, out, config, 0} (see snb_prep_conv_weights_tc_batch in snb200.h).
+__global__ void prep_weights_tc_batch_kernel(const long long* __restrict__ table) {
+  pdl_wait();            // no early trigger: see WEIGHT-IMAGE WRITERS below
+  const long long* e = table + 4 * blockIdx.y;
+  prep_entry(reinterpret_cast<const float*>(e[0]), nullptr, reinterpret_cast<float*>(e[1]), (int)e[2], 0,
+             blockIdx.x * blockDim.x + threadIdx.x, gridDim.x * blockDim.x);
+}
+
+// The same pair of kernels over a table passed BY VALUE (snb_prep_param_launch): no table upload, so a caller's preparation is one
+// capturable launch pair with no host-to-device copy.  PREP_PARAM_MAX entries keep the parameter block under 4 KB.
+constexpr int PREP_PARAM_MAX = 80;
+struct PrepParamTable { snb_prep_item it[PREP_PARAM_MAX]; int n; };
+static_assert(sizeof(PrepParamTable) <= 4096, "kernel parameter block");
+
+__global__ void weight_scale_param_kernel(const __grid_constant__ PrepParamTable t) {
+  pdl_wait();            // no early trigger: see WEIGHT-IMAGE WRITERS below
+  const snb_prep_item& e = t.it[blockIdx.x];
+  weight_scale_entry(e.src, e.out, e.cfg);
+}
+
+__global__ void prep_weights_param_kernel(const __grid_constant__ PrepParamTable t) {
+  pdl_wait();            // no early trigger: see WEIGHT-IMAGE WRITERS below
+  const snb_prep_item& e = t.it[blockIdx.y];
+  prep_entry(e.src, e.aux, e.out, e.cfg, e.count, blockIdx.x * blockDim.x + threadIdx.x, gridDim.x * blockDim.x);
 }
 
 }  // namespace tc
@@ -558,6 +609,20 @@ extern "C" int snb_prep_conv_weights_tc_batch(const long long* table, int n, voi
   SNB_LAUNCH_CHECK("weight_scale_batch_kernel");
   snb_launch(tc::prep_weights_tc_batch_kernel, dim3(36, n), 256, 0, stream, table);
   SNB_LAUNCH_CHECK("prep_weights_tc_batch_kernel");
+  return 0;
+}
+
+int snb_prep_param_launch(const snb_prep_item* items, int n, void* stream) {
+  SNB_REQUIRE(items && n > 0, "snb_prep_param_launch: bad args");
+  for (int base = 0; base < n; base += tc::PREP_PARAM_MAX) {
+    tc::PrepParamTable t;
+    t.n = n - base < tc::PREP_PARAM_MAX ? n - base : tc::PREP_PARAM_MAX;
+    for (int i = 0; i < t.n; ++i) t.it[i] = items[base + i];
+    snb_launch(tc::weight_scale_param_kernel, t.n, 256, 0, stream, t);      // no-op blocks for the kinds without a scale
+    SNB_LAUNCH_CHECK("weight_scale_param_kernel");
+    snb_launch(tc::prep_weights_param_kernel, dim3(36, t.n), 256, 0, stream, t);
+    SNB_LAUNCH_CHECK("prep_weights_param_kernel");
+  }
   return 0;
 }
 

@@ -87,6 +87,12 @@ SIGNATURES = {
   "snb_conv_c4_ws": (_I, [_P, _P, _P, _I, _I, _I, _EP, _P]),
   "snb_bn_running_update": (_I, [_P, _P, _LL, _P, _P, _P, _F, _F, _P]),
   "snb_prep_conv5x5s2_weights_ws": (_I, [_P, _P, _P]),
+  "snb_stereonet_num_params": (_I, [_I]),
+  "snb_stereonet_weights_bytes": (_LL, [_I]),
+  "snb_stereonet_weights_piece": (_I, [_I, _I, C.POINTER(_LL), C.POINTER(_LL)]),
+  "snb_stereonet_prepare": (_I, [_P, _I, _P, _P]),
+  "snb_stereonet_workspace_bytes": (_LL, [_I, _I, _I, _I, _I, _I]),
+  "snb_stereonet_forward": (_I, [_P, _I, _I, _I, _P, _I, _I, _I, _P, _P, _P, _P, _P, _P]),
 }
 
 _lib = None

@@ -150,7 +150,8 @@ SNB_API int snb_conv_weights_tc_floats(int kd);
  * config = nwin | mode << 8 | kind << 16 | a << 24 | b << 28.  kind 0: a [32][32][nwin*3] weight as in
  * snb_prep_conv_weights_tc (nwin = 3 kd).  kind 1: the polyphase 3x3 sub-kernel (a, b) of a [32][32][5][5] stride-2 weight,
  * sub[i][j] = w[2i + a][2j + b] (zero outside the 5x5 support), nwin = 3 (csrc/phase.cu).  kind 2: the image set of
- * snb_conv5x5s2_c32_ws from a [32][32][5][5] weight (nwin = 10, mode = SNB_CONV_WS). */
+ * snb_conv5x5s2_c32_ws from a [32][32][5][5] weight (nwin = 10, mode = SNB_CONV_WS).  kind 3: the snb_conv_c4_ws image from the
+ * refinement input layer's [32][4][3][3] weight (nwin = 3, mode = SNB_CONV_WS). */
 SNB_API int snb_prep_conv_weights_tc_batch(const long long* table, int n, void* stream);
 
 /* Polyphase helpers for the stride-2 5x5 32->32 layers (stereo_net.py:64-70): the convolution is the sum of four stride-1
@@ -316,6 +317,41 @@ SNB_API int snb_adam_clip_step(const long long* chunk_table, int nchunks, const 
                        float* step, long long n_total, long long n_clip, float max_norm, float grad_scale, double lr,
                        double beta1, double beta2, double eps, void* workspace, void* stream);
 SNB_API int snb_adam_clip_workspace_bytes(void);
+
+/* ---------------------------------------------------------------------------------------------------------------
+ * Whole-model inference (eval mode): StereoNet's feature extractor on both images plus the stereo head, as the Python
+ * engine runs it (stereonet_b200.runtime.StereoEngine), for hosts without Python or torch (csrc/model.cu).  Bit-identical
+ * to that path.  Train mode, backward and adaptation are not part of this interface.
+ *
+ * params: HOST array of DEVICE pointers (contiguous fp32), one per tensor the eval forward reads, in the reference's state_dict
+ * order: feature_net (downsample.i.{weight,bias}, residual_blocks.i.conv1.0.0.{weight,bias},
+ * residual_blocks.i.conv1.0.1.{weight,bias,running_mean,running_var}, conv_alone.{weight,bias}), then stereo_net (filter.i.0.0 /
+ * .0.1 as above, conv3d_alone, edge_aware_refinements.0.conv2d_feature.0.0 / .0.1, .residual_astrous_blocks.i.conv1.0.0 / .0.1,
+ * .conv2d_out).  BasicBlock.conv2.* and num_batches_tracked are not read.  2k + 108 tensors (stereonet_b200.native.param_names).
+ * --------------------------------------------------------------------------------------------------------------- */
+SNB_API int snb_stereonet_num_params(int k);
+/* Size of the prepared-weights buffer.  It holds everything the forward reads (tensor-core weight images, folded eval-mode
+ * BatchNorm, copies of the raw biases and small weights), so the caller may free or change `params` after prepare. */
+SNB_API long long snb_stereonet_weights_bytes(int k);
+/* Where the tensor params[index] left its derived piece inside `weights`: byte offset and size (size 0 for the running statistics,
+ * which only feed the fold).  Weight images of the 32->32 convolutions, the ten-image sets of downsample[1:], the refinement input
+ * layer's four-channel image; BatchNorm weight -> folded scale [32], BatchNorm bias -> folded shift [32]; everything else a copy. */
+SNB_API int snb_stereonet_weights_piece(int k, int index, long long* offset, long long* bytes);
+/* Derive `weights` (device, 256-byte aligned, snb_stereonet_weights_bytes(k) bytes) from params: one launch pair, no host-to-device
+ * copy (capturable).  Call again after a parameter changed. */
+SNB_API int snb_stereonet_prepare(const float* const* params, int k, void* weights, void* stream);
+/* Workspace of snb_stereonet_forward in bytes, or -1 (snb_last_error) for arguments the forward rejects. */
+SNB_API long long snb_stereonet_workspace_bytes(int k, int input_scale, int maxdisp, int B, int H, int W);
+/* images [2][B][3][H][W] fp32 NCHW (left batch, then right batch).  With D' = (maxdisp + 1) / 2^(input_scale + k) (in [1, 32])
+ * and h, w the size after k stride-2 layers (h = ceil(H / 2^k) step by step):
+ *   disp   [B,H,W]     = pred_disp_l/{input_scale}
+ *   coarse [B,H,W]     = pred_disp_l/{input_scale + k}, or NULL
+ *   cost   [B,D',h,w]  = cost_volume_l/{input_scale + k}, or NULL
+ *   fcs    [B,h,w]     = feature-contrast score of that cost volume (needs cost and D' > 2), or NULL.
+ * weights and workspace (snb_stereonet_workspace_bytes) 256-byte aligned, the other buffers 16-byte aligned.  Nothing outside
+ * these extents is written.  Independent calls may run concurrently on separate streams with separate workspaces and outputs. */
+SNB_API int snb_stereonet_forward(const void* weights, int k, int input_scale, int maxdisp, const float* images, int B, int H, int W,
+                          void* workspace, float* disp, float* coarse, float* cost, float* fcs, void* stream);
 
 #ifdef __cplusplus
 }
