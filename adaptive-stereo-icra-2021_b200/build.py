@@ -1,7 +1,8 @@
 """Build libsnb200.so (sm_100a only) in-tree with nvcc.  Usage: python build.py [--force] [--example [OUT]]
 
 --example also builds examples/stereonet_infer.cpp (the torch-free whole-model host, include/snb200.h) with the same nvcc flags,
-linked against libsnb200.so; OUT defaults to build/stereonet_infer next to this file."""
+linked against libsnb200.so; OUT defaults to build/stereonet_infer next to this file.  examples/stereonet_adapt.cpp (the torch-free
+adaptation host) is built next to it as stereonet_adapt."""
 import glob
 import os
 import subprocess
@@ -55,16 +56,16 @@ def build(force=False, verbose=False):
   return OUT
 
 
-EXAMPLE = os.path.join(HERE, "..", "examples", "stereonet_infer.cpp")
+EXAMPLES = os.path.join(HERE, "..", "examples")
 
 
-def build_example(out=None):
-  """examples/stereonet_infer.cpp -> `out` (default build/stereonet_infer), linked against (and with an rpath to) libsnb200.so."""
+def build_example(out=None, name="stereonet_infer"):
+  """examples/<name>.cpp -> `out` (default build/<name>), linked against (and with an rpath to) libsnb200.so."""
   lib = build()
-  out = out or os.path.join(HERE, "build", "stereonet_infer")
+  out = out or os.path.join(HERE, "build", name)
   os.makedirs(os.path.dirname(os.path.abspath(out)), exist_ok=True)
   libdir = os.path.dirname(lib)
-  cmd = ([NVCC] + FLAGS + ["-I", os.path.join(HERE, "..", "include"), EXAMPLE, "-o", out,
+  cmd = ([NVCC] + FLAGS + ["-I", os.path.join(HERE, "..", "include"), os.path.join(EXAMPLES, name + ".cpp"), "-o", out,
                            "-L" + libdir, "-lsnb200", "-Xlinker", "-rpath=" + libdir])
   subprocess.check_call(cmd)
   return out
@@ -76,3 +77,4 @@ if __name__ == "__main__":
     i = sys.argv.index("--example")
     nxt = sys.argv[i + 1] if i + 1 < len(sys.argv) and not sys.argv[i + 1].startswith("-") else None
     print(build_example(nxt))
+    print(build_example(os.path.join(os.path.dirname(os.path.abspath(nxt)), "stereonet_adapt") if nxt else None, "stereonet_adapt"))

@@ -55,7 +55,8 @@ static inline int snb_ceil_div(long long a, long long b) { return (int)((a + b -
 
 // ---- one entry of the batched weight preparation with the table passed by value (conv_c32_tc.cu; used by the whole-model
 // prepare of model.cu).  cfg = nwin | mode << 8 | kind << 16 | a << 24 | b << 28 as in snb_prep_conv_weights_tc_batch, plus
-// kind 3 (C4 image), 4 (eval-mode BatchNorm fold: aux = {beta, running_mean, running_var}) and 5 (copy of `count` floats).
+// kind 3 (C4 image), 4 (eval-mode BatchNorm fold: aux = {beta, running_mean, running_var}), 5 (copy of `count` floats) and 6
+// (flipped disparity-channel taps of the refinement input layer, used by the adaptation step's backward).
 struct snb_prep_item { const float* src; const float* aux[3]; float* out; int cfg; int count; };
 int snb_prep_param_launch(const snb_prep_item* items, int n, void* stream);
 

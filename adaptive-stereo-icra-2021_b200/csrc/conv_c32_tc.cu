@@ -427,7 +427,9 @@ __global__ void weight_scale_kernel(const float* __restrict__ w, int numel, floa
 //            W'[co][kw*4 + ch][kh][0] = w[co][ch][kh][kw] (zero elsewhere), nwin = 3, mode = SNB_CONV_WS (what ops.refine_in_weights_ws
 //            builds with torch layout ops);
 //   4        eval-mode BatchNorm fold: src = gamma, aux = {beta, running_mean, running_var}; out[0:32] = scale, out[64:96] = shift;
-//   5        plain copy of `count` floats.
+//   5        plain copy of `count` floats;
+//   6        the data-gradient taps of the refinement input layer's disparity channel from its [32][4][3][3] weight:
+//            out[c*9 + t] = w[c][0][8 - t] (RefineHead.backward's flipped [32][9] weight).
 // Kinds 4 and 5 need the aux pointers / count of snb_prep_item, i.e. the by-value table of snb_prep_param_launch.
 __device__ __forceinline__ int weight_numel_of(int kind, int nwin) {
   return kind == 0 ? 1024 * nwin * 3 : (kind == 3 ? 32 * 4 * 9 : 1024 * 25);
@@ -488,6 +490,10 @@ __device__ __forceinline__ void prep_entry(const float* __restrict__ w, const fl
   }
   if (kind == 5) {
     for (int i = first; i < count; i += step) out[i] = w[i];
+    return;
+  }
+  if (kind == 6) {
+    for (int i = first; i < 32 * 9; i += step) out[i] = w[(i / 9) * 36 + 8 - i % 9];
     return;
   }
   const bool f16 = ((cfg >> 8) & SNB_CONV_F16) != 0, ws = ((cfg >> 8) & SNB_CONV_WS) != 0;

@@ -93,6 +93,13 @@ SIGNATURES = {
   "snb_stereonet_prepare": (_I, [_P, _I, _P, _P]),
   "snb_stereonet_workspace_bytes": (_LL, [_I, _I, _I, _I, _I, _I]),
   "snb_stereonet_forward": (_I, [_P, _I, _I, _I, _P, _I, _I, _I, _P, _P, _P, _P, _P, _P]),
+  "snb_stereonet_adapt_state_bytes": (_LL, [_I]),
+  "snb_stereonet_adapt_state_piece": (_I, [_I, _I, C.POINTER(_LL), C.POINTER(_LL)]),
+  "snb_stereonet_adapt_grad_slot": (_I, [_I, _I, C.POINTER(_LL), C.POINTER(_LL)]),
+  "snb_stereonet_adapt_init": (_I, [_P, _I, _P, _P]),
+  "snb_stereonet_adapt_workspace_bytes": (_LL, [_I, _I, _I, _I, _I, _I]),
+  "snb_stereonet_adapt_forward": (_I, [_P, _P, _I, _I, _I, _P, _I, _I, _I, _P, _P, _P, _P, _P, _P, _P]),
+  "snb_stereonet_adapt_update": (_I, [_P, _I, _I, _I, _I, _I, _I, _P, _P, _F, _D, _D, _D, _D, _P]),
 }
 
 _lib = None

@@ -15,7 +15,8 @@
  *    reference's callers pass them; single-channel maps are [B,H,W] / [B,D,H,W].
  *  - return value 0 on success, non-zero on failure; snb_last_error() returns a thread-local message.
  *  - re-entrant: no global mutable state (the reference may be driven from a ROS callback thread,
- *    ros/stereo_depth_node.py:113).
+ *    ros/stereo_depth_node.py:113), except the mutex-guarded host-side record of the arguments of the last
+ *    snb_stereonet_adapt_forward per workspace, which snb_stereonet_adapt_update checks its own against.
  */
 #ifndef SNB200_H_
 #define SNB200_H_
@@ -321,7 +322,7 @@ SNB_API int snb_adam_clip_workspace_bytes(void);
 /* ---------------------------------------------------------------------------------------------------------------
  * Whole-model inference (eval mode): StereoNet's feature extractor on both images plus the stereo head, as the Python
  * engine runs it (stereonet_b200.runtime.StereoEngine), for hosts without Python or torch (csrc/model.cu).  Bit-identical
- * to that path.  Train mode, backward and adaptation are not part of this interface.
+ * to that path.  The adaptation step (train mode, backward, clip + Adam) is the snb_stereonet_adapt_* group further below.
  *
  * params: HOST array of DEVICE pointers (contiguous fp32), one per tensor the eval forward reads, in the reference's state_dict
  * order: feature_net (downsample.i.{weight,bias}, residual_blocks.i.conv1.0.0.{weight,bias},
@@ -352,6 +353,52 @@ SNB_API long long snb_stereonet_workspace_bytes(int k, int input_scale, int maxd
  * these extents is written.  Independent calls may run concurrently on separate streams with separate workspaces and outputs. */
 SNB_API int snb_stereonet_forward(const void* weights, int k, int input_scale, int maxdisp, const float* images, int B, int H, int W,
                           void* workspace, float* disp, float* coarse, float* cost, float* fcs, void* stream);
+
+/* ---------------------------------------------------------------------------------------------------------------
+ * Whole-model online adaptation, single pass (adapt.py:304-396 without experience replay: the update of the NONE / NONSTOP / VS
+ * modes), for hosts without Python or torch (csrc/adapt.cu).  Bit-identical to the Python step
+ * AdaptStepper(f, s, make_optimizer(f, s, lr, fused=True), two_streams=False).  Two calls per frame, because the host decides
+ * from the loss whether to update (adapt.py:381: not when the frame was just added to the OVS):
+ *   snb_stereonet_adapt_forward  train-mode forward of both images (adapt.py:72-73; BatchNorm running statistics and
+ *                                num_batches_tracked move, left pass, right pass, stereo head, refinement), Monodepth loss
+ *                                (adapt.py:78-86, :328-337) and feature-contrast score (adapt.py:352-353);
+ *   snb_stereonet_adapt_update   backward from what the forward saved in `workspace` (adapt.py:390), every gradient into the flat
+ *                                bucket, clip_grad_norm_ on stereo_net (adapt.py:391-392) and Adam (adapt.py:393).
+ * `params` is the list of snb_stereonet_prepare (2k + 108 tensors, stereonet_b200.native.param_names); Adam rewrites the parameters
+ * in place and the forward rewrites running_mean / running_var.  `state` (snb_stereonet_adapt_state_bytes, 256-byte aligned) holds
+ * the gradient bucket, Adam's moments and step, and the weight images the forward derives from the parameters.  The bucket is laid
+ * out as optim.FusedAdamClip's: used parameters only, stereo_net first, then feature_net, in named_parameters() order, without
+ * BasicBlock.conv2.*; so FusedAdamClip state (and adam.pth through its state_dict) converts by copying the flat buffers.
+ * Contract: update follows a forward with the same workspace and arguments, and the parameter values do not change in between.
+ * The library records each forward's arguments on the host, keyed by the workspace address, and the update rejects by name, before
+ * any launch, a workspace no forward has run on and any k, input_scale, maxdisp, B, H, W, state or params[i] other than its
+ * forward's (this holds under graph capture too, where each call runs on the host once).  The parameter addresses are those given
+ * to snb_stereonet_adapt_init.  No allocation, no synchronisation, no host-to-device copy: both calls are
+ * CUDA-graph capturable.
+ * --------------------------------------------------------------------------------------------------------------- */
+SNB_API long long snb_stereonet_adapt_state_bytes(int k);
+/* what: 0 flat_grad [n] fp32, 1 exp_avg [n], 2 exp_avg_sq [n], 3 step [1] fp32 (Adam's t); byte offset and size inside `state`. */
+SNB_API int snb_stereonet_adapt_state_piece(int k, int what, long long* offset, long long* bytes);
+/* Element offset and count of params[index]'s slot in the bucket (count 0: a running statistic, no slot). */
+SNB_API int snb_stereonet_adapt_grad_slot(int k, int index, long long* offset, long long* count);
+/* Zero the bucket, the moments and step, and write Adam's per-chunk table from the parameter addresses (two launches). */
+SNB_API int snb_stereonet_adapt_init(float* const* params, int k, void* state, void* stream);
+/* Workspace of the forward / update pair in bytes (the activations the update reads and both calls' scratch), or -1. */
+SNB_API long long snb_stereonet_adapt_workspace_bytes(int k, int input_scale, int maxdisp, int B, int H, int W);
+/* images [2][B][3][H][W] as in snb_stereonet_forward.  bn_counters: the 17 num_batches_tracked int64 counters in module order
+ * (feature_net's six BasicBlocks, stereo_net's four filters, the refinement's input layer and six blocks), or NULL.
+ *   loss     [1 + B]  [0] = the batch's masked photometric mean (adapt.py:83), [1 + b] = sample b's
+ *   disp     [B,H,W]  pred_disp_l/{input_scale}, or NULL
+ *   fcs      [B,h,w]  feature-contrast score of the coarse cost volume, or NULL
+ *   fcs_mean [1]      its mean (fixed-order double sum), or NULL.  fcs and fcs_mean need more than 2 coarse disparity levels.
+ * state, workspace 256-byte aligned; images, disp, fcs 16-byte aligned. */
+SNB_API int snb_stereonet_adapt_forward(float* const* params, long long* const* bn_counters, int k, int input_scale, int maxdisp,
+                                const float* images, int B, int H, int W, void* state, void* workspace, float* loss, float* disp,
+                                float* fcs, float* fcs_mean, void* stream);
+/* Gradients of loss[0] into the bucket (slots of parameters without a gradient: zeros), then snb_adam_clip_step with
+ * max_norm (<= 0: no clipping), lr, beta1, beta2, eps (torch.optim.Adam defaults 0.9, 0.999, 1e-8). */
+SNB_API int snb_stereonet_adapt_update(float* const* params, int k, int input_scale, int maxdisp, int B, int H, int W, void* state,
+                               void* workspace, float max_norm, double lr, double beta1, double beta2, double eps, void* stream);
 
 #ifdef __cplusplus
 }
