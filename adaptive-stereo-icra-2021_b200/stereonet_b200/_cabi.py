@@ -100,6 +100,9 @@ SIGNATURES = {
   "snb_stereonet_adapt_workspace_bytes": (_LL, [_I, _I, _I, _I, _I, _I]),
   "snb_stereonet_adapt_forward": (_I, [_P, _P, _I, _I, _I, _P, _I, _I, _I, _P, _P, _P, _P, _P, _P, _P]),
   "snb_stereonet_adapt_update": (_I, [_P, _I, _I, _I, _I, _I, _I, _P, _P, _F, _D, _D, _D, _D, _P]),
+  "snb_stereonet_adapt_replay_workspace_bytes": (_LL, [_I, _I, _I, _I, _I, _I, _I]),
+  "snb_stereonet_adapt_forward_replay": (_I, [_P, _P, _I, _I, _I, _P, _I, _I, _I, _P, _P, _I, _F, _P, _P, _P, _P, _P, _P, _P, _P]),
+  "snb_stereonet_adapt_update_replay": (_I, [_P, _I, _I, _I, _I, _I, _I, _I, _P, _P, _F, _D, _D, _D, _D, _P]),
 }
 
 _lib = None

@@ -1,7 +1,8 @@
 """Bridge to the whole-model C-ABI (snb_stereonet_*, include/snb200.h): the parameter list a C or C++ host hands to
 snb_stereonet_prepare, and a weights file such a host can read without Python or torch (examples/stereonet_infer.cpp).
-Python users keep runtime.StereoEngine; this module adds no inference wrapper.  NativeAdapt drives the single-pass adaptation
-step (snb_stereonet_adapt_*) on a pair of modules and converts its Adam state to and from optim.FusedAdamClip.
+Python users keep runtime.StereoEngine; this module adds no inference wrapper.  NativeAdapt drives the adaptation step
+(snb_stereonet_adapt_*: single pass, or with an experience-replay pass) on a pair of modules and converts its Adam state to and from
+optim.FusedAdamClip.
 
 Parameter order (param_names): the tensors the eval forward reads, in the reference's state_dict order, feature_net first and
 stereo_net second; BasicBlock.conv2.* (constructed, never run) and num_batches_tracked are left out.  2k + 108 tensors.
@@ -97,12 +98,17 @@ class NativeAdapt:
     self._ws, self._last = {}, None
     _cabi.check(lib.snb_stereonet_adapt_init(self.params, self.k, self.state.data_ptr(), _stream(dev)), "snb_stereonet_adapt_init")
 
-  def workspace(self, B, H, W):
-    key = (B, H, W)
+  def workspace(self, B, H, W, RB=0):
+    """The workspace of the forward / update pair at this shape (RB >= 1: with a replay pass of batch RB), allocated once."""
+    key = (B, H, W, RB)
     if key not in self._ws:
-      nb = _cabi.lib().snb_stereonet_adapt_workspace_bytes(self.k, self.s.input_scale, self.s.maxdisp, B, H, W)
+      lib = _cabi.lib()
+      if RB:
+        nb = lib.snb_stereonet_adapt_replay_workspace_bytes(self.k, self.s.input_scale, self.s.maxdisp, B, H, W, RB)
+      else:
+        nb = lib.snb_stereonet_adapt_workspace_bytes(self.k, self.s.input_scale, self.s.maxdisp, B, H, W)
       if nb < 0:
-        raise RuntimeError(_cabi.lib().snb_last_error().decode())
+        raise RuntimeError(lib.snb_last_error().decode())
       self._ws[key] = torch.empty((nb,), device=self.state.device, dtype=torch.uint8)
     return self._ws[key]
 
@@ -113,8 +119,10 @@ class NativeAdapt:
                          f"(got {type(t).__name__} {tuple(getattr(t, 'shape', ()))} {getattr(t, 'dtype', None)} "
                          f"{getattr(t, 'device', None)})")
 
-  def forward(self, images, loss, disp=None, fcs=None, fcs_mean=None):
-    """images [2,B,3,H,W]; writes loss [1 + B] and the optional outputs disp [B,H,W], fcs [B,h,w], fcs_mean [1]."""
+  def forward(self, images, loss, disp=None, fcs=None, fcs_mean=None, replay=None, loss_replay=None, er_weight=0.05):
+    """images [2,B,3,H,W]; writes loss [1 + B] and the optional outputs disp [B,H,W], fcs [B,h,w], fcs_mean [1].
+    replay = (replay_images [2,RB,3,H,W], gt [RB,H,W] or [RB,1,H,W]) adds the experience-replay pass: loss_replay [2] receives
+    {Khamis term, loss[0] + er_weight * Khamis term}, and update() then differentiates both passes."""
     if not (isinstance(images, torch.Tensor) and images.dim() == 5 and images.shape[0] == 2 and images.shape[2] == 3):
       raise RuntimeError(f"stereonet_b200: `images` must be [2,B,3,H,W], got {tuple(getattr(images, 'shape', ()))}")
     _, B, _, H, W = images.shape
@@ -127,21 +135,41 @@ class NativeAdapt:
       if t is not None:
         self._check(t, name, shape)
     p = lambda t: None if t is None else t.data_ptr()
-    _cabi.check(_cabi.lib().snb_stereonet_adapt_forward(
-        self.params, self.counters, self.k, self.s.input_scale, self.s.maxdisp, images.data_ptr(), B, H, W, self.state.data_ptr(),
-        self.workspace(B, H, W).data_ptr(), loss.data_ptr(), p(disp), p(fcs), p(fcs_mean), _stream(images.device)),
-        "snb_stereonet_adapt_forward")
-    self._last = (B, H, W)
+    lib, st = _cabi.lib(), _stream(images.device)
+    if replay is None:
+      _cabi.check(lib.snb_stereonet_adapt_forward(
+          self.params, self.counters, self.k, self.s.input_scale, self.s.maxdisp, images.data_ptr(), B, H, W, self.state.data_ptr(),
+          self.workspace(B, H, W).data_ptr(), loss.data_ptr(), p(disp), p(fcs), p(fcs_mean), st), "snb_stereonet_adapt_forward")
+      self._last = (B, H, W, 0)
+      return
+    rimages, gt = replay
+    if not (isinstance(rimages, torch.Tensor) and rimages.dim() == 5 and rimages.shape[0] == 2 and rimages.shape[1] >= 1
+            and tuple(rimages.shape[2:]) == (3, H, W)):
+      raise RuntimeError(f"stereonet_b200: `replay_images` must be [2,RB,3,{H},{W}], got {tuple(getattr(rimages, 'shape', ()))}")
+    RB = rimages.shape[1]
+    self._check(rimages, "replay_images", rimages.shape)
+    self._check(gt, "replay_gt", (RB, 1, H, W) if isinstance(gt, torch.Tensor) and gt.dim() == 4 else (RB, H, W))
+    self._check(loss_replay, "loss_replay", (2,))
+    _cabi.check(lib.snb_stereonet_adapt_forward_replay(
+        self.params, self.counters, self.k, self.s.input_scale, self.s.maxdisp, images.data_ptr(), B, H, W, rimages.data_ptr(),
+        gt.data_ptr(), RB, float(er_weight), self.state.data_ptr(), self.workspace(B, H, W, RB).data_ptr(), loss.data_ptr(),
+        loss_replay.data_ptr(), p(disp), p(fcs), p(fcs_mean), st), "snb_stereonet_adapt_forward_replay")
+    self._last = (B, H, W, RB)
 
   def update(self):
-    """Backward of the last forward, clip + Adam."""
+    """Backward of the last forward (both passes after a replay forward), clip + Adam."""
     if self._last is None:
       raise RuntimeError("stereonet_b200: NativeAdapt.update() needs a forward() first")
-    B, H, W = self._last
-    _cabi.check(_cabi.lib().snb_stereonet_adapt_update(
-        self.params, self.k, self.s.input_scale, self.s.maxdisp, B, H, W, self.state.data_ptr(), self.workspace(B, H, W).data_ptr(),
-        float(self.clip_norm) if self.clip_norm else 0.0, self.lr, self.betas[0], self.betas[1], self.eps,
-        _stream(self.state.device)), "snb_stereonet_adapt_update")
+    B, H, W, RB = self._last
+    lib = _cabi.lib()
+    common = (self.state.data_ptr(), self.workspace(B, H, W, RB).data_ptr(), float(self.clip_norm) if self.clip_norm else 0.0,
+              self.lr, self.betas[0], self.betas[1], self.eps, _stream(self.state.device))
+    if RB:
+      _cabi.check(lib.snb_stereonet_adapt_update_replay(self.params, self.k, self.s.input_scale, self.s.maxdisp, B, H, W, RB, *common),
+                  "snb_stereonet_adapt_update_replay")
+    else:
+      _cabi.check(lib.snb_stereonet_adapt_update(self.params, self.k, self.s.input_scale, self.s.maxdisp, B, H, W, *common),
+                  "snb_stereonet_adapt_update")
 
   def to_fused(self, opt):
     """Copy the moments and step into an optim.FusedAdamClip of the same modules (same flat layout)."""

@@ -356,7 +356,7 @@ SNB_API int snb_stereonet_forward(const void* weights, int k, int input_scale, i
 
 /* ---------------------------------------------------------------------------------------------------------------
  * Whole-model online adaptation, single pass (adapt.py:304-396 without experience replay: the update of the NONE / NONSTOP / VS
- * modes), for hosts without Python or torch (csrc/adapt.cu).  Bit-identical to the Python step
+ * modes; the replay step of ER and VS+ER follows below), for hosts without Python or torch (csrc/adapt.cu).  Bit-identical to the Python step
  * AdaptStepper(f, s, make_optimizer(f, s, lr, fused=True), two_streams=False).  Two calls per frame, because the host decides
  * from the loss whether to update (adapt.py:381: not when the frame was just added to the OVS):
  *   snb_stereonet_adapt_forward  train-mode forward of both images (adapt.py:72-73; BatchNorm running statistics and
@@ -399,6 +399,33 @@ SNB_API int snb_stereonet_adapt_forward(float* const* params, long long* const* 
  * max_norm (<= 0: no clipping), lr, beta1, beta2, eps (torch.optim.Adam defaults 0.9, 0.999, 1e-8). */
 SNB_API int snb_stereonet_adapt_update(float* const* params, int k, int input_scale, int maxdisp, int B, int H, int W, void* state,
                                void* workspace, float max_norm, double lr, double beta1, double beta2, double eps, void* stream);
+
+/* ---------------------------------------------------------------------------------------------------------------
+ * The same step with experience replay (adapt.py:339-349, :381-394: the update of the ER and VS+ER modes), bit-identical to
+ * AdaptStepper(f, s, make_optimizer(f, s, lr, fused=True), two_streams=False).step(left, right, replay=(rl, rr, gt)).  The forward
+ * runs a second train-mode pass on a stored sample with ground truth and adds er_weight times its Khamis robust loss
+ * (loss_functions.py:6-15) to the photometric loss of the stream frame; the update differentiates both passes and applies clip +
+ * Adam once.  Choosing the sample (reservoir, OVS) stays with the host.  Same contract as the single pass above; the update must be
+ * snb_stereonet_adapt_update_replay with the forward's RB (and a plain forward's update snb_stereonet_adapt_update), which the
+ * update checks by name before any launch.  Both calls are CUDA-graph capturable.
+ * --------------------------------------------------------------------------------------------------------------- */
+/* Workspace of the replay forward / update pair in bytes (RB >= 1), or -1. */
+SNB_API long long snb_stereonet_adapt_replay_workspace_bytes(int k, int input_scale, int maxdisp, int B, int H, int W, int RB);
+/* As snb_stereonet_adapt_forward (images, loss, disp, fcs, fcs_mean keep their meaning: the stream frame's), then the replay pass,
+ * whose BatchNorm running statistics and counters move after the stream pass's (per frame: feature_net's counters + 4, stereo_net's
+ * + 2), and the Khamis loss of its disparity:
+ *   replay_images  [2][RB][3][H][W]  the stored pair (same H and W as the frame, RB >= 1), 16-byte aligned
+ *   replay_gt      [RB][H][W]        its ground-truth disparity, gt <= 0 marks an invalid pixel
+ *   er_weight      weight of the replay term (adapt.py's 0.05), finite and >= 0
+ *   loss_replay    [2]               {khamis term, total = loss[0] + er_weight * khamis} (the loss AdaptStepper.step returns) */
+SNB_API int snb_stereonet_adapt_forward_replay(float* const* params, long long* const* bn_counters, int k, int input_scale,
+                                       int maxdisp, const float* images, int B, int H, int W, const float* replay_images,
+                                       const float* replay_gt, int RB, float er_weight, void* state, void* workspace, float* loss,
+                                       float* loss_replay, float* disp, float* fcs, float* fcs_mean, void* stream);
+/* Gradients of the total loss (both passes) into the bucket, then snb_adam_clip_step as snb_stereonet_adapt_update. */
+SNB_API int snb_stereonet_adapt_update_replay(float* const* params, int k, int input_scale, int maxdisp, int B, int H, int W, int RB,
+                                      void* state, void* workspace, float max_norm, double lr, double beta1, double beta2, double eps,
+                                      void* stream);
 
 #ifdef __cplusplus
 }

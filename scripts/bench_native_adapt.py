@@ -6,7 +6,10 @@ by round:
   python_2s     AdaptStepper(make_optimizer(fused=True), use_graph=True), the default: feature passes and weight gradients on
                 side streams.
 Each variant adapts its own copy of the same seeded model on the same frame; `frame_us` is event time of back-to-back steps.
-Usage: python scripts/bench_native_adapt.py [out.json]"""
+--replay times the experience-replay step instead (snb_stereonet_adapt_forward_replay + _update_replay against
+AdaptStepper.step(..., replay=(rl, rr, gt)), one stored sample, er_weight 0.05).  python_2s then runs the replay pass on a stream of
+its own next to the stream pass; the native step and python_1s run the two passes one after the other.
+Usage: python scripts/bench_native_adapt.py [--replay] [out.json]"""
 import json
 import os
 import statistics
@@ -35,17 +38,26 @@ def nets():
 
 
 def main():
+  argv = [a for a in sys.argv[1:] if a != "--replay"]
+  replay = "--replay" in sys.argv[1:]
   g = torch.Generator(device=DEV).manual_seed(5)
   pair = torch.rand((2, B, 3, H, W), device=DEV, generator=g)
+  rpair = torch.rand((2, B, 3, H, W), device=DEV, generator=g)
+  gt = torch.rand((B, H, W), device=DEV, generator=g) * 40.0 + 0.5
+  gt[:, :, :W // 4] = 0.0
   stream = torch.cuda.current_stream()
 
   nat = native.NativeAdapt(*nets(), lr=5e-5)
   loss = torch.empty((1 + B,), device=DEV)
-  nat.workspace(B, H, W)
+  loss_replay = torch.empty((2,), device=DEV)
+  nat.workspace(B, H, W, B if replay else 0)
   torch.cuda.synchronize()
   g1, g2 = torch.cuda.CUDAGraph(), torch.cuda.CUDAGraph()
   with torch.cuda.graph(g1):
-    nat.forward(pair, loss)
+    if replay:
+      nat.forward(pair, loss, replay=(rpair, gt), loss_replay=loss_replay)
+    else:
+      nat.forward(pair, loss)
   with torch.cuda.graph(g2):
     nat.update()
 
@@ -58,21 +70,24 @@ def main():
     steppers[name] = AdaptStepper(f, n, make_optimizer(f, n, lr=5e-5, fused=True), use_graph=True, two_streams=two)
   paths = {"native": native_step}
   for name, st in steppers.items():
-    paths[name] = (lambda st=st: st.step(pair[0], pair[1]))
+    rep = (rpair[0], rpair[1], gt) if replay else None
+    paths[name] = (lambda st=st, rep=rep: st.step(pair[0], pair[1], replay=rep))
   for fn in paths.values():                                  # capture / warm every path
     timed(fn, 3, stream)
   rows = {name: [] for name in paths}
   for _ in range(ROUNDS):
     for name, fn in paths.items():
       rows[name].append(timed(fn, N, stream)[0])
-  res = dict(card=card(), shape=dict(B=B, H=H, W=W, k=K, maxdisp=MAXDISP, clip=True), rounds=ROUNDS, steps_per_round=N,
-             workspace_bytes=nat.workspace(B, H, W).numel())
+  shape = dict(B=B, H=H, W=W, k=K, maxdisp=MAXDISP, clip=True)
+  if replay:
+    shape.update(RB=B, er_weight=0.05)
+  res = dict(card=card(), shape=shape, rounds=ROUNDS, steps_per_round=N, workspace_bytes=nat.workspace(B, H, W, B if replay else 0).numel())
   for name, r in rows.items():
     res[name] = dict(frame_us_median=statistics.median(r), frame_us_min=min(r), frame_us_max=max(r))
   print(json.dumps(res, indent=1))
-  if len(sys.argv) > 1:
-    os.makedirs(os.path.dirname(os.path.abspath(sys.argv[1])), exist_ok=True)
-    with open(sys.argv[1], "w") as fh:
+  if argv:
+    os.makedirs(os.path.dirname(os.path.abspath(argv[0])), exist_ok=True)
+    with open(argv[0], "w") as fh:
       json.dump(res, fh, indent=1)
 
 
