@@ -149,7 +149,8 @@ __device__ __forceinline__ void mma_f16_i(uint32_t tmem_d, uint32_t tmem_a, uint
 // descriptor is (per-group base) + (compile-time offset), so an MMA costs its UTCHMMA plus a couple of uniform adds — the single
 // issuing thread is slow (a version with per-MMA loops / predicates over runtime group tables ran 2x slower end to end).
 // SKIP_FIRST: the first product(s) of (kw = 0, ks = 0) were issued by the caller (new tile, accumulate = 0).
-template <int MODE, int NG, bool SKIP_FIRST, int NKW>
+// SINGLE: the single-product variant, xh . wh only (see conv_c32_ws_kernel).
+template <int MODE, int NG, bool SKIP_FIRST, int NKW, bool SINGLE>
 __device__ __forceinline__ void issue_window(uint32_t d1, uint32_t d2, const uint32_t (&g_d)[3], uint32_t ta, uint32_t img0,
                                              const uint32_t (&g_b)[3], const uint32_t (&g_i)[3]) {
   using C = Cfg<MODE>;
@@ -170,6 +171,7 @@ __device__ __forceinline__ void issue_window(uint32_t d1, uint32_t d2, const uin
 #pragma unroll
       for (int g = 0; g < NG; ++g) {
         if (!skip) mma_f16_i(dd1[g], a, bd[g] + o1, g_i[g], 1);                      // xh . wh
+        if (SINGLE) continue;
         if (!(skip && D3)) mma_f16_i(dd2[g], a + 16, bd[g] + o2, g_i[g], 1);         // xl' . (3-D: wh -> D2; 2-D: 2^-11 wh)
         mma_f16_i(dd2[g], a, bd[g] + o3, g_i[g], 1);                                 // xh . (3-D: wl'' -> D2; 2-D: wl)
       }
@@ -179,7 +181,11 @@ __device__ __forceinline__ void issue_window(uint32_t d1, uint32_t d2, const uin
 
 // FOLD (the product setting): one N = 96 MMA over the three ring blocks per product (see above) instead of three N = 32 MMAs:
 // 37 / 40 / 44 us against 41 / 44 / 48 us per KITTI refinement block (dilation 1 / 4 / 8), 55 against 61 us per 3-D filter layer.
-template <int MODE, bool FOLD, bool RES2>      // RES2: a residual that is not the layer's input (p.res_mode == 2), added from a TMA-loaded tile
+// SINGLE (MODE_2D / MODE_3D, inference only, no statistics): the reduced-precision variant that keeps only the first product of the
+// split, out = 2^-s (xh . wh) — 10 explicit mantissa bits per operand instead of fp32-grade.  The converters write only the xh half
+// of an A slot, the MMA warp issues one product per (window, kw, k-step) instead of three, the 3-D D2 ring is neither written nor
+// read, and only the wh half of the same weight images is used (2-D: the P block of each image is all that is fetched).
+template <int MODE, bool FOLD, bool RES2, bool SINGLE>      // RES2: a residual that is not the layer's input (p.res_mode == 2), added from a TMA-loaded tile
 __global__ void __launch_bounds__(NTHREADS_WS, 1)
 conv_c32_ws_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_constant__ CUtensorMap tmap_out,
                    const __grid_constant__ CUtensorMap tmap_res, const __grid_constant__ CUtensorMap tmap_p1,
@@ -189,6 +195,8 @@ conv_c32_ws_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_consta
   using C = Cfg<MODE>;
   constexpr int NA = C::NA, NRES = C::NRES, NWIN = C::NWIN;
   constexpr bool D3 = C::FLAT, TWO = C::TWO;
+  static_assert(!SINGLE || MODE == MODE_2D || MODE == MODE_3D, "single-product variant: 2-D and 3-D layers only");
+  constexpr int WLOAD = (SINGLE && !TWO) ? B_BYTES : C::IMG_BYTES;     // bytes fetched per weight image (2-D single: P only)
   extern __shared__ unsigned char smem_dyn[];
   const uint32_t base_u32 = (smem_u32(smem_dyn) + 1023u) & ~1023u;
   unsigned char* base = smem_dyn + (base_u32 - smem_u32(smem_dyn));
@@ -237,9 +245,9 @@ conv_c32_ws_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_consta
   if (warp == 1 && lane == 0) {
     asm volatile("prefetch.tensormap [%0];\n" :: "l"(reinterpret_cast<uint64_t>(&tmap)) : "memory");
     asm volatile("prefetch.tensormap [%0];\n" :: "l"(reinterpret_cast<uint64_t>(&tmap_out)) : "memory");
-    mbar_expect_tx(wbar, C::NIMG * C::IMG_BYTES);
+    mbar_expect_tx(wbar, C::NIMG * WLOAD);
     for (int w = 0; w < C::NIMG; ++w)
-      bulk_g2s(sB + w * C::IMG_BYTES, p.wimg + (size_t)w * (C::IMG_BYTES / 4), C::IMG_BYTES, wbar);
+      bulk_g2s(sB + w * C::IMG_BYTES, p.wimg + (size_t)w * (C::IMG_BYTES / 4), WLOAD, wbar);
   }
   pdl_launch();                                    // only after this CTA owns its TMEM columns
   pdl_wait();
@@ -342,27 +350,27 @@ conv_c32_ws_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_consta
               if (go_i[0]) mma_f16_i(d1 + go_d[0], ta, make_desc(img0 + go_b[0]), go_i[0], 1);
               if (go_i[1]) mma_f16_i(d1 + go_d[1], ta, make_desc(img0 + go_b[1]), go_i[1], 1);
               mma_f16_i(d1 + new_d, ta, make_desc(img0 + 2 * 4096), idesc_n(1), 0);             // D1 = xh . wh
-              if (TWO) {
+              if (TWO && !SINGLE) {
                 if (go_i[0]) mma_f16_i(d2 + go_d[0], ta + 16, make_desc(img0 + go_b[0]), go_i[0], 1);
                 if (go_i[1]) mma_f16_i(d2 + go_d[1], ta + 16, make_desc(img0 + go_b[1]), go_i[1], 1);
                 mma_f16_i(d2 + new_d, ta + 16, make_desc(img0 + 2 * 4096), idesc_n(1), 0);      // D2 = xl' . wh
               }
               constexpr int NKW0 = C::nkw(0);                   // (window 0 has three kw taps; C4: one)
-              if (ng == 1) issue_window<MODE, 1, true, NKW0>(d1, d2, g_d, ta, img0, g_b, g_i);
-              else if (ng == 2) issue_window<MODE, 2, true, NKW0>(d1, d2, g_d, ta, img0, g_b, g_i);
-              else issue_window<MODE, 3, true, NKW0>(d1, d2, g_d, ta, img0, g_b, g_i);
+              if (ng == 1) issue_window<MODE, 1, true, NKW0, SINGLE>(d1, d2, g_d, ta, img0, g_b, g_i);
+              else if (ng == 2) issue_window<MODE, 2, true, NKW0, SINGLE>(d1, d2, g_d, ta, img0, g_b, g_i);
+              else issue_window<MODE, 3, true, NKW0, SINGLE>(d1, d2, g_d, ta, img0, g_b, g_i);
             } else if (MODE == MODE_C4) {
-              if (ng == 1) issue_window<MODE, 1, false, 1>(d1, d2, g_d, ta, img0, g_b, g_i);
-              else if (ng == 2) issue_window<MODE, 2, false, 1>(d1, d2, g_d, ta, img0, g_b, g_i);
-              else issue_window<MODE, 3, false, 1>(d1, d2, g_d, ta, img0, g_b, g_i);
+              if (ng == 1) issue_window<MODE, 1, false, 1, SINGLE>(d1, d2, g_d, ta, img0, g_b, g_i);
+              else if (ng == 2) issue_window<MODE, 2, false, 1, SINGLE>(d1, d2, g_d, ta, img0, g_b, g_i);
+              else issue_window<MODE, 3, false, 1, SINGLE>(d1, d2, g_d, ta, img0, g_b, g_i);
             } else if (nkw == 3) {
-              if (ng == 1) issue_window<MODE, 1, false, 3>(d1, d2, g_d, ta, img0, g_b, g_i);
-              else if (ng == 2) issue_window<MODE, 2, false, 3>(d1, d2, g_d, ta, img0, g_b, g_i);
-              else issue_window<MODE, 3, false, 3>(d1, d2, g_d, ta, img0, g_b, g_i);
+              if (ng == 1) issue_window<MODE, 1, false, 3, SINGLE>(d1, d2, g_d, ta, img0, g_b, g_i);
+              else if (ng == 2) issue_window<MODE, 2, false, 3, SINGLE>(d1, d2, g_d, ta, img0, g_b, g_i);
+              else issue_window<MODE, 3, false, 3, SINGLE>(d1, d2, g_d, ta, img0, g_b, g_i);
             } else {                                            // P4, odd-column phase (never the first window of a step)
-              if (ng == 1) issue_window<MODE, 1, false, 2>(d1, d2, g_d, ta, img0, g_b, g_i);
-              else if (ng == 2) issue_window<MODE, 2, false, 2>(d1, d2, g_d, ta, img0, g_b, g_i);
-              else issue_window<MODE, 3, false, 2>(d1, d2, g_d, ta, img0, g_b, g_i);
+              if (ng == 1) issue_window<MODE, 1, false, 2, SINGLE>(d1, d2, g_d, ta, img0, g_b, g_i);
+              else if (ng == 2) issue_window<MODE, 2, false, 2, SINGLE>(d1, d2, g_d, ta, img0, g_b, g_i);
+              else issue_window<MODE, 3, false, 2, SINGLE>(d1, d2, g_d, ta, img0, g_b, g_i);
             }
             if (win == NWIN - 1 && u >= 2) mma_commit_raw(&tfull[(tile_base + (uint32_t)(u - 2)) % RING]);   // tile u-2 has all its kz taps
             mma_commit_raw(&aempty[aslot]);
@@ -439,23 +447,34 @@ conv_c32_ws_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_consta
               float4 v[8];
 #pragma unroll
               for (int c = 0; c < 8; ++c) v[c] = *reinterpret_cast<const float4*>(rp + ((c ^ (m & 7)) << 4));
-              uint32_t hl[32];
-              split_f16(v, hl);
+              if (SINGLE) {                                   // the xh half only (chunks 0..3); chunks 4..7 are never read
+                uint32_t h[16];
+                hi_f16(v, h);
 #pragma unroll
-              for (int c = 0; c < 8; ++c)
-                *reinterpret_cast<uint4*>(rp + ((c ^ (m & 7)) << 4)) = make_uint4(hl[4 * c], hl[4 * c + 1], hl[4 * c + 2], hl[4 * c + 3]);
+                for (int c = 0; c < 4; ++c)
+                  *reinterpret_cast<uint4*>(rp + ((c ^ (m & 7)) << 4)) = make_uint4(h[4 * c], h[4 * c + 1], h[4 * c + 2], h[4 * c + 3]);
+              } else {
+                uint32_t hl[32];
+                split_f16(v, hl);
+#pragma unroll
+                for (int c = 0; c < 8; ++c)
+                  *reinterpret_cast<uint4*>(rp + ((c ^ (m & 7)) << 4)) = make_uint4(hl[4 * c], hl[4 * c + 1], hl[4 * c + 2], hl[4 * c + 3]);
+              }
             }
             if (quad == 3 && lane < 16) {                     // the two halo rows 128, 129: one 16-B input chunk per lane
               const int row = 128 + (lane >> 3), c = lane & 7;
               unsigned char* rp = rw + row * 128;
               const float4 x = *reinterpret_cast<const float4*>(rp + ((c ^ (row & 7)) << 4));
               const uint32_t h0 = pack_f16x2(x.x, x.y), h1 = pack_f16x2(x.z, x.w);
-              const float2 f0 = unpack_f16x2(h0), f1 = unpack_f16x2(h1);
-              const uint32_t l0 = pack_f16x2((x.x - f0.x) * 2048.f, (x.y - f0.y) * 2048.f);
-              const uint32_t l1 = pack_f16x2((x.z - f1.x) * 2048.f, (x.w - f1.y) * 2048.f);
+              uint32_t l0 = 0u, l1 = 0u;
+              if (!SINGLE) {
+                const float2 f0 = unpack_f16x2(h0), f1 = unpack_f16x2(h1);
+                l0 = pack_f16x2((x.x - f0.x) * 2048.f, (x.y - f0.y) * 2048.f);
+                l1 = pack_f16x2((x.z - f1.x) * 2048.f, (x.w - f1.y) * 2048.f);
+              }
               __syncwarp(0x0000ffffu);                        // in place: every lane has read its chunk before any lane writes
               *reinterpret_cast<uint2*>(rp + (((c >> 1) ^ (row & 7)) << 4) + (c & 1) * 8) = make_uint2(h0, h1);
-              *reinterpret_cast<uint2*>(rp + (((4 + (c >> 1)) ^ (row & 7)) << 4) + (c & 1) * 8) = make_uint2(l0, l1);
+              if (!SINGLE) *reinterpret_cast<uint2*>(rp + (((4 + (c >> 1)) ^ (row & 7)) << 4) + (c & 1) * 8) = make_uint2(l0, l1);
             }
             fence_async_smem();                               // these generic-proxy writes precede the TMA's next write of the slot
             group_bar(7 + (int)grp);                          // the split rows of all four warps are visible
@@ -466,6 +485,25 @@ conv_c32_ws_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_consta
               if (kw >= nkw) break;
               const int row = m + kw;
               const unsigned char* rp = rw + row * 128;
+              if (SINGLE) {                                   // xh half of the split row -> xh half of A slot [kw]
+                uint32_t h[16];
+#pragma unroll
+                for (int c = 0; c < 4; ++c) {
+                  const uint4 q = *reinterpret_cast<const uint4*>(rp + ((c ^ (row & 7)) << 4));
+                  h[4 * c] = q.x; h[4 * c + 1] = q.y; h[4 * c + 2] = q.z; h[4 * c + 3] = q.w;
+                }
+                if (kw == nkw - 1) {
+                  const uint32_t dep = h[0] ^ h[4] ^ h[8] ^ h[12];
+                  __syncwarp();
+                  if (lane == 0) mbar_arrive_after(&rempty[sr], dep);
+                }
+                if ((kw == 0 && wcol == 0) || (kw == 2 && wcol == p.W - 1)) {
+#pragma unroll
+                  for (int i = 0; i < 16; ++i) h[i] = 0u;
+                }
+                tmem_st16(ta + kw * 32, h);
+                continue;
+              }
               uint32_t hl[32];
 #pragma unroll
               for (int c = 0; c < 8; ++c) {
@@ -495,9 +533,11 @@ conv_c32_ws_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_consta
 #pragma unroll
             for (int c = 0; c < 8; ++c) v[c] = *reinterpret_cast<const float4*>(rp + ((c ^ (row & 7)) << 4));
             uint32_t hl[32];
-            split_f16(v, hl);
+            if (SINGLE) hi_f16(v, reinterpret_cast<uint32_t (&)[16]>(hl));     // xh only: hl[0..15]
+            else split_f16(v, hl);
             if (kw == nkw - 1) {                             // last read of the raw window: release it once the loads have returned
-              const uint32_t dep = hl[0] ^ hl[5] ^ hl[10] ^ hl[15] ^ hl[3] ^ hl[6] ^ hl[9] ^ hl[12];     // one word of each of the 8 loads
+              const uint32_t dep = SINGLE ? hl[0] ^ hl[2] ^ hl[4] ^ hl[6] ^ hl[8] ^ hl[10] ^ hl[12] ^ hl[14]
+                                          : hl[0] ^ hl[5] ^ hl[10] ^ hl[15] ^ hl[3] ^ hl[6] ^ hl[9] ^ hl[12];     // one word of each of the 8 loads
               __syncwarp();
               if (lane == 0) mbar_arrive_after(&rempty[sr], dep);
             }
@@ -511,7 +551,8 @@ conv_c32_ws_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_consta
               tc_fence_after();
               a_free = true;
             }
-            tmem_st32(ta + kw * 32, hl);
+            if (SINGLE) tmem_st16(ta + kw * 32, reinterpret_cast<const uint32_t (&)[16]>(hl));
+            else tmem_st32(ta + kw * 32, hl);
             if (MODE == MODE_2D && kw == 1 && centre) {
               const int rslot = (int)(tcount % NRES);
               WSWAIT(w_rs, tc::mbar_wait(&rsempty[rslot], (uint32_t)(((tcount / NRES) & 1) ^ 1)));
@@ -545,7 +586,7 @@ conv_c32_ws_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_consta
     const int chunk = et & 7, rg = et >> 3;          // coalesced pass: rows rg + 16*i, 16-B chunk `chunk`
     const uint32_t tlane = tmem_base + ((uint32_t)(quad * 32) << 16);
     const snb_conv_epilogue& e = p.e;
-    const bool has_stats = e.stats != nullptr;
+    const bool has_stats = !SINGLE && e.stats != nullptr;
     const float slope = e.lrelu ? SNB_LRELU_SLOPE : 1.f;
     float* red = sRed + egrp * 256;
     // Output path: the staged tile (SWIZZLE_128B image of 128 positions x 32 ch) leaves through ONE TMA tile store (positions
@@ -591,7 +632,7 @@ conv_c32_ws_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_consta
         const long long tB = p.dbg ? clock64() : 0;
         {
           float acc[32], res[32];
-          if (TWO) {
+          if (TWO && !SINGLE) {
             tmem_ld32x2(tlane + C::D1_BASE + slot * 32, tlane + C::D2_BASE + slot * 32, acc, res);
 #pragma unroll
             for (int i = 0; i < 32; ++i) acc[i] = fmaf(res[i], 1.f / 2048.f, acc[i]);             // D1 + 2^-11 D2
@@ -761,8 +802,9 @@ extern "C" int snb_conv_weights_ws_floats(int kd) {      // kd = 5: the ten-imag
 
 // p4: 0 = plain conv; 1 = MODE_P4 over a split input x = phases [4][B][OH][OW][32]; 2 = MODE_P4 over the un-split input
 // x [B][in_h][in_w][32] through strided tensor maps (phase (a,b) = x[2i+a][2j+b], zero fill past the odd edge).
+// single: the single-product variant of MODE_2D / MODE_3D (snb_conv_c32_ws_f16).
 static int ws_launch(const float* x, const float* wimg, float* y, const snb_conv_geom* g, const snb_conv_epilogue* e,
-                     long long* dbg, void* stream, int p4 = 0, int in_h = 0, int in_w = 0, bool c4 = false) {
+                     long long* dbg, void* stream, int p4 = 0, int in_h = 0, int in_w = 0, bool c4 = false, bool single = false) {
   wsk::Params p;
   if (int rc = ws_setup(g, p, "snb_conv_c32_ws")) return rc;
   SNB_REQUIRE(x && wimg && y && e, "snb_conv_c32_ws: null pointer");
@@ -831,14 +873,18 @@ static int ws_launch(const float* x, const float* wimg, float* y, const snb_conv
   SNB_CUDA(cudaGetDevice(&dev));
   SNB_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
   const int grid = p.nstrips < sms ? p.nstrips : sms;
-#define WS_GO(MODEV, FOLDV, RESV) do { \
-    SNB_CUDA(cudaFuncSetAttribute(wsk::conv_c32_ws_kernel<MODEV, FOLDV, RESV>, cudaFuncAttributeMaxDynamicSharedMemorySize, wsk::Cfg<MODEV>::SMEM_BYTES)); \
-    snb_launch(wsk::conv_c32_ws_kernel<MODEV, FOLDV, RESV>, grid, wsk::NTHREADS_WS, wsk::Cfg<MODEV>::SMEM_BYTES, stream, tmap, tmap_out, tmap_res, tmap_ph[1], tmap_ph[2], tmap_ph[3], p); } while (0)
+#define WS_GO(MODEV, FOLDV, RESV, SINGLEV) do { \
+    SNB_CUDA(cudaFuncSetAttribute(wsk::conv_c32_ws_kernel<MODEV, FOLDV, RESV, SINGLEV>, cudaFuncAttributeMaxDynamicSharedMemorySize, wsk::Cfg<MODEV>::SMEM_BYTES)); \
+    snb_launch(wsk::conv_c32_ws_kernel<MODEV, FOLDV, RESV, SINGLEV>, grid, wsk::NTHREADS_WS, wsk::Cfg<MODEV>::SMEM_BYTES, stream, tmap, tmap_out, tmap_res, tmap_ph[1], tmap_ph[2], tmap_ph[3], p); } while (0)
   const bool res2 = p.res_mode == 2;
-  if (c4) WS_GO(wsk::MODE_C4, true, false);
-  else if (p4) { if (res2) WS_GO(wsk::MODE_P4, true, true); else WS_GO(wsk::MODE_P4, true, false); }
-  else if (d3) { if (res2) WS_GO(wsk::MODE_3D, true, true); else WS_GO(wsk::MODE_3D, true, false); }
-  else    { if (res2) WS_GO(wsk::MODE_2D, true, true); else WS_GO(wsk::MODE_2D, true, false); }
+  if (single) {
+    if (d3) { if (res2) WS_GO(wsk::MODE_3D, true, true, true); else WS_GO(wsk::MODE_3D, true, false, true); }
+    else    { if (res2) WS_GO(wsk::MODE_2D, true, true, true); else WS_GO(wsk::MODE_2D, true, false, true); }
+  }
+  else if (c4) WS_GO(wsk::MODE_C4, true, false, false);
+  else if (p4) { if (res2) WS_GO(wsk::MODE_P4, true, true, false); else WS_GO(wsk::MODE_P4, true, false, false); }
+  else if (d3) { if (res2) WS_GO(wsk::MODE_3D, true, true, false); else WS_GO(wsk::MODE_3D, true, false, false); }
+  else    { if (res2) WS_GO(wsk::MODE_2D, true, true, false); else WS_GO(wsk::MODE_2D, true, false, false); }
 #undef WS_GO
   SNB_LAUNCH_CHECK("conv_c32_ws_kernel");
   return 0;
@@ -847,6 +893,14 @@ static int ws_launch(const float* x, const float* wimg, float* y, const snb_conv
 extern "C" int snb_conv_c32_ws(const float* x, const float* wimg, float* y, const snb_conv_geom* g, const snb_conv_epilogue* e,
                                void* stream) {
   return ws_launch(x, wimg, y, g, e, nullptr, stream);
+}
+
+// The single-product variant: same contract and weight image as snb_conv_c32_ws, out = 2^-s (xh . wh); inference only (no `stats`).
+extern "C" int snb_conv_c32_ws_f16(const float* x, const float* wimg, float* y, const snb_conv_geom* g, const snb_conv_epilogue* e,
+                                   void* stream) {
+  SNB_REQUIRE(e != nullptr, "snb_conv_c32_ws_f16: null epilogue");
+  SNB_REQUIRE(e->stats == nullptr, "snb_conv_c32_ws_f16: `stats` must be NULL (train-mode BatchNorm statistics stay on snb_conv_c32_ws)");
+  return ws_launch(x, wimg, y, g, e, nullptr, stream, 0, 0, 0, false, true);
 }
 
 extern "C" int snb_conv_c32_ws_profile(const float* x, const float* wimg, float* y, const snb_conv_geom* g,

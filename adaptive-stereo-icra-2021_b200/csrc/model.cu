@@ -97,9 +97,14 @@ extern "C" long long snb_stereonet_workspace_bytes(int k, int input_scale, int m
   return carve(d).total;
 }
 
-extern "C" int snb_stereonet_forward(const void* weights, int k, int input_scale, int maxdisp, const float* images, int B, int H, int W,
-                                     void* workspace, float* disp, float* coarse, float* cost, float* fcs, void* stream) {
-  const char* who = "snb_stereonet_forward";
+// Which 32->32 walk-kernel layers the reduced-precision forward runs on the single-product variant (snb_conv_c32_ws_f16).
+constexpr int F16_2D = 1, F16_3D = 2;
+constexpr int F16_LAYERS = F16_2D | F16_3D;
+
+// The forward of both exported entry points: `single` = 0 (snb_stereonet_forward) or F16_LAYERS (snb_stereonet_forward_f16).
+static int stereonet_forward(int single, const char* who, const void* weights, int k, int input_scale, int maxdisp,
+                             const float* images, int B, int H, int W, void* workspace, float* disp, float* coarse, float* cost,
+                             float* fcs, void* stream) {
   Dims d;
   if (int rc = check_dims(who, k, input_scale, maxdisp, B, H, W, d)) return rc;
   SNB_REQUIRE(weights != nullptr && aligned(weights, ALIGN), "%s: `weights` must be a non-null 256-byte aligned pointer", who);
@@ -147,11 +152,12 @@ extern "C" int snb_stereonet_forward(const void* weights, int k, int input_scale
     x = y;
   }
   const int h = d.h, w = d.w;
+  auto conv_ws = [&](int kind) { return (single & kind) ? snb_conv_c32_ws_f16 : snb_conv_c32_ws; };
   auto conv_bn_lrelu = [&](float* in, float* out, const snb_conv_geom& g, bool residual) {
     const float* wi = next(); const float* bi = next(); const float* sc = next(); const float* sh = next();
     ti += 2;                                                       // running statistics: folded into sc / sh
     snb_conv_epilogue e = {bi, sc, sh, residual ? in : nullptr, nullptr, 1};
-    return snb_conv_c32_ws(in, wi, out, &g, &e, stream);
+    return conv_ws(g.KD == 3 ? F16_3D : F16_2D)(in, wi, out, &g, &e, stream);
   };
   const snb_conv_geom gf = geom3x3(N2, 1, h, w, 1, false);
   for (int i = 0; i < 6; ++i) {                                    // BasicBlock: x + LeakyReLU(BN(conv1(x)))
@@ -163,7 +169,7 @@ extern "C" int snb_stereonet_forward(const void* weights, int k, int input_scale
     const float* wi = next(); const float* bi = next();
     float* y = x == fa ? fb : fa;
     snb_conv_epilogue e = {bi, nullptr, nullptr, nullptr, nullptr, 0};
-    if (int rc = snb_conv_c32_ws(x, wi, y, &gf, &e, stream)) return rc;
+    if (int rc = conv_ws(F16_2D)(x, wi, y, &gf, &e, stream)) return rc;
     x = y;
   }
   const float* left = x;
@@ -217,4 +223,16 @@ extern "C" int snb_stereonet_forward(const void* weights, int k, int input_scale
   if (fcs)
     if (int rc = snb_feature_contrast(cost, fcs, B, d.D, h, w, stream)) return rc;
   return 0;
+}
+
+extern "C" int snb_stereonet_forward(const void* weights, int k, int input_scale, int maxdisp, const float* images, int B, int H, int W,
+                                     void* workspace, float* disp, float* coarse, float* cost, float* fcs, void* stream) {
+  return stereonet_forward(0, "snb_stereonet_forward", weights, k, input_scale, maxdisp, images, B, H, W, workspace, disp, coarse,
+                           cost, fcs, stream);
+}
+
+extern "C" int snb_stereonet_forward_f16(const void* weights, int k, int input_scale, int maxdisp, const float* images, int B, int H,
+                                         int W, void* workspace, float* disp, float* coarse, float* cost, float* fcs, void* stream) {
+  return stereonet_forward(F16_LAYERS, "snb_stereonet_forward_f16", weights, k, input_scale, maxdisp, images, B, H, W, workspace, disp,
+                           coarse, cost, fcs, stream);
 }

@@ -131,6 +131,15 @@ __device__ __forceinline__ void tmem_st32(uint32_t taddr, const uint32_t (&r)[32
       : "memory");
 }
 __device__ __forceinline__ void tmem_wait_st() { asm volatile("tcgen05.wait::st.sync.aligned;\n" ::: "memory"); }
+// registers -> TMEM, 16 consecutive 32-bit columns
+__device__ __forceinline__ void tmem_st16(uint32_t taddr, const uint32_t (&r)[16]) {
+  asm volatile(
+      "tcgen05.st.sync.aligned.32x32b.x16.b32 [%0], "
+      "{%1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, %16};\n"
+      :: "r"(taddr), "r"(r[0]), "r"(r[1]), "r"(r[2]), "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7]),
+         "r"(r[8]), "r"(r[9]), "r"(r[10]), "r"(r[11]), "r"(r[12]), "r"(r[13]), "r"(r[14]), "r"(r[15])
+      : "memory");
+}
 
 __device__ __forceinline__ void tmem_ld16(uint32_t taddr, float (&v)[16]) {
   uint32_t r[16];
@@ -217,6 +226,11 @@ __device__ __forceinline__ void split_f16(const float4 (&v)[8], uint32_t (&hl)[3
     hl[16 + 2 * c] = pack_f16x2((v[c].x - f0.x) * 2048.f, (v[c].y - f0.y) * 2048.f);
     hl[16 + 2 * c + 1] = pack_f16x2((v[c].z - f1.x) * 2048.f, (v[c].w - f1.y) * 2048.f);
   }
+}
+// 32 fp32 channels of one position -> the 16 packed xh words only (single-product operands: no xl')
+__device__ __forceinline__ void hi_f16(const float4 (&v)[8], uint32_t (&h)[16]) {
+#pragma unroll
+  for (int c = 0; c < 8; ++c) { h[2 * c] = pack_f16x2(v[c].x, v[c].y); h[2 * c + 1] = pack_f16x2(v[c].z, v[c].w); }
 }
 
 // mbarrier.arrive that is data-dependent on `dep`: the arrive cannot ISSUE before the instructions that produced `dep` have

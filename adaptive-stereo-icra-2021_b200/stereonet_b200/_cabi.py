@@ -35,6 +35,7 @@ SIGNATURES = {
   "snb_conv_c32_tc_profile": (_I, [_P, _P, _P, _GP, _EP, _I, _P, _P]),
   "snb_conv_c32_ws": (_I, [_P, _P, _P, _GP, _EP, _P]),
   "snb_conv_c32_ws_num_tiles": (_I, [_GP]),
+  "snb_conv_c32_ws_f16": (_I, [_P, _P, _P, _GP, _EP, _P]),
   "snb_conv_weights_ws_floats": (_I, [_I]),
   "snb_conv_c32_ws_profile": (_I, [_P, _P, _P, _GP, _EP, _P, _P]),
   "snb_prep_conv_weights_tc": (_I, [_P, _P, _I, _I, _P]),
@@ -93,6 +94,7 @@ SIGNATURES = {
   "snb_stereonet_prepare": (_I, [_P, _I, _P, _P]),
   "snb_stereonet_workspace_bytes": (_LL, [_I, _I, _I, _I, _I, _I]),
   "snb_stereonet_forward": (_I, [_P, _I, _I, _I, _P, _I, _I, _I, _P, _P, _P, _P, _P, _P]),
+  "snb_stereonet_forward_f16": (_I, [_P, _I, _I, _I, _P, _I, _I, _I, _P, _P, _P, _P, _P, _P]),
   "snb_stereonet_adapt_state_bytes": (_LL, [_I]),
   "snb_stereonet_adapt_state_piece": (_I, [_I, _I, C.POINTER(_LL), C.POINTER(_LL)]),
   "snb_stereonet_adapt_grad_slot": (_I, [_I, _I, C.POINTER(_LL), C.POINTER(_LL)]),

@@ -116,6 +116,21 @@ _FMT = {"ws": "ws", "h3": "h", "tc3": 3, "tc1": 1}
 WS_3D_FMT = "ws"
 
 
+# Reduced-precision inference (runtime.StereoEngine(..., precision="fp16")): the kinds of 32->32 walk-kernel layer, "2d" (3x3, dilated)
+# and "3d" (3x3x3), that run on the single-product variant snb_conv_c32_ws_f16 instead of the fp32-grade split.  Empty (the default)
+# everywhere but inside the engine's own no-grad eval forward, which sets it to F16_SHIPPED and resets it, as AdaptStepper does with
+# DEFER_BN / WGRAD_STREAM.  The nn.Module forward, the grad-enabled paths and AdaptStepper never see it set; a layer that finds it set
+# while grad is enabled raises.  F16_SHIPPED is the layer set of snb_stereonet_forward_f16 (csrc/model.cu F16_LAYERS).
+F16_LAYERS = frozenset()
+F16_SHIPPED = frozenset(("2d", "3d"))
+
+
+def _f16_guard():
+  if F16_LAYERS and torch.is_grad_enabled():
+    raise RuntimeError("stereonet_b200: the fp16 inference forward runs under torch.no_grad() only "
+                       "(training and the adaptation step stay on the fp32-grade kernels)")
+
+
 def _fmt(three_d):
   f = _FMT[CONV_BACKEND]
   return WS_3D_FMT if (f == "ws" and three_d) else f
@@ -140,6 +155,11 @@ def wprep_tc(conv, mode=0):
 
 def conv3x3_c32(x, conv, g, **kw):
   """Backend dispatch for the 'same' 3x3(x3) convolution + fused epilogue."""
+  if F16_LAYERS and ("3d" if x.dim() == 5 else "2d") in F16_LAYERS:
+    _f16_guard()
+    if CONV_BACKEND != "ws" or kw.pop("want_stats", False):
+      raise RuntimeError("stereonet_b200: the fp16 inference forward needs the 'ws' back end and eval-mode BatchNorm")
+    return ops.conv_c32_ws_f16(x, wprep_tc(conv), g, **kw), None
   if CONV_BACKEND == "ffma":
     return ops.conv_c32(x, wprep(conv), g, **kw)
   return ops.conv_c32_tc(x, wprep_tc(conv), g, **_tc_kw(x.dim() == 5), **kw)
@@ -329,6 +349,7 @@ def downsample_pair(img, conv0, conv1):
 def conv_plain(x, conv, ksize, stride):
   """Conv2d 32->32 with bias only (downsample[1:], conv_alone)."""
   g = ops.geom(x.shape, ksize, stride=stride, dil=1, pad=ksize // 2)
+  _f16_guard()
   if _needs_grad(x, conv):
     from . import functions
     return functions.conv_c32_autograd(x, conv, ksize, stride)
@@ -345,6 +366,7 @@ def conv_plain(x, conv, ksize, stride):
 def conv_bn_lrelu(x, conv, bn, dil, residual, training):
   """[x +] LeakyReLU(BN(conv(x))) for 3x3 (2-D, dilated) and 3x3x3 convs (stereo_net.py:8-18,21-30,44-51,155-160)."""
   g = ops.geom(x.shape, 3, stride=1, dil=dil)
+  _f16_guard()
   if _needs_grad(x, conv, bn):
     from . import functions
     return functions.conv_bn_lrelu_autograd(x, conv, bn, dil, residual, training)

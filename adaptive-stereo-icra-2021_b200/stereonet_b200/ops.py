@@ -238,6 +238,26 @@ def conv_c32_tc(x, wimg, g, bias=None, scale=None, shift=None, residual=None, lr
   return y, stats
 
 
+def conv_c32_ws_f16(x, wimg, g, bias=None, scale=None, shift=None, residual=None, lrelu=False, out=None):
+  """Reduced-precision inference variant of conv_c32_tc(fmt="ws") (snb_conv_c32_ws_f16): one fp16 product per tap, same weight
+  image and epilogue, no BatchNorm statistics.  Returns y."""
+  three_d = x.dim() == 5
+  _req(x, "x"); _req(wimg, "wimg")
+  y = out if out is not None else torch.empty(out_shape(g, three_d), device=x.device, dtype=torch.float32)
+  if out is not None:
+    _req(out, "out")
+    if tuple(out.shape) != tuple(out_shape(g, three_d)):
+      raise RuntimeError("stereonet_b200: `out` shape mismatch")
+  if residual is not None:
+    _req(residual, "residual")
+    if residual.shape != y.shape:
+      raise RuntimeError("stereonet_b200: residual shape mismatch")
+  e = ConvEpilogue(_p(bias), _p(scale), _p(shift), _p(residual), None, 1 if lrelu else 0)
+  check(_cabi.lib().snb_conv_c32_ws_f16(_p(x), _p(wimg), _p(y), C.byref(g), C.byref(e), _stream(x)), "snb_conv_c32_ws_f16")
+  _count()
+  return y
+
+
 def phase_split(x):
   """[B,H,W,32] -> [4,B,ceil(H/2),ceil(W/2),32]: phase a*2+b holds x[:, a::2, b::2] (zero padded to the common size)."""
   _req(x, "x", 4)

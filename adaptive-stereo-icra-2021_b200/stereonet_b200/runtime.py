@@ -5,7 +5,12 @@ images, folded BatchNorm) of the moment of capture, so every entry remembers the
 (autograd.fused.state_epoch(): advanced by optimizer steps, graph-replayed adaptation steps and train-mode BatchNorm updates) and
 is re-captured on the next call after a change — an adaptation loop that alternates AdaptStepper.step and engine(left, right)
 (adapt.py's validate / evaluate pattern) never sees stale weights.  `invalidate()` is only needed after parameters were
-re-assigned by other means (e.g. raw `.data` writes)."""
+re-assigned by other means (e.g. raw `.data` writes).
+
+precision="fp16" selects the opt-in reduced-precision forward for throughput inference: the 32->32 3x3 and 3x3x3 walk-kernel
+layers run one fp16 product per tap (snb_conv_c32_ws_f16) instead of the fp32-grade split.  Its disparities are reported separately
+from the fp32 parity contract (DESIGN.md section 4.2f16 lists the measured errors); it is bit-identical to snb_stereonet_forward_f16.
+Eval mode only: train-mode BatchNorm statistics stay on the fp32-grade path."""
 import torch
 
 from . import ops
@@ -13,7 +18,10 @@ from .autograd import fused
 
 
 class StereoEngine:
-  def __init__(self, feature_net, stereo_net, output_cost_volume=False, use_graph=True):
+  def __init__(self, feature_net, stereo_net, output_cost_volume=False, use_graph=True, precision="fp32"):
+    if precision not in ("fp32", "fp16"):
+      raise ValueError(f"precision must be 'fp32' or 'fp16', got {precision!r}")
+    self.precision = precision
     self.feature_net, self.stereo_net = feature_net, stereo_net
     self.output_cost_volume = output_cost_volume
     self.use_graph = use_graph
@@ -29,6 +37,18 @@ class StereoEngine:
     one batch (no op mixes samples when BN uses running statistics, SURVEY.md §8e: bit-identical to two calls, half
     the launches); in train mode the two calls stay separate because BN batch statistics are per call
     (adapt.py:72: feature_net(left), feature_net(right))."""
+    if self.precision == "fp32":
+      return self._forward_pair(pair)
+    if self.feature_net.training or self.stereo_net.training:
+      raise RuntimeError("stereonet_b200: StereoEngine(precision='fp16') runs eval-mode modules only")
+    old = fused.F16_LAYERS
+    fused.F16_LAYERS = fused.F16_SHIPPED
+    try:
+      return self._forward_pair(pair)
+    finally:
+      fused.F16_LAYERS = old
+
+  def _forward_pair(self, pair):
     B = pair.shape[0] // 2
     left, right = pair[:B], pair[B:]
     if self.feature_net.training:
@@ -42,7 +62,7 @@ class StereoEngine:
     """The captured forward for this input shape.  `slot` selects one of several independent captures (own static input and
     output buffers): the streaming API alternates between two so that the copies of one frame never touch the buffers the
     forward of its neighbour is using."""
-    key = (tuple(shape), str(device), self.feature_net.training, slot)
+    key = (tuple(shape), str(device), self.feature_net.training, slot, self.precision)
     e = self._graphs.get(key)
     if e is not None:
       if e["epoch"] == fused.state_epoch():

@@ -1,11 +1,12 @@
 // Whole-model StereoNet inference from C++ through include/snb200.h: no Python, no torch.
 //
-//   stereonet_infer WEIGHTS IMAGES B H W OUT [ITERS]
+//   stereonet_infer WEIGHTS IMAGES B H W OUT [ITERS [f16]]
 //
 // WEIGHTS  a file written by stereonet_b200.native.export_weights (format in that module's docstring)
 // IMAGES   raw float32 [2][B][3][H][W] (left batch, then right batch), NCHW
 // OUT      receives the full-resolution disparity, raw float32 [B][H][W]
 // ITERS    graph replays to time (default 100)
+// f16      run the opt-in reduced-precision forward snb_stereonet_forward_f16 instead (results reported apart from fp32 parity)
 //
 // Uploads the parameters, runs snb_stereonet_prepare, captures one snb_stereonet_forward into a CUDA graph, replays it ITERS
 // times and reports the mean time per frame from CUDA events.  Build: python adaptive-stereo-icra-2021_b200/build.py --example
@@ -42,11 +43,15 @@ static void* device_alloc(size_t bytes) {        // cudaMalloc returns 256-byte 
 
 int main(int argc, char** argv) {
   if (argc < 7) {
-    fprintf(stderr, "usage: %s WEIGHTS IMAGES B H W OUT [ITERS]\n", argv[0]);
+    fprintf(stderr, "usage: %s WEIGHTS IMAGES B H W OUT [ITERS [f16]]\n", argv[0]);
     return 2;
   }
   const int B = atoi(argv[3]), H = atoi(argv[4]), W = atoi(argv[5]);
   const int iters = argc > 7 ? atoi(argv[7]) : 100;
+  const bool f16 = argc > 8 && strcmp(argv[8], "f16") == 0;
+  if (argc > 8 && !f16) { fprintf(stderr, "%s: the only precision option is f16\n", argv[8]); return 2; }
+  auto forward = f16 ? snb_stereonet_forward_f16 : snb_stereonet_forward;
+  const char* fwd_name = f16 ? "snb_stereonet_forward_f16" : "snb_stereonet_forward";
 
   // ---- weights file: magic, {k, input_scale, maxdisp, n}, then n x {numel, data}
   std::vector<char> wf;
@@ -111,10 +116,9 @@ int main(int argc, char** argv) {
   cudaGraph_t graph;
   cudaGraphExec_t exec;
   CK(cudaStreamBeginCapture(stream, cudaStreamCaptureModeThreadLocal));
-  const int rc = snb_stereonet_forward(weights, k, input_scale, maxdisp, dimg, B, H, W, workspace, disp, nullptr, nullptr, nullptr,
-                                       stream);
+  const int rc = forward(weights, k, input_scale, maxdisp, dimg, B, H, W, workspace, disp, nullptr, nullptr, nullptr, stream);
   CK(cudaStreamEndCapture(stream, &graph));
-  if (rc != 0) { fprintf(stderr, "snb_stereonet_forward: %s\n", snb_last_error()); return 1; }
+  if (rc != 0) { fprintf(stderr, "%s: %s\n", fwd_name, snb_last_error()); return 1; }
   CK(cudaGraphInstantiate(&exec, graph, 0));
 
   CK(cudaGraphLaunch(exec, stream));                // warm-up
@@ -127,8 +131,8 @@ int main(int argc, char** argv) {
   CK(cudaEventSynchronize(t1));
   float ms = 0.f;
   CK(cudaEventElapsedTime(&ms, t0, t1));
-  printf("stereonet_infer: k=%d input_scale=%d maxdisp=%d B=%d %dx%d: %.3f ms per frame (mean of %d graph replays)\n",
-         k, input_scale, maxdisp, B, H, W, iters > 0 ? ms / iters : 0.f, iters);
+  printf("stereonet_infer: k=%d input_scale=%d maxdisp=%d B=%d %dx%d%s: %.3f ms per frame (mean of %d graph replays)\n",
+         k, input_scale, maxdisp, B, H, W, f16 ? " f16" : "", iters > 0 ? ms / iters : 0.f, iters);
 
   std::vector<float> out((size_t)B * H * W);
   CK(cudaMemcpyAsync(out.data(), disp, out.size() * sizeof(float), cudaMemcpyDeviceToHost, stream));

@@ -120,6 +120,13 @@ SNB_API int snb_conv2d_c32_tc_profile(const float* x, const float* wimg, float* 
 SNB_API int snb_conv_c32_ws(const float* x, const float* wimg, float* y, const snb_conv_geom* g, const snb_conv_epilogue* e,
                     void* stream);
 SNB_API int snb_conv_c32_ws_num_tiles(const snb_conv_geom* g);
+/* Reduced-precision inference variant of snb_conv_c32_ws (same arguments, same weight image, same epilogue): ONE fp16 product per
+ * tap, out = 2^-s (xh . wh) with xh = fp16(x) and wh the high half of the prepared weight, fp32 accumulation.  That is about
+ * 1e-3 relative error per layer, so its results are reported separately from the fp32 parity contract of every other call here.
+ * Inputs below 2^-14 in magnitude are fp16 subnormals and lose relative precision (BatchNorm-normalised activations and cost-volume
+ * differences sit well above that).  Inference only: `stats` must be NULL (rejected by name, nothing launched). */
+SNB_API int snb_conv_c32_ws_f16(const float* x, const float* wimg, float* y, const snb_conv_geom* g, const snb_conv_epilogue* e,
+                        void* stream);
 SNB_API int snb_conv_weights_ws_floats(int kd);      /* kd = 1, 3; 5: the image set of snb_conv5x5s2_c32_ws */
 /* downsample[1:] (nn.Conv2d(32, 32, 5, stride 2, padding 2), stereo_net.py:64-70) in ONE launch of the same kernel: the four
  * polyphase images of the input (snb_phase_split / snb_conv5x5s2_c3 with phases = 1; [4][B][OH][OW][32]) are four raw windows per
@@ -353,6 +360,15 @@ SNB_API long long snb_stereonet_workspace_bytes(int k, int input_scale, int maxd
  * these extents is written.  Independent calls may run concurrently on separate streams with separate workspaces and outputs. */
 SNB_API int snb_stereonet_forward(const void* weights, int k, int input_scale, int maxdisp, const float* images, int B, int H, int W,
                           void* workspace, float* disp, float* coarse, float* cost, float* fcs, void* stream);
+/* Opt-in reduced-precision forward for throughput inference: the same arguments, weights buffer, workspace size and launch sequence
+ * as snb_stereonet_forward, with the 32->32 3x3 layers of the feature extractor and the refinement and the 3x3x3 cost-filter layers
+ * on snb_conv_c32_ws_f16 (one fp16 product per tap instead of the fp32-grade three).  The 5x5 stride-2 layers, the refinement's
+ * input layer, the first layer and the 32->1 heads are unchanged.  Its disparities differ from snb_stereonet_forward's by far more
+ * than the fp32 parity tolerance, so its numbers are reported separately from that contract (DESIGN.md section 4.2f16 lists the
+ * measured errors).  Inputs below 2^-14 in magnitude lose relative precision in fp16 (see snb_conv_c32_ws_f16).  Bit-identical to
+ * stereonet_b200.runtime.StereoEngine(..., precision="fp16"). */
+SNB_API int snb_stereonet_forward_f16(const void* weights, int k, int input_scale, int maxdisp, const float* images, int B, int H, int W,
+                              void* workspace, float* disp, float* coarse, float* cost, float* fcs, void* stream);
 
 /* ---------------------------------------------------------------------------------------------------------------
  * Whole-model online adaptation, single pass (adapt.py:304-396 without experience replay: the update of the NONE / NONSTOP / VS
