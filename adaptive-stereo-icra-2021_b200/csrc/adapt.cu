@@ -242,7 +242,7 @@ int forward_impl(float* const* params, long long* const* bn_counters, const Dims
     const long long m = ar.mark(), npos = (long long)g.B * g.D * g.H * g.W;
     const int nt = snb_conv_c32_ws_num_tiles(&g);
     float* stats = ar.take((long long)nt * 64);
-    float* scratch = ar.take(64 * 64);
+    double* scratch = reinterpret_cast<double*>(ar.take(2 * 64 * 64));      // 64 x 64 doubles
     snb_conv_epilogue e = {P(ti + 1), nullptr, nullptr, nullptr, stats, 0};
     RUN(snb_conv_c32_ws(x, IMGF(ti), z, &g, &e, stream));
     RUN(snb_bn_finalize_ws(stats, nt, npos, P(ti + 2), P(ti + 3), params[ti + 4], params[ti + 5], nbt, BN_MOMENTUM, BN_EPS,
@@ -299,7 +299,7 @@ int forward_impl(float* const* params, long long* const* bn_counters, const Dims
       const long long m = ar.mark();
       const int nt = snb_refine_in_conv_num_tiles(B, H, W);
       float* stats = ar.take((long long)nt * 64);
-      float* scratch = ar.take(64 * 64);
+      double* scratch = reinterpret_cast<double*>(ar.take(2 * 64 * 64));      // 64 x 64 doubles
       snb_conv_epilogue e = {P(r0 + 1), nullptr, nullptr, nullptr, stats, 0};
       RUN(snb_refine_in_conv(sv.pred, left, P(r0), sv.up, sv.zr[0], B, h, w, H, W, mul, &e, stream));
       RUN(snb_bn_finalize_ws(stats, nt, B * HW, P(r0 + 2), P(r0 + 3), params[r0 + 4], params[r0 + 5], counter(10), BN_MOMENTUM, BN_EPS,

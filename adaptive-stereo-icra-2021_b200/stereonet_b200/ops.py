@@ -423,7 +423,7 @@ def bn_finalize(stats, count, bn, update_running=True):
   out = torch.empty((4, 32), device=dev, dtype=torch.float32)
   rm = bn.running_mean if update_running else None
   rv = bn.running_var if update_running else None
-  scratch = torch.empty((64, 64), device=dev, dtype=torch.float32)
+  scratch = torch.empty((64, 64), device=dev, dtype=torch.float64)
   nbt = bn.num_batches_tracked if (update_running and bn.num_batches_tracked is not None) else None   # += 1 in the same launch
   check(_cabi.lib().snb_bn_finalize_ws(_p(stats), stats.shape[0], int(count), _p(bn.weight.detach()), _p(bn.bias.detach()),
                                        _p(rm), _p(rv), _p(nbt), BN_MOMENTUM, BN_EPS, _p(out[0]), _p(out[1]), _p(out[2]), _p(out[3]),

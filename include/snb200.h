@@ -219,12 +219,12 @@ SNB_API int snb_upsample_bilinear_bwd(const float* dout, float* din, int B, int 
 SNB_API int snb_bn_finalize(const float* stats, int ntiles, long long count, const float* gamma, const float* beta,
                     float* running_mean, float* running_var, float momentum, float eps,
                     float* scale, float* shift, float* mean, float* invstd, void* stream);
-/* Same, with a caller-provided scratch of 64 x 64 floats: more than 256 partial rows are first reduced by 64 CTAs (a single
- * CTA walking ~1 MB of partials is bound by one SM's load bandwidth).  num_batches_tracked (nn.BatchNorm's int64 counter, or
+/* Same, with a caller-provided scratch of 64 x 64 doubles: more than 256 partial rows are first reduced by 64 CTAs (a single
+ * CTA walking ~1 MB of partials is bound by one SM's load bandwidth) into fp64 chunk sums.  num_batches_tracked (nn.BatchNorm's int64 counter, or
  * NULL) is incremented by the same launch when the running statistics are updated. */
 SNB_API int snb_bn_finalize_ws(const float* stats, int ntiles, long long count, const float* gamma, const float* beta,
                        float* running_mean, float* running_var, long long* num_batches_tracked, float momentum, float eps,
-                       float* scale, float* shift, float* mean, float* invstd, float* scratch, void* stream);
+                       float* scale, float* shift, float* mean, float* invstd, double* scratch, void* stream);
 /* The running-statistics half of snb_bn_finalize[_ws] for a call that was made WITHOUT running buffers: running = (1 - m) running
  * + m batch statistic (unbiased variance from invstd), num_batches_tracked += 1.  Lets the left / right feature passes of one
  * adaptation step (adapt.py:72) run on two streams and still update nn.BatchNorm's buffers in the reference's order. */
