@@ -190,8 +190,10 @@ photo_loss_tile_kernel(const float* __restrict__ left, const float* __restrict__
       gi += mk * (0.15f / 3.f) * (df > 0.f ? 1.f : (df < 0.f ? -1.f : 0.f));
       g = fmaf(gi, sDI[c * TH * TW + i], g);
     }
-    // edge-aware smoothness on dn = d / (mean + eps)   (loss_functions.py:64-75,106-138)
-    const float dn = sD[c2] * inv_m;
+    // edge-aware smoothness on dn = d / (mean + eps)   (loss_functions.py:64-75,106-138).  Each difference of dn is taken as
+    // (d_a - d_b) * inv_m: its sign is exact and it is 0 exactly where d_a == d_b, as in the reference.  (d_a * inv_m -
+    // d_b * inv_m contracts to an FMA that leaves the rounding error of d_a * inv_m, of either sign, for equal disparities.)
+    const float d0 = sD[c2];
     float sval = 0.f, h = 0.f;
     auto edge = [&](int q2a, int q2b) {           // exp(-mean_c |L(a) - L(b)|)
       const float e0 = fabsf(sL[q2a] - sL[q2b]), e1 = fabsf(sL[R2H * R2W + q2a] - sL[R2H * R2W + q2b]),
@@ -199,10 +201,10 @@ photo_loss_tile_kernel(const float* __restrict__ left, const float* __restrict__
       return __expf(-(e0 + e1 + e2) * (1.f / 3.f));
     };
     auto sgn = [](float v) { return v > 0.f ? 1.f : (v < 0.f ? -1.f : 0.f); };
-    if (x + 1 < W) { const float df = dn - sD[c2 + 1] * inv_m; const float ex = edge(c2, c2 + 1); sval += fabsf(df) * ex; h += mk * sgn(df) * ex; }
-    if (y + 1 < H) { const float df = dn - sD[c2 + R2W] * inv_m; const float ey = edge(c2, c2 + R2W); sval += fabsf(df) * ey; h += mk * sgn(df) * ey; }
-    if (x >= 1) { const float df = sD[c2 - 1] * inv_m - dn; h -= sM[c2 - 1] * sgn(df) * edge(c2 - 1, c2); }
-    if (y >= 1) { const float df = sD[c2 - R2W] * inv_m - dn; h -= sM[c2 - R2W] * sgn(df) * edge(c2 - R2W, c2); }
+    if (x + 1 < W) { const float df = (d0 - sD[c2 + 1]) * inv_m; const float ex = edge(c2, c2 + 1); sval += fabsf(df) * ex; h += mk * sgn(df) * ex; }
+    if (y + 1 < H) { const float df = (d0 - sD[c2 + R2W]) * inv_m; const float ey = edge(c2, c2 + R2W); sval += fabsf(df) * ey; h += mk * sgn(df) * ey; }
+    if (x >= 1) { const float df = (sD[c2 - 1] - d0) * inv_m; h -= sM[c2 - 1] * sgn(df) * edge(c2 - 1, c2); }
+    if (y >= 1) { const float df = (sD[c2 - R2W] - d0) * inv_m; h -= sM[c2 - R2W] * sgn(df) * edge(c2 - R2W, c2); }
     loss_acc += (double)(mk * smooth_w * sval);
     t_acc += (double)(smooth_w * h * sD[c2]);
     g_out[(size_t)b * HW + y * W + x] = g + smooth_w * h * inv_m;
@@ -225,8 +227,8 @@ photo_loss_tile_kernel(const float* __restrict__ left, const float* __restrict__
   }
 }
 
-// loss = sum / count;  ddisp = (g - T_b / ((m_b + eps)^2 HW)) / count.  Every block re-reduces the (few hundred) partials in the
-// same fixed order, so the result is deterministic and needs no extra launch.
+// loss = sum / count;  ddisp = (g - T_b / ((m_b + eps)^2 HW)) / count (0 when count is 0).  Every block re-reduces the (few
+// hundred) partials in the same fixed order, so the result is deterministic and needs no extra launch.
 __global__ void __launch_bounds__(256)
 photo_loss_finalize_kernel(const float* __restrict__ part, const float* __restrict__ dsum_part, float* __restrict__ g,
                            float* __restrict__ loss_out, int B, int HW, int blocks_per_batch) {
@@ -249,7 +251,9 @@ photo_loss_finalize_kernel(const float* __restrict__ part, const float* __restri
     __syncthreads();
   }
   const double cnt = sh[1];
-  const float inv_cnt = (float)(1.0 / cnt);
+  // an empty mask: the reference's total[mask].mean() is NaN with an all-zero gradient, so the loss stays 0/0 and the
+  // gradient scale is 0 (every g and the coupling are 0 there; 1/0 would turn them into NaN)
+  const float inv_cnt = cnt > 0.0 ? (float)(1.0 / cnt) : 0.f;
   const float m_eps = mean_disp(dsum_part, b, HW) + 1e-7f;
   const float coupling = (float)(sh[2] / ((double)m_eps * (double)m_eps * (double)HW));
   if (blockIdx.x == 0 && b == 0 && t == 0) loss_out[0] = (float)(sh[0] / cnt);
