@@ -2,7 +2,9 @@
 
 --example also builds examples/stereonet_infer.cpp (the torch-free whole-model host, include/snb200.h) with the same nvcc flags,
 linked against libsnb200.so; OUT defaults to build/stereonet_infer next to this file.  examples/stereonet_adapt.cpp (the torch-free
-adaptation host) is built next to it as stereonet_adapt."""
+adaptation host) is built next to it as stereonet_adapt, and examples/stereonet_adapt_dp.cpp (the torch-free multi-GPU data-parallel
+host) as stereonet_adapt_dp when NCCL is installed (the nvidia.nccl package that comes with torch; without it that one example is
+skipped with a message)."""
 import glob
 import os
 import subprocess
@@ -59,14 +61,35 @@ def build(force=False, verbose=False):
 EXAMPLES = os.path.join(HERE, "..", "examples")
 
 
+def find_nccl():
+  """(include dir, library file) of the NCCL that the nvidia.nccl package installs, or None."""
+  try:
+    import nvidia.nccl
+  except ImportError:
+    return None
+  for d in nvidia.nccl.__path__:
+    inc, libs = os.path.join(d, "include"), sorted(glob.glob(os.path.join(d, "lib", "libnccl.so*")))
+    if os.path.exists(os.path.join(inc, "nccl.h")) and libs:
+      return inc, libs[0]
+  return None
+
+
 def build_example(out=None, name="stereonet_infer"):
-  """examples/<name>.cpp -> `out` (default build/<name>), linked against (and with an rpath to) libsnb200.so."""
+  """examples/<name>.cpp -> `out` (default build/<name>), linked against (and with an rpath to) libsnb200.so; stereonet_adapt_dp
+  also against NCCL (RuntimeError if find_nccl() finds none)."""
   lib = build()
   out = out or os.path.join(HERE, "build", name)
   os.makedirs(os.path.dirname(os.path.abspath(out)), exist_ok=True)
   libdir = os.path.dirname(lib)
   cmd = ([NVCC] + FLAGS + ["-I", os.path.join(HERE, "..", "include"), os.path.join(EXAMPLES, name + ".cpp"), "-o", out,
                            "-L" + libdir, "-lsnb200", "-Xlinker", "-rpath=" + libdir])
+  if name == "stereonet_adapt_dp":
+    nccl = find_nccl()
+    if nccl is None:
+      raise RuntimeError("stereonet_adapt_dp needs NCCL: no nccl.h / libnccl.so in the nvidia.nccl package")
+    inc, so = nccl
+    cmd += ["-I", inc, "-Xlinker", "-l:" + os.path.basename(so), "-L" + os.path.dirname(so),
+            "-Xlinker", "-rpath=" + os.path.dirname(so)]
   subprocess.check_call(cmd)
   return out
 
@@ -78,3 +101,8 @@ if __name__ == "__main__":
     nxt = sys.argv[i + 1] if i + 1 < len(sys.argv) and not sys.argv[i + 1].startswith("-") else None
     print(build_example(nxt))
     print(build_example(os.path.join(os.path.dirname(os.path.abspath(nxt)), "stereonet_adapt") if nxt else None, "stereonet_adapt"))
+    if find_nccl() is None:
+      print("stereonet_adapt_dp: skipped (NCCL not found: no nvidia.nccl package with nccl.h and libnccl.so)")
+    else:
+      print(build_example(os.path.join(os.path.dirname(os.path.abspath(nxt)), "stereonet_adapt_dp") if nxt else None,
+                          "stereonet_adapt_dp"))

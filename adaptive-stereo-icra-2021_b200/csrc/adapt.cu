@@ -5,11 +5,15 @@
 // the total) and differentiate both passes.  All issue the launch sequence of the Python step AdaptStepper(..., FusedAdamClip,
 // two_streams=False) with gradients enabled (autograd/functions.py forward + backward) through the same launchers, so both sides
 // agree bit for bit; tests/test_gpu_native_adapt.py and tests/test_gpu_native_adapt_replay.py hold them to it.
+// For shared-model data parallelism the update also comes in two halves around the host's all-reduce: snb_stereonet_adapt_backward
+// (the update's backward and pack, plus a copy of the BatchNorm running statistics next to the bucket) and snb_stereonet_adapt_apply
+// (statistics * 1 / world back into the parameters, clip + Adam with grad_scale 1 / world), the three stages of
+// AdaptStepper.step(..., dp_bucket=parallel.DPBucket(...)); tests/test_gpu_native_adapt_dp.py.
 //
-// Four small kernels are new here: the gradient pack (layout moves + the sum of the per-pass, per-side gradients in autograd's
+// Five small kernels are new here: the gradient pack (layout moves + the sum of the per-pass, per-side gradients in autograd's
 // order into the bucket, one launch per 64 tensors), the scaling of the replay loss gradient with the total loss, the fixed-order
-// mean of the feature-contrast map, and the writer of Adam's chunk table.  Every table travels as a kernel parameter: no
-// allocation, no synchronisation, no host-to-device copy.
+// mean of the feature-contrast map, the writer of Adam's chunk table and the scatter of the all-reduced statistics.  Every table
+// travels as a kernel parameter: no allocation, no synchronisation, no host-to-device copy.
 #include <cmath>
 #include <mutex>
 #include <unordered_map>
@@ -84,17 +88,35 @@ __global__ void chunk_table_kernel(const __grid_constant__ ChunkTable t, long lo
   }
 }
 
+// The running statistics after the all-reduce: dst = fl(src[off..off + n) * scale), one CTA per tensor (torch's
+// stats.mul_(1.0 / world) on the float32 statistics, written back to the module buffers).
+struct StatItem { float* dst; int off, n; };
+constexpr int STAT_MAX = 64;
+struct StatTable { StatItem it[STAT_MAX]; int n; };
+static_assert(sizeof(StatTable) <= 4096, "kernel parameter block");
+
+__global__ void __launch_bounds__(64) stats_scatter_kernel(const __grid_constant__ StatTable t, const float* __restrict__ src,
+                                                           float scale) {
+  pdl_launch(); pdl_wait();
+  const StatItem& e = t.it[blockIdx.x];
+  for (int i = threadIdx.x; i < e.n; i += blockDim.x) e.dst[i] = __fmul_rn(src[e.off + i], scale);
+}
+
 // ------------------------------------------------------------------------------------------------ state
 constexpr int N_BN = 17;                   // BatchNorm layers the step trains, module order
 constexpr float BN_MOMENTUM = 0.1f, BN_EPS = 1e-5f, SMOOTH_W = 1e-3f;
 
+// The bucket is followed, without padding, by the running statistics of the trained BatchNorm layers (running_mean, then
+// running_var, per layer in parallel.used_bn_buffers order): [bucket | statistics] is the span a data-parallel host all-reduces,
+// laid out as parallel.DPBucket.flat.
 struct StateLayout {
   std::vector<Tensor> t;
   std::vector<long long> slot;             // per tensor: element offset in the bucket, -1 for the running statistics
+  std::vector<int> stat_idx;               // tensors of the statistics piece, in its order
   std::vector<long long> img_f, img_b;     // per tensor: byte offsets of the forward / data-gradient weight images, -1 if none
   long long img_b_stride = 0;              // between the four phase images of a 5x5 stride-2 layer
-  long long n_total = 0, n_clip = 0;
-  long long grad, m, v, step, adam_ws, table, wflip, total;
+  long long n_total = 0, n_clip = 0, n_stats = 0;
+  long long grad, stats, m, v, step, adam_ws, table, wflip, total;
   int nchunks = 0, nused = 0;
 };
 
@@ -106,7 +128,11 @@ StateLayout state_layout(int k) {
   long long off = 0;
   for (int pass = 0; pass < 2; ++pass)     // FusedAdamClip's order: stereo_net, then feature_net; parameters only
     for (int i = pass == 0 ? s0 : 0; i < (pass == 0 ? n : s0); ++i) {
-      if (L.t[i].role == R_NONE) continue;
+      if (L.t[i].role == R_NONE) {
+        L.stat_idx.push_back(i);           // used_bn_buffers' order: the same walk
+        L.n_stats += L.t[i].numel;
+        continue;
+      }
       L.slot[i] = off;
       off += L.t[i].numel;
       L.nchunks += (L.t[i].numel + 1023) / 1024;
@@ -116,7 +142,9 @@ StateLayout state_layout(int k) {
   L.n_total = off;
   long long b = 0;
   auto take = [&](long long bytes) { const long long o = b; b += align_up(bytes); return o; };
-  L.grad = take(L.n_total * 4); L.m = take(L.n_total * 4); L.v = take(L.n_total * 4); L.step = take(4);
+  L.grad = take((L.n_total + L.n_stats) * 4);
+  L.stats = L.grad + L.n_total * 4;
+  L.m = take(L.n_total * 4); L.v = take(L.n_total * 4); L.step = take(4);
   L.adam_ws = take(snb_adam_clip_workspace_bytes());
   L.table = take(L.nchunks * 24ll);
   const long long ws1 = snb_conv_weights_ws_floats(1) * 4ll;
@@ -365,9 +393,10 @@ int accumulation_rank(int pass, int side, int npass) { return (npass - 1 - pass)
 // bucket), then scratch, released phase by phase (refinement, stereo head, each feature pass) and pass by pass.  The high-water mark
 // is the refinement phase: four full-resolution buffers (dres and three 32-channel gradients, ~180 MB at KITTI) on top of the Saved
 // blocks; the forward needs less.  `dr`: the replay pass's dims, or NULL.  `bytes` / `grad_bytes` (measuring run): total size and
-// the size of the gradient region.
-int update_impl(float* const* params, const Dims& d, const Dims* dr, char* state, uintptr_t workspace, float max_norm, double lr,
-                double beta1, double beta2, double eps, void* stream, long long* bytes, long long* grad_bytes) {
+// the size of the gradient region.  Ends with the bucket packed; `stats` also copies the running statistics into their piece
+// (snb_stereonet_adapt_backward), in the same pack launches.
+int backward_impl(float* const* params, const Dims& d, const Dims* dr, char* state, uintptr_t workspace, bool stats, void* stream,
+                  long long* bytes, long long* grad_bytes) {
   const bool dry = workspace == 0;
   const StateLayout L = state_layout(d.k);
   Arena ar{workspace};
@@ -376,7 +405,7 @@ int update_impl(float* const* params, const Dims& d, const Dims* dr, char* state
   long long gsize = 0;
   if (!dry) {
     long long total = 0;
-    if (int rc = update_impl(nullptr, d, dr, nullptr, 0, 0.f, 0.0, 0.0, 0.0, 0.0, nullptr, &total, &gsize)) return rc;
+    if (int rc = backward_impl(nullptr, d, dr, nullptr, 0, false, nullptr, &total, &gsize)) return rc;
   }
   Arena ga{dry ? 0 : workspace + ar.off};                         // gradients
   ar.off += gsize;
@@ -599,7 +628,7 @@ int update_impl(float* const* params, const Dims& d, const Dims* dr, char* state
     return 0;
   }
 
-  // ---- the bucket (FusedAdamClip.pack: every pass's gradients summed as autograd accumulates them), then clip + Adam
+  // ---- the bucket (FusedAdamClip.pack: every pass's gradients summed as autograd accumulates them) [, the running statistics]
   float* grad = reinterpret_cast<float*>(state + L.grad);
   std::vector<PackItem> items;
   for (size_t i = 0; i < L.t.size(); ++i) {
@@ -612,6 +641,13 @@ int update_impl(float* const* params, const Dims& d, const Dims* dr, char* state
     if (n) { it.rows = s.rows; it.cols = s.cols; it.rs = s.rs; it.cs = s.cs; }
     items.push_back(it);
   }
+  if (stats) {
+    float* dst = reinterpret_cast<float*>(state + L.stats);
+    for (const int i : L.stat_idx) {
+      items.push_back(PackItem{{params[i], nullptr, nullptr, nullptr}, dst, 1, L.t[i].numel, 0, 1});
+      dst += L.t[i].numel;
+    }
+  }
   for (size_t base = 0; base < items.size(); base += PACK_MAX) {
     PackTable t;
     t.n = (int)(items.size() - base < (size_t)PACK_MAX ? items.size() - base : PACK_MAX);
@@ -623,12 +659,25 @@ int update_impl(float* const* params, const Dims& d, const Dims* dr, char* state
     snb_launch(grad_pack_kernel, dim3(snb_ceil_div(mx, 2048), t.n), 256, 0, stream, t);
     SNB_LAUNCH_CHECK("grad_pack_kernel");
   }
-  return snb_adam_clip_step(reinterpret_cast<const long long*>(state + L.table), L.nchunks, grad, reinterpret_cast<float*>(state + L.m),
-                            reinterpret_cast<float*>(state + L.v), reinterpret_cast<float*>(state + L.step), L.n_total, L.n_clip,
-                            max_norm, 1.f, lr, beta1, beta2, eps, state + L.adam_ws, stream);
+  return 0;
 }
 
 #undef RUN
+
+// clip + Adam over the bucket (FusedAdamClip.step); grad_scale 1 / world after a data-parallel all-reduce.
+int adam_step(const StateLayout& L, char* state, float max_norm, float grad_scale, double lr, double beta1, double beta2, double eps,
+              void* stream) {
+  return snb_adam_clip_step(reinterpret_cast<const long long*>(state + L.table), L.nchunks, reinterpret_cast<const float*>(state + L.grad),
+                            reinterpret_cast<float*>(state + L.m), reinterpret_cast<float*>(state + L.v),
+                            reinterpret_cast<float*>(state + L.step), L.n_total, L.n_clip, max_norm, grad_scale, lr, beta1, beta2, eps,
+                            state + L.adam_ws, stream);
+}
+
+int update_impl(float* const* params, const Dims& d, const Dims* dr, char* state, uintptr_t workspace, float max_norm, double lr,
+                double beta1, double beta2, double eps, void* stream) {
+  if (int rc = backward_impl(params, d, dr, state, workspace, false, stream, nullptr, nullptr)) return rc;
+  return adam_step(state_layout(d.k), state, max_norm, 1.f, lr, beta1, beta2, eps, stream);
+}
 
 // What the last forward on each workspace was called with, so that its update can reject other arguments before launching
 // anything (an update with a larger shape than its forward's would write past a workspace sized for the forward).  Host-side and
@@ -670,6 +719,38 @@ int check_against_forward(const char* who, float* const* params, const Dims& d, 
   return 0;
 }
 
+// What snb_stereonet_adapt_backward last packed into each state, so that snb_stereonet_adapt_apply can reject, before launching
+// anything, a state whose bucket holds no fresh gradients (no backward, or already applied or updated) and parameters other than
+// the ones the statistics came from.  Host-side and keyed by the state address, like ForwardRecord.
+struct BackwardRecord {
+  int k;
+  std::vector<const float*> params;
+};
+std::mutex g_backwards_mutex;
+std::unordered_map<uintptr_t, BackwardRecord> g_backwards;
+
+void record_backward(const void* state, BackwardRecord r) {
+  std::lock_guard<std::mutex> lock(g_backwards_mutex);
+  g_backwards[reinterpret_cast<uintptr_t>(state)] = std::move(r);
+}
+
+void forget_backward(const void* state) {
+  std::lock_guard<std::mutex> lock(g_backwards_mutex);
+  g_backwards.erase(reinterpret_cast<uintptr_t>(state));
+}
+
+int check_against_backward(const char* who, float* const* params, int k, const void* state) {
+  std::lock_guard<std::mutex> lock(g_backwards_mutex);
+  const auto it = g_backwards.find(reinterpret_cast<uintptr_t>(state));
+  SNB_REQUIRE(it != g_backwards.end(), "%s: no snb_stereonet_adapt_backward or _backward_replay has run on this `state` since its "
+              "last apply or update", who);
+  const BackwardRecord& r = it->second;
+  SNB_REQUIRE(k == r.k, "%s: `k` is %d but the backward on this state ran with %d", who, k, r.k);
+  for (size_t i = 0; i < r.params.size(); ++i)
+    SNB_REQUIRE(params[i] == r.params[i], "%s: `params[%d]` is not the tensor the backward on this state read", who, (int)i);
+  return 0;
+}
+
 int check_params(const char* who, float* const* params, int k) {
   SNB_REQUIRE(params != nullptr, "%s: null `params`", who);
   const int n = 2 * k + 108;
@@ -689,11 +770,13 @@ extern "C" int snb_stereonet_adapt_state_piece(int k, int what, long long* offse
   const char* who = "snb_stereonet_adapt_state_piece";
   SNB_REQUIRE(k >= 1 && k <= 16, "%s: k must be in [1, 16] (got %d)", who, k);
   SNB_REQUIRE(offset && bytes, "%s: null `offset` / `bytes`", who);
-  SNB_REQUIRE(what >= 0 && what <= 3, "%s: `what` must be 0 (flat_grad), 1 (exp_avg), 2 (exp_avg_sq) or 3 (step) (got %d)", who, what);
+  SNB_REQUIRE(what >= 0 && what <= 5, "%s: `what` must be 0 (flat_grad), 1 (exp_avg), 2 (exp_avg_sq), 3 (step), 4 (bn_stats) or "
+              "5 (dp_flat) (got %d)", who, what);
   const StateLayout L = state_layout(k);
-  const long long offs[4] = {L.grad, L.m, L.v, L.step};
+  const long long offs[6] = {L.grad, L.m, L.v, L.step, L.stats, L.grad};
+  const long long sizes[6] = {L.n_total * 4, L.n_total * 4, L.n_total * 4, 4, L.n_stats * 4, (L.n_total + L.n_stats) * 4};
   *offset = offs[what];
-  *bytes = what == 3 ? 4 : L.n_total * 4;
+  *bytes = sizes[what];
   return 0;
 }
 
@@ -742,7 +825,7 @@ long long workspace_bytes(const char* who, int k, int input_scale, int maxdisp, 
   long long f = 0, u = 0;
   float dummy = 0.f;
   if (forward_impl(nullptr, nullptr, d, nullptr, rp, nullptr, 0, &dummy, nullptr, nullptr, nullptr, nullptr, &f)) return -1;
-  if (update_impl(nullptr, d, RB ? &dr : nullptr, nullptr, 0, 0.f, 0.0, 0.0, 0.0, 0.0, nullptr, &u, nullptr)) return -1;
+  if (backward_impl(nullptr, d, RB ? &dr : nullptr, nullptr, 0, false, nullptr, &u, nullptr)) return -1;
   return f > u ? f : u;
 }
 
@@ -783,14 +866,21 @@ int check_forward(const char* who, float* const* params, long long* const* bn_co
   return 0;
 }
 
+int check_adam(const char* who, double lr, double beta1, double beta2, double eps) {
+  SNB_REQUIRE(lr >= 0.0 && beta1 >= 0.0 && beta1 < 1.0 && beta2 >= 0.0 && beta2 < 1.0 && eps >= 0.0,
+              "%s: `beta1` and `beta2` must be in [0, 1), `lr` and `eps` >= 0 (got %g, %g, %g, %g)", who, beta1, beta2, lr, eps);
+  return 0;
+}
+
+// The argument checks of the updates and the backward calls (adam: an update, whose optimizer arguments are checked too).
 int check_update(const char* who, float* const* params, int k, int input_scale, int maxdisp, int B, int H, int W, int RB, void* state,
-                 void* workspace, double lr, double beta1, double beta2, double eps, Dims& d) {
+                 void* workspace, bool adam, double lr, double beta1, double beta2, double eps, Dims& d) {
   if (int rc = check_dims(who, k, input_scale, maxdisp, B, H, W, d)) return rc;
   if (int rc = check_params(who, params, k)) return rc;
   SNB_REQUIRE(state != nullptr && aligned(state, ALIGN), "%s: `state` must be a non-null 256-byte aligned pointer", who);
   SNB_REQUIRE(workspace != nullptr && aligned(workspace, ALIGN), "%s: `workspace` must be a non-null 256-byte aligned pointer", who);
-  SNB_REQUIRE(lr >= 0.0 && beta1 >= 0.0 && beta1 < 1.0 && beta2 >= 0.0 && beta2 < 1.0 && eps >= 0.0,
-              "%s: `beta1` and `beta2` must be in [0, 1), `lr` and `eps` >= 0 (got %g, %g, %g, %g)", who, beta1, beta2, lr, eps);
+  if (adam)
+    if (int rc = check_adam(who, lr, beta1, beta2, eps)) return rc;
   return check_against_forward(who, params, d, maxdisp, RB, state, workspace);
 }
 
@@ -835,10 +925,11 @@ extern "C" int snb_stereonet_adapt_update(float* const* params, int k, int input
                                           void* workspace, float max_norm, double lr, double beta1, double beta2, double eps,
                                           void* stream) {
   Dims d;
-  if (int rc = check_update("snb_stereonet_adapt_update", params, k, input_scale, maxdisp, B, H, W, 0, state, workspace, lr, beta1, beta2,
-                            eps, d)) return rc;
+  if (int rc = check_update("snb_stereonet_adapt_update", params, k, input_scale, maxdisp, B, H, W, 0, state, workspace, true, lr, beta1,
+                            beta2, eps, d)) return rc;
+  forget_backward(state);                                         // the bucket now holds this update's gradients, applied
   return update_impl(params, d, nullptr, static_cast<char*>(state), reinterpret_cast<uintptr_t>(workspace), max_norm, lr, beta1, beta2,
-                     eps, stream, nullptr, nullptr);
+                     eps, stream);
 }
 
 extern "C" int snb_stereonet_adapt_update_replay(float* const* params, int k, int input_scale, int maxdisp, int B, int H, int W, int RB,
@@ -847,8 +938,63 @@ extern "C" int snb_stereonet_adapt_update_replay(float* const* params, int k, in
   const char* who = "snb_stereonet_adapt_update_replay";
   SNB_REQUIRE(RB >= 1, "%s: `RB` must be >= 1 (got %d)", who, RB);
   Dims d;
-  if (int rc = check_update(who, params, k, input_scale, maxdisp, B, H, W, RB, state, workspace, lr, beta1, beta2, eps, d)) return rc;
+  if (int rc = check_update(who, params, k, input_scale, maxdisp, B, H, W, RB, state, workspace, true, lr, beta1, beta2, eps, d))
+    return rc;
+  forget_backward(state);
   const Dims dr = replay_dims(d, RB);
   return update_impl(params, d, &dr, static_cast<char*>(state), reinterpret_cast<uintptr_t>(workspace), max_norm, lr, beta1, beta2, eps,
-                     stream, nullptr, nullptr);
+                     stream);
+}
+
+namespace {
+
+int backward_entry(const char* who, float* const* params, int k, int input_scale, int maxdisp, int B, int H, int W, int RB, void* state,
+                   void* workspace, void* stream) {
+  Dims d;
+  if (int rc = check_update(who, params, k, input_scale, maxdisp, B, H, W, RB, state, workspace, false, 0.0, 0.0, 0.0, 0.0, d))
+    return rc;
+  const Dims dr = replay_dims(d, RB);
+  if (int rc = backward_impl(params, d, RB ? &dr : nullptr, static_cast<char*>(state), reinterpret_cast<uintptr_t>(workspace), true,
+                             stream, nullptr, nullptr)) return rc;
+  record_backward(state, BackwardRecord{k, std::vector<const float*>(params, params + 2 * k + 108)});
+  return 0;
+}
+
+}  // namespace
+
+extern "C" int snb_stereonet_adapt_backward(float* const* params, int k, int input_scale, int maxdisp, int B, int H, int W, void* state,
+                                            void* workspace, void* stream) {
+  return backward_entry("snb_stereonet_adapt_backward", params, k, input_scale, maxdisp, B, H, W, 0, state, workspace, stream);
+}
+
+extern "C" int snb_stereonet_adapt_backward_replay(float* const* params, int k, int input_scale, int maxdisp, int B, int H, int W, int RB,
+                                                   void* state, void* workspace, void* stream) {
+  const char* who = "snb_stereonet_adapt_backward_replay";
+  SNB_REQUIRE(RB >= 1, "%s: `RB` must be >= 1 (got %d)", who, RB);
+  return backward_entry(who, params, k, input_scale, maxdisp, B, H, W, RB, state, workspace, stream);
+}
+
+extern "C" int snb_stereonet_adapt_apply(float* const* params, int k, void* state, int world, float max_norm, double lr, double beta1,
+                                         double beta2, double eps, void* stream) {
+  const char* who = "snb_stereonet_adapt_apply";
+  SNB_REQUIRE(k >= 1 && k <= 16, "%s: k must be in [1, 16] (got %d)", who, k);
+  if (int rc = check_params(who, params, k)) return rc;
+  SNB_REQUIRE(state != nullptr && aligned(state, ALIGN), "%s: `state` must be a non-null 256-byte aligned pointer", who);
+  SNB_REQUIRE(world >= 1, "%s: `world` must be >= 1 (got %d)", who, world);
+  if (int rc = check_adam(who, lr, beta1, beta2, eps)) return rc;
+  if (int rc = check_against_backward(who, params, k, state)) return rc;
+  forget_backward(state);
+  const StateLayout L = state_layout(k);
+  char* st = static_cast<char*>(state);
+  const float scale = (float)(1.0 / world);
+  StatTable t;
+  t.n = 0;
+  int off = 0;
+  for (const int i : L.stat_idx) {
+    t.it[t.n++] = StatItem{params[i], off, L.t[i].numel};
+    off += L.t[i].numel;
+  }
+  snb_launch(stats_scatter_kernel, t.n, 64, 0, stream, t, reinterpret_cast<const float*>(st + L.stats), scale);
+  SNB_LAUNCH_CHECK("stats_scatter_kernel");
+  return adam_step(L, st, max_norm, scale, lr, beta1, beta2, eps, stream);
 }

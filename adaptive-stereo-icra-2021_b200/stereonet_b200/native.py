@@ -2,7 +2,8 @@
 snb_stereonet_prepare, and a weights file such a host can read without Python or torch (examples/stereonet_infer.cpp).
 Python users keep runtime.StereoEngine; this module adds no inference wrapper.  NativeAdapt drives the adaptation step
 (snb_stereonet_adapt_*: single pass, or with an experience-replay pass) on a pair of modules and converts its Adam state to and from
-optim.FusedAdamClip.
+optim.FusedAdamClip; for shared-model data parallelism it splits the update into backward() and apply(world) around an all-reduce of
+`dp_flat`.
 
 Parameter order (param_names): the tensors the eval forward reads, in the reference's state_dict order, feature_net first and
 stereo_net second; BasicBlock.conv2.* (constructed, never run) and num_batches_tracked are left out.  2k + 108 tensors.
@@ -79,7 +80,8 @@ def bn_counters(feature_net, stereo_net):
 
 class NativeAdapt:
   """State, workspace and pointer arrays of the native adaptation step on (feature_net, stereo_net), whose tensors it updates in
-  place.  `flat_grad`, `exp_avg`, `exp_avg_sq` and `step` are views of the state, laid out as optim.FusedAdamClip's buffers."""
+  place.  `flat_grad`, `exp_avg`, `exp_avg_sq` and `step` are views of the state, laid out as optim.FusedAdamClip's buffers;
+  `bn_stats` holds the running statistics backward() copies and `dp_flat` is [flat_grad | bn_stats], laid out as parallel.DPBucket.flat."""
 
   def __init__(self, feature_net, stereo_net, lr=5e-5, betas=(0.9, 0.999), eps=1e-8, clip_norm=1.0):
     self.f, self.s, self.k = feature_net, stereo_net, feature_net.k
@@ -90,11 +92,11 @@ class NativeAdapt:
     dev = next(feature_net.parameters()).device
     self.state = torch.empty((lib.snb_stereonet_adapt_state_bytes(self.k),), device=dev, dtype=torch.uint8)
     views = []
-    for what in range(4):
+    for what in range(6):
       off, nb = C.c_longlong(), C.c_longlong()
       _cabi.check(lib.snb_stereonet_adapt_state_piece(self.k, what, C.byref(off), C.byref(nb)), "snb_stereonet_adapt_state_piece")
       views.append(self.state[off.value:off.value + nb.value].view(torch.float32))
-    self.flat_grad, self.exp_avg, self.exp_avg_sq, self.step_t = views
+    self.flat_grad, self.exp_avg, self.exp_avg_sq, self.step_t, self.bn_stats, self.dp_flat = views
     self._ws, self._last = {}, None
     _cabi.check(lib.snb_stereonet_adapt_init(self.params, self.k, self.state.data_ptr(), _stream(dev)), "snb_stereonet_adapt_init")
 
@@ -156,20 +158,52 @@ class NativeAdapt:
         loss_replay.data_ptr(), p(disp), p(fcs), p(fcs_mean), st), "snb_stereonet_adapt_forward_replay")
     self._last = (B, H, W, RB)
 
-  def update(self):
-    """Backward of the last forward (both passes after a replay forward), clip + Adam."""
+  def update(self, dp_group=None):
+    """Backward of the last forward (both passes after a replay forward), clip + Adam.  With `dp_group` (a torch.distributed
+    group, e.g. dist.group.WORLD): backward(), a SUM all-reduce of dp_flat over the group, apply(world) — the shared-model
+    data-parallel step of AdaptStepper.step(..., dp_bucket=parallel.DPBucket(...))."""
+    if dp_group is not None:
+      import torch.distributed as dist
+      self.backward()
+      dist.all_reduce(self.dp_flat, op=dist.ReduceOp.SUM, group=dp_group)
+      self.apply(dist.get_world_size(dp_group))
+      return
     if self._last is None:
       raise RuntimeError("stereonet_b200: NativeAdapt.update() needs a forward() first")
     B, H, W, RB = self._last
     lib = _cabi.lib()
-    common = (self.state.data_ptr(), self.workspace(B, H, W, RB).data_ptr(), float(self.clip_norm) if self.clip_norm else 0.0,
-              self.lr, self.betas[0], self.betas[1], self.eps, _stream(self.state.device))
+    common = (self.state.data_ptr(), self.workspace(B, H, W, RB).data_ptr(), self._max_norm(), self.lr, self.betas[0], self.betas[1],
+              self.eps, _stream(self.state.device))
     if RB:
       _cabi.check(lib.snb_stereonet_adapt_update_replay(self.params, self.k, self.s.input_scale, self.s.maxdisp, B, H, W, RB, *common),
                   "snb_stereonet_adapt_update_replay")
     else:
       _cabi.check(lib.snb_stereonet_adapt_update(self.params, self.k, self.s.input_scale, self.s.maxdisp, B, H, W, *common),
                   "snb_stereonet_adapt_update")
+
+  def backward(self):
+    """Gradients of the last forward into flat_grad (no clip, no Adam) and the running statistics into bn_stats."""
+    if self._last is None:
+      raise RuntimeError("stereonet_b200: NativeAdapt.backward() needs a forward() first")
+    B, H, W, RB = self._last
+    lib = _cabi.lib()
+    common = (self.state.data_ptr(), self.workspace(B, H, W, RB).data_ptr(), _stream(self.state.device))
+    if RB:
+      _cabi.check(lib.snb_stereonet_adapt_backward_replay(self.params, self.k, self.s.input_scale, self.s.maxdisp, B, H, W, RB, *common),
+                  "snb_stereonet_adapt_backward_replay")
+    else:
+      _cabi.check(lib.snb_stereonet_adapt_backward(self.params, self.k, self.s.input_scale, self.s.maxdisp, B, H, W, *common),
+                  "snb_stereonet_adapt_backward")
+
+  def apply(self, world=1):
+    """After dp_flat has been SUM-all-reduced over `world` replicas: running statistics = bn_stats / world into the modules, then
+    clip + Adam on flat_grad / world."""
+    _cabi.check(_cabi.lib().snb_stereonet_adapt_apply(self.params, self.k, self.state.data_ptr(), int(world), self._max_norm(), self.lr,
+                                                      self.betas[0], self.betas[1], self.eps, _stream(self.state.device)),
+                "snb_stereonet_adapt_apply")
+
+  def _max_norm(self):
+    return float(self.clip_norm) if self.clip_norm else 0.0
 
   def to_fused(self, opt):
     """Copy the moments and step into an optim.FusedAdamClip of the same modules (same flat layout)."""

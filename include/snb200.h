@@ -393,7 +393,9 @@ SNB_API int snb_stereonet_forward_f16(const void* weights, int k, int input_scal
  * CUDA-graph capturable.
  * --------------------------------------------------------------------------------------------------------------- */
 SNB_API long long snb_stereonet_adapt_state_bytes(int k);
-/* what: 0 flat_grad [n] fp32, 1 exp_avg [n], 2 exp_avg_sq [n], 3 step [1] fp32 (Adam's t); byte offset and size inside `state`. */
+/* what: 0 flat_grad [n] fp32, 1 exp_avg [n], 2 exp_avg_sq [n], 3 step [1] fp32 (Adam's t), 4 bn_stats [1088] fp32 (the running
+ * statistics snb_stereonet_adapt_backward copies, right after flat_grad), 5 dp_flat [n + 1088] fp32 (flat_grad followed by bn_stats:
+ * the span a data-parallel host all-reduces); byte offset and size inside `state`.  Pieces 0 to 3 start 256-byte aligned. */
 SNB_API int snb_stereonet_adapt_state_piece(int k, int what, long long* offset, long long* bytes);
 /* Element offset and count of params[index]'s slot in the bucket (count 0: a running statistic, no slot). */
 SNB_API int snb_stereonet_adapt_grad_slot(int k, int index, long long* offset, long long* count);
@@ -442,6 +444,33 @@ SNB_API int snb_stereonet_adapt_forward_replay(float* const* params, long long* 
 SNB_API int snb_stereonet_adapt_update_replay(float* const* params, int k, int input_scale, int maxdisp, int B, int H, int W, int RB,
                                       void* state, void* workspace, float max_norm, double lr, double beta1, double beta2, double eps,
                                       void* stream);
+
+/* ---------------------------------------------------------------------------------------------------------------
+ * Shared-model data-parallel adaptation (SURVEY.md section 8e, BASELINE.json configs[4]): G replicas of one model, each adapting its
+ * own stream, kept identical by ONE sum all-reduce per step over [gradient bucket | BatchNorm running statistics].  The update is
+ * split around the host's collective, as AdaptStepper.step(..., dp_bucket=parallel.DPBucket(...)) splits it:
+ *   forward (snb_stereonet_adapt_forward[_replay]) -> snb_stereonet_adapt_backward[_replay] -> the host all-reduces (SUM) the
+ *   state piece 5 (dp_flat, laid out as parallel.DPBucket.flat) over its replicas -> snb_stereonet_adapt_apply(world).
+ * Piece 4 (bn_stats) holds running_mean then running_var of each of the 17 trained BatchNorm layers, in
+ * parallel.used_bn_buffers(stereo_net, feature_net) order (stereo_net first).  With world = 1 and no collective, backward + apply
+ * computes what snb_stereonet_adapt_update computes, bit for bit.  The library records each backward's parameters on the host, keyed
+ * by the state address, and apply rejects by name, before any launch, world < 1, a state with no backward since its last apply or
+ * update, and params other than the backward's.  No allocation, no synchronisation, no host-to-device copy: all calls are
+ * CUDA-graph capturable (the collective itself is best left eager, between two graphs).
+ * --------------------------------------------------------------------------------------------------------------- */
+/* Gradients of loss[0] into the bucket, exactly as the update computes them (no clip, no Adam).  Then a copy of the 17 layers'
+ * running_mean / running_var from params into piece 4.  Same checks as snb_stereonet_adapt_update (forward record, RB pairing);
+ * every launch on `stream`. */
+SNB_API int snb_stereonet_adapt_backward(float* const* params, int k, int input_scale, int maxdisp, int B, int H, int W, void* state,
+                                 void* workspace, void* stream);
+/* The same after snb_stereonet_adapt_forward_replay: gradients of the total loss (both passes). */
+SNB_API int snb_stereonet_adapt_backward_replay(float* const* params, int k, int input_scale, int maxdisp, int B, int H, int W, int RB,
+                                        void* state, void* workspace, void* stream);
+/* After the host has SUM-all-reduced piece 5 over `world` replicas: running statistics = fl(piece4 * (float)(1.0 / world)) written
+ * back to params, then snb_adam_clip_step over the bucket with grad_scale = (float)(1.0 / world) and max_norm, lr, beta1, beta2, eps
+ * as snb_stereonet_adapt_update. */
+SNB_API int snb_stereonet_adapt_apply(float* const* params, int k, void* state, int world, float max_norm, double lr, double beta1,
+                              double beta2, double eps, void* stream);
 
 #ifdef __cplusplus
 }
