@@ -36,8 +36,9 @@ class AdaptStepper:
     # frame instead of a second full pass (adapt.py:339-349).  Off by default: train-mode BatchNorm then normalises with the
     # statistics of both samples together, which is NOT what the reference's two batch-1 passes compute.
     self.batched_replay = batched_replay
-    self.two_streams, self._side, self._wstream, self._acc_stream, self._acc_nodes = two_streams, None, None, None, None
-    self._rstream, self._rside = None, None
+    self.two_streams, self._wstream, self._acc_stream, self._acc_nodes = two_streams, None, None, None
+    self._forks = {}                        # the side streams of _fork, by name
+    self._feature_fork = "side"             # which of them predict's right feature pass runs on
     self._graphs = {}
     self._wprep = None                      # fused.WeightPrepBatch: all derived weight images in one launch per step
     self.launches_per_step = None
@@ -49,34 +50,45 @@ class AdaptStepper:
       raise RuntimeError("AdaptStepper(use_graph=True) needs make_optimizer(..., capturable=True) or fused=True")
 
   def predict(self, left, right):
-    if not (self.two_streams and left.is_cuda and torch.is_grad_enabled()):
-      fl, fr = self.feature_net(left), self.feature_net(right)                     # adapt.py:72
-      return self.stereo_net(left, fl, fr, "l", output_cost_volume=True)           # adapt.py:73
     # The two feature passes (and, through autograd, their backward passes) are independent chains of small, latency-bound
-    # kernels on a fraction of the SMs: the right-image pass runs on a second stream next to the left one.  Both passes update
-    # the same BatchNorm buffers, left first in the reference, so the right pass defers its running-statistics updates and
-    # they are applied on the main stream after the join.
+    # kernels on a fraction of the SMs: in the two-stream schedule the right-image pass runs on a side stream next to the left one.
+    # Both passes update the same BatchNorm buffers, left first in the reference: the fork applies the right pass's updates after.
+    join = self._fork(self._feature_fork, left)
+    fl = self.feature_net(left)                                                     # adapt.py:72
+    fr = join(self.feature_net, right)
+    return self.stereo_net(left, fl, fr, "l", output_cost_volume=True)             # adapt.py:73
+
+  def _fork(self, side, like):
+    """Forks the work that follows onto the side stream named `side` (created on first use): the stream waits here for what
+    is already enqueued on the current one, and the returned `join(fn, *args)` runs fn on it, with its train-mode BatchNorm
+    running-statistics updates deferred — into the enclosing fork's list, if there is one, else applied after the join on the
+    current stream, behind whatever ran there since the fork.  In the single-stream schedule (two_streams=False, a CPU
+    tensor, no grad) nothing forks and join(fn, *args) is fn(*args)."""
+    if not (self.two_streams and like.is_cuda and torch.is_grad_enabled()):
+      return lambda fn, *args: fn(*args)
     from .autograd import fused
-    main = torch.cuda.current_stream(left.device)
-    if self._side is None:
-      self._side = torch.cuda.Stream(device=left.device)
-    side = self._side
-    side.wait_stream(main)
-    fl = self.feature_net(left)
-    outer = fused.DEFER_BN                     # not None when this whole pass already defers (the replay pass, below)
-    pending = outer if outer is not None else []
-    with torch.cuda.stream(side):
-      fused.DEFER_BN = pending
-      try:
-        fr = self.feature_net(right)
-      finally:
-        fused.DEFER_BN = outer
-    main.wait_stream(side)
-    if not torch.cuda.is_current_stream_capturing():
-      fr.record_stream(main)
-    if outer is None:
-      fused.flush_deferred_bn(pending)
-    return self.stereo_net(left, fl, fr, "l", output_cost_volume=True)
+    stream = self._forks.get(side)
+    if stream is None:
+      stream = self._forks[side] = torch.cuda.Stream(device=like.device)
+    main = torch.cuda.current_stream(like.device)
+    stream.wait_stream(main)
+
+    def join(fn, *args):
+      outer = fused.DEFER_BN
+      pending = outer if outer is not None else []
+      with torch.cuda.stream(stream):
+        fused.DEFER_BN = pending
+        try:
+          out = fn(*args)
+        finally:
+          fused.DEFER_BN = outer
+      main.wait_stream(stream)
+      if not torch.cuda.is_current_stream_capturing():
+        out.record_stream(main)
+      if outer is None:
+        fused.flush_deferred_bn(pending)
+      return out
+    return join
 
   def step(self, left, right, replay=None, sync_grads=None, dp_params=None, dp_group=None, dp_bucket=None):
     """One gradient update (adapt.py:313-314,328-337,381-394).  `replay` = (left, right, gt_disp) adds the
@@ -123,44 +135,29 @@ class AdaptStepper:
       fused.WGRAD_STREAM = self._wstream                                            # weight gradients next to the data path
       fused.wgrad_token((1,), left.device)                                          # (creates the token buffer outside any capture)
     try:
-      if replay is not None and self.two_streams and left.is_cuda:
-        # The replay pass (adapt.py:339-349) is independent of the stream pass until the two losses are added: it runs on its own
-        # stream (its feature passes side by side on two more), with ALL its BatchNorm running-statistics updates deferred and
-        # applied after the stream pass's — the reference's order.
-        main = torch.cuda.current_stream(left.device)
-        if self._rstream is None:
-          self._rstream = torch.cuda.Stream(device=left.device)
-          self._rside = torch.cuda.Stream(device=left.device)
-        self._rstream.wait_stream(main)
-        outputs = self.predict(left, right)
-        loss = monodepth_single_loss(left, right, outputs, s)                      # adapt.py:328-337 (snb_photo_loss)
-        pend_r = []
-        side_main, self._side = self._side, self._rside
-        with torch.cuda.stream(self._rstream):
-          fused.DEFER_BN = pend_r
-          try:
-            out_er = self.predict(replay[0], replay[1])
-            loss_er = khamis_robust_loss(out_er["pred_disp_l/{}".format(s)], replay[2])
-          finally:
-            fused.DEFER_BN = None
-            self._side = side_main
-        main.wait_stream(self._rstream)
-        if not torch.cuda.is_current_stream_capturing():
-          loss_er.record_stream(main)
-        fused.flush_deferred_bn(pend_r)
-        loss = loss + self.er_loss_weight * loss_er
-      else:
-        outputs = self.predict(left, right)
-        loss = monodepth_single_loss(left, right, outputs, s)                      # adapt.py:328-337 (snb_photo_loss)
-        if replay is not None:
-          out_er = self.predict(replay[0], replay[1])                               # adapt.py:339-349: a second full pass
-          loss = loss + self.er_loss_weight * khamis_robust_loss(out_er["pred_disp_l/{}".format(s)], replay[2])
+      # The replay pass (adapt.py:339-349) is independent of the stream pass until the two losses are added: it runs on its own
+      # stream (its feature passes side by side on a second one) with ALL its BatchNorm running-statistics updates applied after
+      # the stream pass's, the reference's order.  The fork comes before the stream pass is enqueued: forking where the replay
+      # pass starts would make it wait for the whole stream pass.
+      join_replay = self._fork("replay", left) if replay is not None else None
+      outputs = self.predict(left, right)
+      loss = monodepth_single_loss(left, right, outputs, s)                        # adapt.py:328-337 (snb_photo_loss)
+      if replay is not None:
+        loss = loss + self.er_loss_weight * join_replay(self._replay_loss, replay)
     finally:
       fused.WGRAD_STREAM = None
     fcs = feature_contrast_mean(outputs["cost_volume_l/{}".format(s + self.stereo_net.k)]).mean()
     self.optimizer.zero_grad()
     loss.backward()
     return loss.detach(), fcs, outputs
+
+  def _replay_loss(self, replay):
+    self._feature_fork = "replay side"      # the replay pass runs on a side stream already: its right feature pass needs another
+    try:
+      out = self.predict(replay[0], replay[1])                                      # adapt.py:339-349: a second full pass
+    finally:
+      self._feature_fork = "side"
+    return khamis_robust_loss(out["pred_disp_l/{}".format(self.stereo_net.input_scale)], replay[2])
 
   def _refresh_weights(self):
     from .autograd import fused

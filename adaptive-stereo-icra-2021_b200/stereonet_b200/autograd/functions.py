@@ -1,5 +1,10 @@
 """torch.autograd.Function wrappers for the adaptation step (adapt.py:381-394).  Forward and backward both run in the
-library's CUDA kernels; torch only carries the graph, the saved tensors and a few layout views."""
+library's CUDA kernels; torch only carries the graph, the saved tensors and a few layout views.
+
+The layers with a weight gradient worth moving off the data path (ConvBnLrelu, ConvC32, RefineHead) serve both schedules of the
+adaptation step.  Without fused.WGRAD_STREAM, the weight is their input and they compute its gradient.  With it, the weight's
+WgradToken takes the weight's place, and the layer returns its output gradient as the token's gradient and computes no weight
+gradient (RefineHead, whose forward reads the weight, then also takes the weight detached: see refine_head_autograd)."""
 import torch
 
 from .. import ops
@@ -8,36 +13,6 @@ from . import fused
 
 def _c(t):
   return t if t.is_contiguous() else t.contiguous()
-
-
-class ConvBnLrelu(torch.autograd.Function):
-  """[x +] LeakyReLU(BN(conv3x3(x) + b)), train (batch stats) or eval (running stats)."""
-
-  @staticmethod
-  def forward(ctx, x, w, b, gamma, beta, conv, bn, dil, residual, training):
-    g = ops.geom(x.shape, 3, stride=1, dil=dil)
-    z, stats = fused.conv3x3_c32(x, conv, g, bias=b.detach(), want_stats=training)
-    if training:
-      scale, shift, mean, invstd = fused.bn_finalize(stats, z.numel() // 32, bn)
-    else:
-      scale, shift = fused.bn_fold(bn)
-      mean, invstd = bn.running_mean, fused.bn_invstd(bn)
-    y = ops.bn_apply(z, scale, shift, residual=x if residual else None, lrelu=True)
-    ctx.save_for_backward(x, z, scale, shift, mean, invstd)
-    ctx.conv, ctx.dil, ctx.residual, ctx.training, ctx.wshape = conv, dil, residual, training, tuple(w.shape)
-    return y
-
-  @staticmethod
-  def backward(ctx, dy):
-    x, z, scale, shift, mean, invstd = ctx.saved_tensors
-    dy = _c(dy)
-    dz, dgamma, dbeta, dbias = ops.bn_lrelu_bwd(z, dy, scale, shift, mean, invstd, ctx.training, lrelu=True)
-    g = ops.geom(x.shape, 3, stride=1, dil=ctx.dil)
-    dx = None
-    if ctx.needs_input_grad[0]:
-      dx, _ = fused.conv3x3_c32_dgrad(dz, ctx.conv, g, residual=dy if ctx.residual else None)
-    dw = fused.conv3x3_c32_wgrad(x, dz, g, ctx.wshape)
-    return dx, dw, dbias, dgamma, dbeta, None, None, None, None, None
 
 
 def _on_this_stream(*tensors):
@@ -49,41 +24,45 @@ def _on_this_stream(*tensors):
 
 
 class WgradToken(torch.autograd.Function):
-  """Carries the weight of a conv into the graph on its OWN stream.  forward returns a zero-stride token shaped like the conv's
-  output (one float of storage, no kernel); ConvBnLreluSplit returns dz as the token's gradient, so THIS node's backward — which
-  autograd runs on the stream this forward ran on, with the proper event waits — computes the weight gradient next to the data
-  path instead of inside it: the tensor-bound wgrad kernel overlaps the HBM-bound BatchNorm backward of the next layer."""
+  """Carries the weight of a conv into the graph on its OWN stream.  forward returns a zero-stride token of the conv's output
+  `shape` (one float of storage, no kernel); the layer's Function returns its output gradient dz as the token's gradient, so THIS
+  node's backward — which autograd runs on the stream this forward ran on, with the proper event waits — computes the weight
+  gradient `wgrad(*saved, dz)` next to the data path instead of inside it: the tensor-bound wgrad kernel overlaps the HBM-bound
+  BatchNorm backward of the next layer."""
 
   @staticmethod
-  def forward(ctx, w, x, dil):
-    ctx.save_for_backward(x)
-    ctx.dil, ctx.wshape = dil, tuple(w.shape)
-    return fused.wgrad_token(x.shape, x.device)
+  def forward(ctx, w, shape, wgrad, *saved):
+    ctx.save_for_backward(*saved)
+    ctx.wgrad = wgrad
+    return fused.wgrad_token(shape, w.device)
 
   @staticmethod
   def backward(ctx, dz):
-    (x,) = ctx.saved_tensors
+    saved = ctx.saved_tensors
     dz = _c(dz)
-    _on_this_stream(x, dz)
-    g = ops.geom(x.shape, 3, stride=1, dil=ctx.dil)
-    return fused.conv3x3_c32_wgrad(x, dz, g, ctx.wshape), None, None
+    _on_this_stream(*saved, dz)
+    return (ctx.wgrad(*saved, dz), None, None) + (None,) * len(saved)
 
 
-class ConvBnLreluSplit(torch.autograd.Function):
-  """ConvBnLrelu with the weight gradient split off into WgradToken (same kernels, same arithmetic)."""
+def _token(conv, shape, wgrad, *saved):
+  """conv.weight's WgradToken, made on fused.WGRAD_STREAM; None when no such stream is installed or the weight is frozen."""
+  ws = fused.WGRAD_STREAM
+  if ws is None or not conv.weight.requires_grad:
+    return None
+  with torch.cuda.stream(ws):
+    return WgradToken.apply(conv.weight, shape, wgrad, *saved)
+
+
+class ConvBnLrelu(torch.autograd.Function):
+  """[x +] LeakyReLU(BN(conv3x3(x) + b)), train (batch stats) or eval (running stats).  `w`: conv.weight, or its WgradToken."""
 
   @staticmethod
-  def forward(ctx, x, tok, b, gamma, beta, conv, bn, dil, residual, training):
+  def forward(ctx, x, w, b, gamma, beta, conv, bn, dil, residual, training):
     g = ops.geom(x.shape, 3, stride=1, dil=dil)
     z, stats = fused.conv3x3_c32(x, conv, g, bias=b.detach(), want_stats=training)
-    if training:
-      scale, shift, mean, invstd = fused.bn_finalize(stats, z.numel() // 32, bn)
-    else:
-      scale, shift = fused.bn_fold(bn)
-      mean, invstd = bn.running_mean, fused.bn_invstd(bn)
-    y = ops.bn_apply(z, scale, shift, residual=x if residual else None, lrelu=True)
-    ctx.save_for_backward(x, z, scale, shift, mean, invstd)
-    ctx.conv, ctx.dil, ctx.residual, ctx.training = conv, dil, residual, training
+    y, bn_saved = fused.bn_lrelu(z, stats, bn, training, residual=x if residual else None)
+    ctx.save_for_backward(x, z, *bn_saved)
+    ctx.conv, ctx.g, ctx.residual, ctx.training, ctx.token = conv, g, residual, training, w is not conv.weight
     return y
 
   @staticmethod
@@ -91,118 +70,46 @@ class ConvBnLreluSplit(torch.autograd.Function):
     x, z, scale, shift, mean, invstd = ctx.saved_tensors
     dy = _c(dy)
     dz, dgamma, dbeta, dbias = ops.bn_lrelu_bwd(z, dy, scale, shift, mean, invstd, ctx.training, lrelu=True)
-    g = ops.geom(x.shape, 3, stride=1, dil=ctx.dil)
     dx = None
     if ctx.needs_input_grad[0]:
-      dx, _ = fused.conv3x3_c32_dgrad(dz, ctx.conv, g, residual=dy if ctx.residual else None)
-    return dx, dz, dbias, dgamma, dbeta, None, None, None, None, None
+      dx, _ = fused.conv3x3_c32_dgrad(dz, ctx.conv, ctx.g, residual=dy if ctx.residual else None)
+    dw = dz if ctx.token else fused.conv3x3_c32_wgrad(x, dz, ctx.g, tuple(ctx.conv.weight.shape))
+    return dx, dw, dbias, dgamma, dbeta, None, None, None, None, None
 
 
 def conv_bn_lrelu_autograd(x, conv, bn, dil, residual, training):
-  ws = fused.WGRAD_STREAM
-  if ws is None or not conv.weight.requires_grad:
-    return ConvBnLrelu.apply(x, conv.weight, conv.bias, bn.weight, bn.bias, conv, bn, dil, residual, training)
-  with torch.cuda.stream(ws):
-    tok = WgradToken.apply(conv.weight, x.detach(), dil)
-  return ConvBnLreluSplit.apply(x, tok, conv.bias, bn.weight, bn.bias, conv, bn, dil, residual, training)
+  g, wshape = ops.geom(x.shape, 3, stride=1, dil=dil), tuple(conv.weight.shape)
+  tok = _token(conv, x.shape, lambda x, dz: fused.conv3x3_c32_wgrad(x, dz, g, wshape), x.detach())
+  return ConvBnLrelu.apply(x, conv.weight if tok is None else tok, conv.bias, bn.weight, bn.bias, conv, bn, dil, residual, training)
 
 
 class ConvC32(torch.autograd.Function):
-  """Conv2d 32->32 with bias only: 5x5 stride 2 (downsample[1:]) or 3x3 stride 1 (conv_alone)."""
+  """Conv2d 32->32 with bias only: 5x5 stride 2 (downsample[1:]) or 3x3 stride 1 (conv_alone).  `w`: conv.weight, or its
+  WgradToken."""
 
   @staticmethod
   def forward(ctx, x, w, b, conv, ksize, stride):
-    g = ops.geom(x.shape, ksize, stride=stride, dil=1, pad=ksize // 2)
-    if ksize == 3 and stride == 1:
-      y, _ = fused.conv3x3_c32(x, conv, g, bias=b.detach())
-    elif ksize == 5 and stride == 2:
-      y = fused.conv5x5s2_c32(x, conv, b.detach())
-    else:
-      y, _ = ops.conv_c32(x, fused.wprep(conv), g, bias=b.detach())
-    ctx.save_for_backward(x)
-    ctx.conv, ctx.ksize, ctx.stride, ctx.wshape = conv, ksize, stride, tuple(w.shape)
-    return y
+    g = fused.plain_geom(x.shape, ksize, stride)
+    ctx.conv, ctx.g, ctx.token = conv, g, w is not conv.weight
+    if not ctx.token:
+      ctx.save_for_backward(x)               # for the weight gradient; with a token, x is the token's to keep
+    return fused.plain_conv(x, conv, g, b.detach())
 
   @staticmethod
   def backward(ctx, dy):
-    (x,) = ctx.saved_tensors
     dy = _c(dy)
-    g = ops.geom(x.shape, ctx.ksize, stride=ctx.stride, dil=1, pad=ctx.ksize // 2)
-    dx = None
-    if ctx.needs_input_grad[0]:
-      if ctx.ksize == 3 and ctx.stride == 1:
-        dx, _ = fused.conv3x3_c32_dgrad(dy, ctx.conv, g)
-      elif ctx.ksize == 5 and ctx.stride == 2:
-        dx = fused.conv5x5s2_c32_dgrad(dy, ctx.conv, x.shape[1], x.shape[2])
-      else:
-        gt = ops.geom_transposed(g)
-        dx, _ = ops.conv_c32(dy, fused.wprep(ctx.conv, 2), gt)
-    if ctx.ksize == 3 and ctx.stride == 1:
-      dw = fused.conv3x3_c32_wgrad(x, dy, g, ctx.wshape)
-    else:
-      dw = ops.conv_c32_wgrad(x, dy, g, ctx.wshape)
+    dx = fused.plain_conv_dgrad(dy, ctx.conv, ctx.g) if ctx.needs_input_grad[0] else None
+    dw = dy
+    if not ctx.token:
+      (x,) = ctx.saved_tensors
+      dw = fused.plain_conv_wgrad(x, dy, ctx.g, tuple(ctx.conv.weight.shape))
     return dx, dw, ops.channel_sum(dy), None, None, None
 
 
-class WgradTokenC32(torch.autograd.Function):
-  """WgradToken for ConvC32 (bias-only 32->32 convs: 5x5 stride 2, 3x3): see WgradToken."""
-
-  @staticmethod
-  def forward(ctx, w, x, ksize, stride):
-    g = ops.geom(x.shape, ksize, stride=stride, dil=1, pad=ksize // 2)
-    ctx.save_for_backward(x)
-    ctx.ksize, ctx.stride, ctx.wshape = ksize, stride, tuple(w.shape)
-    oshape = tuple(ops.out_shape(g, False))
-    return fused.wgrad_token(oshape, x.device)
-
-  @staticmethod
-  def backward(ctx, dy):
-    (x,) = ctx.saved_tensors
-    dy = _c(dy)
-    _on_this_stream(x, dy)
-    g = ops.geom(x.shape, ctx.ksize, stride=ctx.stride, dil=1, pad=ctx.ksize // 2)
-    if ctx.ksize == 3 and ctx.stride == 1:
-      return fused.conv3x3_c32_wgrad(x, dy, g, ctx.wshape), None, None, None
-    return ops.conv_c32_wgrad(x, dy, g, ctx.wshape), None, None, None
-
-
-class ConvC32Split(torch.autograd.Function):
-  """ConvC32 with the weight gradient split off into WgradTokenC32."""
-
-  @staticmethod
-  def forward(ctx, x, tok, b, conv, ksize, stride):
-    g = ops.geom(x.shape, ksize, stride=stride, dil=1, pad=ksize // 2)
-    if ksize == 3 and stride == 1:
-      y, _ = fused.conv3x3_c32(x, conv, g, bias=b.detach())
-    elif ksize == 5 and stride == 2:
-      y = fused.conv5x5s2_c32(x, conv, b.detach())
-    else:
-      y, _ = ops.conv_c32(x, fused.wprep(conv), g, bias=b.detach())
-    ctx.conv, ctx.ksize, ctx.stride, ctx.xshape = conv, ksize, stride, tuple(x.shape)
-    return y
-
-  @staticmethod
-  def backward(ctx, dy):
-    dy = _c(dy)
-    g = ops.geom(ctx.xshape, ctx.ksize, stride=ctx.stride, dil=1, pad=ctx.ksize // 2)
-    dx = None
-    if ctx.needs_input_grad[0]:
-      if ctx.ksize == 3 and ctx.stride == 1:
-        dx, _ = fused.conv3x3_c32_dgrad(dy, ctx.conv, g)
-      elif ctx.ksize == 5 and ctx.stride == 2:
-        dx = fused.conv5x5s2_c32_dgrad(dy, ctx.conv, ctx.xshape[1], ctx.xshape[2])
-      else:
-        dx, _ = ops.conv_c32(dy, fused.wprep(ctx.conv, 2), ops.geom_transposed(g))
-    return dx, dy, ops.channel_sum(dy), None, None, None
-
-
 def conv_c32_autograd(x, conv, ksize, stride):
-  ws = fused.WGRAD_STREAM
-  if ws is None or not conv.weight.requires_grad:
-    return ConvC32.apply(x, conv.weight, conv.bias, conv, ksize, stride)
-  with torch.cuda.stream(ws):
-    tok = WgradTokenC32.apply(conv.weight, x.detach(), ksize, stride)
-  return ConvC32Split.apply(x, tok, conv.bias, conv, ksize, stride)
+  g, wshape = fused.plain_geom(x.shape, ksize, stride), tuple(conv.weight.shape)
+  tok = _token(conv, ops.out_shape(g, False), lambda x, dy: fused.plain_conv_wgrad(x, dy, g, wshape), x.detach())
+  return ConvC32.apply(x, conv.weight if tok is None else tok, conv.bias, conv, ksize, stride)
 
 
 class Conv5x5s2First(torch.autograd.Function):
@@ -268,88 +175,30 @@ class Upsample(torch.autograd.Function):
 
 
 class RefineHead(torch.autograd.Function):
-  """Upsample + scale + concat + Conv2d(4->32) + BN + LeakyReLU.  Outputs (up [B,H,W], y [B,H,W,32])."""
-
-  @staticmethod
-  def forward(ctx, coarse, rgb, w, b, gamma, beta, bn, training):
-    up, z, stats = ops.refine_in_conv(coarse, rgb, w, b.detach(), want_stats=training)
-    if training:
-      scale, shift, mean, invstd = fused.bn_finalize(stats, z.numel() // 32, bn)
-    else:
-      scale, shift = fused.bn_fold(bn)
-      mean, invstd = bn.running_mean, fused.bn_invstd(bn)
-    y = ops.bn_apply(z, scale, shift, residual=None, lrelu=True)
-    ctx.save_for_backward(coarse, rgb, w, z, scale, shift, mean, invstd)
-    ctx.training = training
-    return up, y
-
-  @staticmethod
-  def backward(ctx, dup, dy):
-    coarse, rgb, w, z, scale, shift, mean, invstd = ctx.saved_tensors
-    dz, dgamma, dbeta, dbias = ops.bn_lrelu_bwd(z, _c(dy), scale, shift, mean, invstd, ctx.training, lrelu=True)
-    dw = ops.refine_in_wgrad(coarse, rgb, dz)
-    dcoarse = None
-    if ctx.needs_input_grad[0]:
-      # d(input channel 0)[q] = sum_tap sum_co dz[q - off(tap)][co] * W[co][0][tap]: a 32->1 "conv" with flipped taps
-      wflip = torch.flip(w.detach()[:, 0].reshape(32, 9), dims=(1,)).reshape(1, 32, 3, 3).contiguous()
-      taps = ops.conv_c32_taps(dz, wflip, 9)
-      d_up = ops.tapsum_refine_out(taps, None, _c(dup), relu=False)          # + gradient arriving directly on `up`
-      dcoarse = ops.upsample_bilinear_bwd(d_up, coarse.shape[-2], coarse.shape[-1], float(rgb.shape[-1]) / float(coarse.shape[-1]))
-    return dcoarse, None, dw, dbias, dgamma, dbeta, None, None
-
-
-class WgradTokenRefine(torch.autograd.Function):
-  """WgradToken for RefineHead's Conv2d(4 -> 32): see WgradToken."""
-
-  @staticmethod
-  def forward(ctx, w, coarse, rgb):
-    ctx.save_for_backward(coarse, rgb)
-    return fused.wgrad_token((rgb.shape[0], rgb.shape[2], rgb.shape[3], 32), rgb.device)
-
-  @staticmethod
-  def backward(ctx, dz):
-    coarse, rgb = ctx.saved_tensors
-    dz = _c(dz)
-    _on_this_stream(coarse, rgb, dz)
-    return ops.refine_in_wgrad(coarse, rgb, dz), None, None
-
-
-class RefineHeadSplit(torch.autograd.Function):
-  """RefineHead with the weight gradient split off into WgradTokenRefine."""
+  """Upsample + scale + concat + Conv2d(4->32) + BN + LeakyReLU.  Outputs (up [B,H,W], y [B,H,W,32]).  `tok, w`: None and
+  conv.weight, or the weight's WgradToken and the weight detached."""
 
   @staticmethod
   def forward(ctx, coarse, rgb, tok, w, b, gamma, beta, bn, training):
     up, z, stats = ops.refine_in_conv(coarse, rgb, w, b.detach(), want_stats=training)
-    if training:
-      scale, shift, mean, invstd = fused.bn_finalize(stats, z.numel() // 32, bn)
-    else:
-      scale, shift = fused.bn_fold(bn)
-      mean, invstd = bn.running_mean, fused.bn_invstd(bn)
-    y = ops.bn_apply(z, scale, shift, residual=None, lrelu=True)
-    ctx.save_for_backward(coarse, rgb, w, z, scale, shift, mean, invstd)
-    ctx.training = training
+    y, bn_saved = fused.bn_lrelu(z, stats, bn, training)
+    ctx.save_for_backward(coarse, rgb, w, z, *bn_saved)
+    ctx.training, ctx.token = training, tok is not None
     return up, y
 
   @staticmethod
   def backward(ctx, dup, dy):
     coarse, rgb, w, z, scale, shift, mean, invstd = ctx.saved_tensors
     dz, dgamma, dbeta, dbias = ops.bn_lrelu_bwd(z, _c(dy), scale, shift, mean, invstd, ctx.training, lrelu=True)
-    dcoarse = None
-    if ctx.needs_input_grad[0]:
-      wflip = torch.flip(w[:, 0].reshape(32, 9), dims=(1,)).reshape(1, 32, 3, 3).contiguous()
-      taps = ops.conv_c32_taps(dz, wflip, 9)
-      d_up = ops.tapsum_refine_out(taps, None, _c(dup), relu=False)
-      dcoarse = ops.upsample_bilinear_bwd(d_up, coarse.shape[-2], coarse.shape[-1], float(rgb.shape[-1]) / float(coarse.shape[-1]))
-    return dcoarse, None, dz, None, dbias, dgamma, dbeta, None, None
+    dw = None if ctx.token else ops.refine_in_wgrad(coarse, rgb, dz)
+    dcoarse = fused.refine_in_dgrad(dz, dup, w, coarse, rgb) if ctx.needs_input_grad[0] else None
+    return dcoarse, None, dz if ctx.token else None, dw, dbias, dgamma, dbeta, None, None
 
 
 def refine_head_autograd(coarse, rgb, conv, bn, training):
-  ws = fused.WGRAD_STREAM
-  if ws is None or not conv.weight.requires_grad:
-    return RefineHead.apply(coarse, rgb, conv.weight, conv.bias, bn.weight, bn.bias, bn, training)
-  with torch.cuda.stream(ws):
-    tok = WgradTokenRefine.apply(conv.weight, coarse.detach(), rgb)
-  return RefineHeadSplit.apply(coarse, rgb, tok, conv.weight.detach(), conv.bias, bn.weight, bn.bias, bn, training)
+  tok = _token(conv, (rgb.shape[0], rgb.shape[2], rgb.shape[3], 32), ops.refine_in_wgrad, coarse.detach(), rgb)
+  w = conv.weight if tok is None else conv.weight.detach()
+  return RefineHead.apply(coarse, rgb, tok, w, conv.bias, bn.weight, bn.bias, bn, training)
 
 
 class RefineTail(torch.autograd.Function):

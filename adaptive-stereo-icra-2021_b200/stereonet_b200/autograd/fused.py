@@ -34,7 +34,7 @@ def state_epoch():
 
 
 # A torch.cuda.Stream installed here (adapt.AdaptStepper does, around its forward) moves the weight gradients of the conv + BN +
-# LeakyReLU layers onto that stream: see functions.WgradToken.
+# LeakyReLU layers, the plain 32->32 convs and the refinement input layer onto that stream: see functions.WgradToken.
 WGRAD_STREAM = None
 _TOKEN = {}
 
@@ -62,6 +62,17 @@ def bn_finalize(stats, count, bn):
   out = ops.bn_finalize(stats, count, bn)
   bump_bn_epoch()
   return out
+
+
+def bn_lrelu(z, stats, bn, training, residual=None):
+  """[residual +] LeakyReLU(BN(z)) of a conv output z: batch statistics in training (from `stats`, the conv epilogue's partial
+  sums), running statistics otherwise.  Returns y and (scale, shift, mean, invstd), what ops.bn_lrelu_bwd needs."""
+  if training:
+    scale, shift, mean, invstd = bn_finalize(stats, z.numel() // 32, bn)
+  else:
+    scale, shift = bn_fold(bn)
+    mean, invstd = bn.running_mean, bn_invstd(bn)
+  return ops.bn_apply(z, scale, shift, residual=residual, lrelu=True), (scale, shift, mean, invstd)
 
 
 def flush_deferred_bn(pending):
@@ -346,20 +357,40 @@ def downsample_pair(img, conv0, conv1):
   return conv_plain(conv5x5s2_first(img, conv0), conv1, ksize=5, stride=2)
 
 
+def plain_geom(x_shape, ksize, stride):
+  """Geometry of a bias-only 32->32 conv: 5x5 stride 2 (downsample[1:]) or 3x3 stride 1 (conv_alone), the two the model has."""
+  if (ksize, stride) not in ((5, 2), (3, 1)):
+    raise ValueError(f"stereonet_b200: no 32->32 convolution kernels for {ksize}x{ksize} stride {stride} "
+                     "(there are for 5x5 stride 2 and 3x3 stride 1)")
+  return ops.geom(x_shape, ksize, stride=stride, dil=1, pad=ksize // 2)
+
+
+def plain_conv(x, conv, g, bias):
+  if g.stride == 1:
+    return conv3x3_c32(x, conv, g, bias=bias)[0]
+  return conv5x5s2_c32(x, conv, bias)
+
+
+def plain_conv_dgrad(dy, conv, g):
+  if g.stride == 1:
+    return conv3x3_c32_dgrad(dy, conv, g)[0]
+  return conv5x5s2_c32_dgrad(dy, conv, g.H, g.W)
+
+
+def plain_conv_wgrad(x, dy, g, wshape):
+  if g.stride == 1:
+    return conv3x3_c32_wgrad(x, dy, g, wshape)
+  return ops.conv_c32_wgrad(x, dy, g, wshape)
+
+
 def conv_plain(x, conv, ksize, stride):
   """Conv2d 32->32 with bias only (downsample[1:], conv_alone)."""
-  g = ops.geom(x.shape, ksize, stride=stride, dil=1, pad=ksize // 2)
+  g = plain_geom(x.shape, ksize, stride)
   _f16_guard()
   if _needs_grad(x, conv):
     from . import functions
     return functions.conv_c32_autograd(x, conv, ksize, stride)
-  if ksize == 3 and stride == 1:
-    y, _ = conv3x3_c32(x, conv, g, bias=conv.bias.detach())
-  elif ksize == 5 and stride == 2:
-    y = conv5x5s2_c32(x, conv, conv.bias.detach())
-  else:
-    y, _ = ops.conv_c32(x, wprep(conv), g, bias=conv.bias.detach())
-  return y
+  return plain_conv(x, conv, g, conv.bias.detach())
 
 
 # ------------------------------------------------------------------------------------------------ conv + BN + LeakyReLU
@@ -376,8 +407,7 @@ def conv_bn_lrelu(x, conv, bn, dil, residual, training):
                        residual=x if residual else None, lrelu=True)
     return y
   z, stats = conv3x3_c32(x, conv, g, bias=conv.bias.detach(), want_stats=True)
-  scale, shift, _, _ = bn_finalize(stats, z.numel() // 32, bn)
-  return ops.bn_apply(z, scale, shift, residual=x if residual else None, lrelu=True)
+  return bn_lrelu(z, stats, bn, True, residual=x if residual else None)[0]
 
 
 # ------------------------------------------------------------------------------------------------ stereo head
@@ -423,8 +453,17 @@ def refine_head(coarse, rgb, conv, bn, training):
     up, x, _ = ops.refine_in_conv(coarse, rgb, conv.weight, conv.bias.detach(), scale=scale, shift=shift, lrelu=True)
     return up, x
   up, z, stats = ops.refine_in_conv(coarse, rgb, conv.weight, conv.bias.detach(), want_stats=True)
-  scale, shift, _, _ = bn_finalize(stats, z.numel() // 32, bn)
-  return up, ops.bn_apply(z, scale, shift, residual=None, lrelu=True)
+  return up, bn_lrelu(z, stats, bn, True)[0]
+
+
+def refine_in_dgrad(dz, dup, w, coarse, rgb):
+  """Gradient of the refinement input layer's coarse disparity: dz back through the conv's disparity channel plus dup, the
+  gradient arriving on the upsampled disparity directly, both back through the upsampling."""
+  # d(input channel 0)[q] = sum_tap sum_co dz[q - off(tap)][co] * W[co][0][tap]: a 32->1 "conv" with flipped taps
+  wflip = torch.flip(w.detach()[:, 0].reshape(32, 9), dims=(1,)).reshape(1, 32, 3, 3).contiguous()
+  taps = ops.conv_c32_taps(dz, wflip, 9)
+  d_up = ops.tapsum_refine_out(taps, None, dup.contiguous(), relu=False)
+  return ops.upsample_bilinear_bwd(d_up, coarse.shape[-2], coarse.shape[-1], float(rgb.shape[-1]) / float(coarse.shape[-1]))
 
 
 def refine_tail(x, conv, up):

@@ -18,16 +18,47 @@ pytestmark = pytest.mark.gpu
 GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
 
+# The per-layer backward tests below run each layer as the single-stream adaptation step does (fused.WGRAD_STREAM None) and,
+# with the wgrad_side parameter, again as the two-stream step does: WGRAD_STREAM set to a side stream, the weight gradients then
+# coming from WgradToken nodes on it.  The second run must give the first run's output and gradients bit for bit.
+WGRAD_SIDE = pytest.mark.parametrize("wgrad_side", [pytest.param(False, id=pytest.HIDDEN_PARAM), pytest.param(True, id="wgrad_side")])
+
+
+def _with_wgrad_stream(stream, run):
+  old = fused.WGRAD_STREAM
+  fused.WGRAD_STREAM = stream
+  try:
+    out = run()
+  finally:
+    fused.WGRAD_STREAM = old
+  torch.cuda.synchronize()
+  return out
+
+
+def layer_grads(wgrad_side, run):
+  """run() -> (output, {name: gradient}) with fused.WGRAD_STREAM None; with wgrad_side, also with a side stream installed, which
+  must reproduce the first run exactly.  Returns the last run's output and gradients."""
+  y, grads = _with_wgrad_stream(None, run)
+  if wgrad_side:
+    y2, grads2 = _with_wgrad_stream(torch.cuda.Stream(device=DEV), run)
+    assert torch.equal(y2, y), "forward with WGRAD_STREAM set"
+    for name, g in grads.items():
+      assert torch.equal(grads2[name], g), f"{name} with WGRAD_STREAM set"
+    y, grads = y2, grads2
+  return y, grads
+
+
 def randomize_bn(bn, seed):
   with torch.no_grad():
     bn.weight.copy_(rnd(32, seed=seed).abs() + 0.5); bn.bias.copy_(rnd(32, seed=seed + 1))
     bn.running_mean.copy_(rnd(32, seed=seed + 2) * 0.1); bn.running_var.copy_(rnd(32, seed=seed + 3).abs() + 0.5)
 
 
+@WGRAD_SIDE
 @pytest.mark.parametrize("backend", ["ffma", "tc3"])
 @pytest.mark.parametrize("training", [True, False])
 @pytest.mark.parametrize("three_d,dil,residual", [(False, 1, True), (False, 4, True), (True, 1, False)])
-def test_conv_bn_lrelu_backward(three_d, dil, residual, training, backend):
+def test_conv_bn_lrelu_backward(three_d, dil, residual, training, backend, wgrad_side):
   shape = (1, 32, 6, 9, 21) if three_d else (2, 32, 17, 29)
   # Small-integer inputs and dyadic weights make every convolution sum exact in fp32 (and in the 3xTF32 split), so z is
   # bit-identical on CPU and GPU and no activation sits within rounding distance of the LeakyReLU kink (a flipped
@@ -40,48 +71,60 @@ def test_conv_bn_lrelu_backward(three_d, dil, residual, training, backend):
     conv.bias.copy_(torch.randint(-4, 5, (32,), generator=torch.Generator().manual_seed(4)).float() / 8)
   bn = torch.nn.BatchNorm3d(32) if three_d else torch.nn.BatchNorm2d(32)
   randomize_bn(bn, 7)
-  gconv, gbn = copy.deepcopy(conv).to(DEV), copy.deepcopy(bn).to(DEV)
-  conv.train(training); bn.train(training); gbn.train(training)
+  conv0, bn0 = copy.deepcopy(conv), copy.deepcopy(bn)
+  conv.train(training); bn.train(training)
   y = F.leaky_relu(bn(conv(x)), 0.2)
   if residual:
     y = x + y
   gy = rnd(*shape, seed=2)
   y.backward(gy)
-  old = fused.CONV_BACKEND
-  fused.set_conv_backend(backend)
-  try:
+
+  def run():
+    gconv, gbn = copy.deepcopy(conv0).to(DEV), copy.deepcopy(bn0).to(DEV)
+    gbn.train(training)
     xg = cl(x.detach()).requires_grad_()
-    yg = Fn.conv_bn_lrelu_autograd(xg, gconv, gbn, dil, residual, training)
-    yg.backward(cl(gy))
-  finally:
-    fused.set_conv_backend(old)
-  close(uncl(yg.detach()), y.detach(), 1e-5, "forward")
-  close(uncl(xg.grad), x.grad, 2e-5, "dx")
-  close(gconv.weight.grad.cpu(), conv.weight.grad, 2e-5, "dW")
-  close(gbn.weight.grad.cpu(), bn.weight.grad, 2e-5, "dgamma")
-  close(gbn.bias.grad.cpu(), bn.bias.grad, 2e-5, "dbeta")
+    old = fused.CONV_BACKEND
+    fused.set_conv_backend(backend)
+    try:
+      yg = Fn.conv_bn_lrelu_autograd(xg, gconv, gbn, dil, residual, training)
+      yg.backward(cl(gy))
+    finally:
+      fused.set_conv_backend(old)
+    return yg.detach(), dict(dx=xg.grad, dW=gconv.weight.grad, dbias=gconv.bias.grad, dgamma=gbn.weight.grad, dbeta=gbn.bias.grad)
+  yg, d = layer_grads(wgrad_side, run)
+  close(uncl(yg), y.detach(), 1e-5, "forward")
+  close(uncl(d["dx"]), x.grad, 2e-5, "dx")
+  close(d["dW"].cpu(), conv.weight.grad, 2e-5, "dW")
+  close(d["dgamma"].cpu(), bn.weight.grad, 2e-5, "dgamma")
+  close(d["dbeta"].cpu(), bn.bias.grad, 2e-5, "dbeta")
   if training:   # the conv-bias gradient under batch-stat BN is mathematically zero: compare absolutely
-    assert gconv.bias.grad.abs().max().item() <= 1e-3 * (conv.weight.grad.abs().max().item() + 1.0)
+    assert d["dbias"].abs().max().item() <= 1e-3 * (conv.weight.grad.abs().max().item() + 1.0)
   else:
-    close(gconv.bias.grad.cpu(), conv.bias.grad, 2e-5, "dbias")
+    close(d["dbias"].cpu(), conv.bias.grad, 2e-5, "dbias")
 
 
+@WGRAD_SIDE
 @pytest.mark.parametrize("ksize,stride,H,W", [(5, 2, 23, 37), (5, 2, 24, 40), (3, 1, 12, 19)])
-def test_conv_plain_backward(ksize, stride, H, W):
+def test_conv_plain_backward(ksize, stride, H, W, wgrad_side):
   x = rnd(2, 32, H, W, seed=1).requires_grad_()
   torch.manual_seed(5)
   conv = torch.nn.Conv2d(32, 32, ksize, stride=stride, padding=ksize // 2)
-  gconv = copy.deepcopy(conv).to(DEV)
+  conv0 = copy.deepcopy(conv)
   y = conv(x)
   gy = rnd(*y.shape, seed=2)
   y.backward(gy)
-  xg = cl(x.detach()).requires_grad_()
-  yg = Fn.ConvC32.apply(xg, gconv.weight, gconv.bias, gconv, ksize, stride)
-  yg.backward(cl(gy))
-  close(uncl(yg.detach()), y.detach(), 1e-5, "forward")
-  close(uncl(xg.grad), x.grad, 2e-5, "dx")
-  close(gconv.weight.grad.cpu(), conv.weight.grad, 2e-5, "dW")
-  close(gconv.bias.grad.cpu(), conv.bias.grad, 2e-5, "dbias")
+
+  def run():
+    gconv = copy.deepcopy(conv0).to(DEV)
+    xg = cl(x.detach()).requires_grad_()
+    yg = Fn.conv_c32_autograd(xg, gconv, ksize, stride)
+    yg.backward(cl(gy))
+    return yg.detach(), dict(dx=xg.grad, dW=gconv.weight.grad, dbias=gconv.bias.grad)
+  yg, d = layer_grads(wgrad_side, run)
+  close(uncl(yg), y.detach(), 1e-5, "forward")
+  close(uncl(d["dx"]), x.grad, 2e-5, "dx")
+  close(d["dW"].cpu(), conv.weight.grad, 2e-5, "dW")
+  close(d["dbias"].cpu(), conv.bias.grad, 2e-5, "dbias")
 
 
 def test_first_conv_backward():
@@ -238,9 +281,10 @@ def test_adapt_step_vs_reference_golden(name, loss_impl):
       assert d.max() <= 2.1 * 5e-5 and (d <= 3e-6).mean() >= 0.97, (key, d.max(), (d <= 3e-6).mean())
 
 
+@WGRAD_SIDE
 @pytest.mark.parametrize("training", [True, False])
 @pytest.mark.parametrize("bn_bias", [60.0, -60.0])
-def test_refine_head_backward_exact_side_of_kink(training, bn_bias):
+def test_refine_head_backward_exact_side_of_kink(training, bn_bias, wgrad_side):
   """RefineHead (upsample + concat + conv 4->32 + BN + LeakyReLU) with the BN shift pushed far from the LeakyReLU kink, so
   every mask is unambiguous and gradients must agree to fp32 rounding."""
   B, h, w, H, W = 2, 9, 15, 68, 120
@@ -253,20 +297,27 @@ def test_refine_head_backward_exact_side_of_kink(training, bn_bias):
     bn.bias.fill_(bn_bias)
     if not training:
       bn.running_var.fill_(400.0)          # keep |BN(z)| << |shift| with running statistics as well
-  gconv, gbn = copy.deepcopy(conv).to(DEV), copy.deepcopy(bn).to(DEV)
-  bn.train(training); gbn.train(training)
+  conv0, bn0 = copy.deepcopy(conv), copy.deepcopy(bn)
+  bn.train(training)
   up = F.interpolate(coarse.unsqueeze(1), size=(H, W), mode="bilinear", align_corners=False) * (W / w)
   y = F.leaky_relu(bn(conv(torch.cat([up, rgb], 1))), 0.2)
   gy, gu = rnd(B, 32, H, W, seed=3), rnd(B, H, W, seed=4)
   ((y * gy).sum() + (up.squeeze(1) * gu).sum()).backward()
-  cg = coarse.detach().to(DEV).requires_grad_()
-  upg, yg = Fn.refine_head_autograd(cg, rgb.to(DEV), gconv, gbn, training)
-  ((yg * cl(gy)).sum() + (upg * gu.to(DEV)).sum()).backward()
-  close(uncl(yg.detach()), y.detach(), 1e-5, "forward")
-  close(cg.grad.cpu(), coarse.grad, 3e-5, "dcoarse")
-  close(gconv.weight.grad.cpu(), conv.weight.grad, 3e-5, "dW")
-  close(gbn.weight.grad.cpu(), bn.weight.grad, 3e-5, "dgamma")
-  close(gbn.bias.grad.cpu(), bn.bias.grad, 3e-5, "dbeta")
+
+  def run():
+    gconv, gbn = copy.deepcopy(conv0).to(DEV), copy.deepcopy(bn0).to(DEV)
+    gbn.train(training)
+    cg = coarse.detach().to(DEV).requires_grad_()
+    upg, yg = Fn.refine_head_autograd(cg, rgb.to(DEV), gconv, gbn, training)
+    ((yg * cl(gy)).sum() + (upg * gu.to(DEV)).sum()).backward()
+    return yg.detach(), dict(dcoarse=cg.grad, dW=gconv.weight.grad, dbias=gconv.bias.grad, dgamma=gbn.weight.grad,
+                             dbeta=gbn.bias.grad)
+  yg, d = layer_grads(wgrad_side, run)
+  close(uncl(yg), y.detach(), 1e-5, "forward")
+  close(d["dcoarse"].cpu(), coarse.grad, 3e-5, "dcoarse")
+  close(d["dW"].cpu(), conv.weight.grad, 3e-5, "dW")
+  close(d["dgamma"].cpu(), bn.weight.grad, 3e-5, "dgamma")
+  close(d["dbeta"].cpu(), bn.bias.grad, 3e-5, "dbeta")
 
 
 def test_refine_tail_backward():

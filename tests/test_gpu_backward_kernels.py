@@ -10,7 +10,8 @@ bound and its reason written beside it.  Where a LeakyReLU / ReLU kink makes rou
 for integer-grid data, a checked margin) away from it, so no tolerance has to absorb a flipped mask.
 
 The composite tests at the end run the autograd Functions of the adaptation step at the sizes the step runs, on the product
-"ws" convolution back end and on "tc3" as a cross-check, in the pattern of test_gpu_backward.test_conv_bn_lrelu_backward."""
+"ws" convolution back end and on "tc3" as a cross-check, in the pattern of test_gpu_backward.test_conv_bn_lrelu_backward, and
+(wgrad_side) again with their weight gradients on a side stream, as the two-stream step runs them."""
 import copy
 
 import numpy as np
@@ -22,6 +23,7 @@ import stereonet_oracle as O
 from stereonet_b200 import ops
 from stereonet_b200.autograd import functions as Fn, fused
 from test_gpu_kernels import cl, uncl, rnd, close, DEV
+from test_gpu_backward import WGRAD_SIDE, layer_grads
 
 pytestmark = pytest.mark.gpu
 
@@ -491,9 +493,10 @@ CBL_CASES = [((1, 32, 376, 1248), 1, True), ((1, 32, 376, 1248), 2, True), ((1, 
              ((1, 32, 376, 1248), 8, True), ((2, 32, 47, 156), 1, True), ((1, 32, 24, 47, 156), 1, False)]
 
 
+@WGRAD_SIDE
 @pytest.mark.parametrize("training", [True, False])
 @pytest.mark.parametrize("shape,dil,residual", CBL_CASES)
-def test_conv_bn_lrelu_backward_kitti(shape, dil, residual, training):
+def test_conv_bn_lrelu_backward_kitti(shape, dil, residual, training, wgrad_side):
   """ConvBnLrelu (conv + BN + LeakyReLU [+ x]) forward and backward on the product "ws" back end and on "tc3".  Integer x and
   weights k/16 make every convolution sum exact, so z is bit-identical on CPU and GPU; the BN pre-activation is checked to sit
   >= 1e-5 from the kink (a flipped mask there would be a legitimate O(1) difference).  Reference: float64 CPU autograd, one per
@@ -520,29 +523,30 @@ def test_conv_bn_lrelu_backward_kitti(shape, dil, residual, training):
   gy = rnd(*shape, seed=2)
   y.backward(gy.double())
   for backend in ("ws", "tc3"):
-    gconv, gbn = copy.deepcopy(gconv0).to(DEV), copy.deepcopy(gbn0).to(DEV)
-    gbn.train(training)
-    xg = cl(x).requires_grad_()
 
     def run():
+      gconv, gbn = copy.deepcopy(gconv0).to(DEV), copy.deepcopy(gbn0).to(DEV)
+      gbn.train(training)
+      xg = cl(x).requires_grad_()
       yg = Fn.conv_bn_lrelu_autograd(xg, gconv, gbn, dil, residual, training)
       yg.backward(cl(gy))
-      return yg
-    yg = with_backend(backend, run)
+      return yg.detach(), dict(dx=xg.grad, dW=gconv.weight.grad, dbias=gconv.bias.grad, dgamma=gbn.weight.grad, dbeta=gbn.bias.grad)
+    yg, d = layer_grads(wgrad_side, lambda: with_backend(backend, run))
     what = f"ConvBnLrelu {backend} {tuple(shape)} dil={dil} train={training}"
-    close(uncl(yg.detach()), y.detach(), 1e-5, what + ": forward")
-    close(uncl(xg.grad), x64.grad, 2e-5, what + ": dx")
-    close(gconv.weight.grad.cpu(), conv.weight.grad, 2e-5, what + ": dW")
-    close(gbn.weight.grad.cpu(), bn.weight.grad, 2e-5, what + ": dgamma")
-    close(gbn.bias.grad.cpu(), bn.bias.grad, 2e-5, what + ": dbeta")
+    close(uncl(yg), y.detach(), 1e-5, what + ": forward")
+    close(uncl(d["dx"]), x64.grad, 2e-5, what + ": dx")
+    close(d["dW"].cpu(), conv.weight.grad, 2e-5, what + ": dW")
+    close(d["dgamma"].cpu(), bn.weight.grad, 2e-5, what + ": dgamma")
+    close(d["dbeta"].cpu(), bn.bias.grad, 2e-5, what + ": dbeta")
     if training:   # the conv-bias gradient under batch-stat BN is mathematically zero: compare absolutely
-      assert gconv.bias.grad.abs().max().item() <= 1e-3 * (conv.weight.grad.abs().max().item() + 1.0), what + ": dbias"
+      assert d["dbias"].abs().max().item() <= 1e-3 * (conv.weight.grad.abs().max().item() + 1.0), what + ": dbias"
     else:
-      close(gconv.bias.grad.cpu(), conv.bias.grad, 2e-5, what + ": dbias")
+      close(d["dbias"].cpu(), conv.bias.grad, 2e-5, what + ": dbias")
 
 
+@WGRAD_SIDE
 @pytest.mark.parametrize("H,W", [(188, 624), (188, 621)])
-def test_conv5x5s2_c32_backward_exact(H, W):
+def test_conv5x5s2_c32_backward_exact(H, W, wgrad_side):
   """ConvC32 5x5 stride 2 (downsample[1]) from 188x624 and the odd 188x621.  On "ws" the data gradient is four polyphase 3x3
   convolutions + phase_merge; on "tc3" the same through the 3xTF32 kernels.  Integer x and dy, weights k/16: every product and
   sum is exact in fp32 and in both operand splits.  Reference: float64 autograd.  Bit-exact (forward, dx, dW, dbias)."""
@@ -554,21 +558,21 @@ def test_conv5x5s2_c32_backward_exact(H, W):
   y64 = F.conv2d(x64, w64, b64, stride=2, padding=2)
   y64.backward(dy.double())
   for backend in ("ws", "tc3"):
-    conv = torch.nn.Conv2d(32, 32, 5, stride=2, padding=2).to(DEV)
-    with torch.no_grad():
-      conv.weight.copy_(w); conv.bias.copy_(b)
-    xg = cl(x).requires_grad_()
 
     def run():
-      yg = Fn.ConvC32.apply(xg, conv.weight, conv.bias, conv, 5, 2)
+      conv = torch.nn.Conv2d(32, 32, 5, stride=2, padding=2).to(DEV)
+      with torch.no_grad():
+        conv.weight.copy_(w); conv.bias.copy_(b)
+      xg = cl(x).requires_grad_()
+      yg = Fn.conv_c32_autograd(xg, conv, 5, 2)
       yg.backward(cl(dy))
-      return yg
-    yg = with_backend(backend, run)
+      return yg.detach(), dict(dx=xg.grad, dW=conv.weight.grad, dbias=conv.bias.grad)
+    yg, d = layer_grads(wgrad_side, lambda: with_backend(backend, run))
     what = f"ConvC32 5x5s2 {backend} 1x{H}x{W}"
-    exact(uncl(yg.detach()), y64.detach(), what + ": forward")
-    exact(uncl(xg.grad), x64.grad, what + ": dx (polyphase dgrad + phase_merge)")
-    exact(conv.weight.grad, w64.grad, what + ": dW")
-    exact(conv.bias.grad, b64.grad, what + ": dbias (channel_sum)")
+    exact(uncl(yg), y64.detach(), what + ": forward")
+    exact(uncl(d["dx"]), x64.grad, what + ": dx (polyphase dgrad + phase_merge)")
+    exact(d["dW"], w64.grad, what + ": dW")
+    exact(d["dbias"], b64.grad, what + ": dbias (channel_sum)")
 
 
 def test_conv3d_out_softargmin_backward_kitti():
@@ -606,9 +610,10 @@ def kitti_refine_inputs():
   return coarse, rgb
 
 
+@WGRAD_SIDE
 @pytest.mark.parametrize("training", [True, False])
 @pytest.mark.parametrize("bn_bias", [60.0, -60.0])
-def test_refine_head_backward_kitti(kitti_refine_inputs, training, bn_bias):
+def test_refine_head_backward_kitti(kitti_refine_inputs, training, bn_bias, wgrad_side):
   """RefineHead (upsample + concat + conv 4 -> 32 + BN + LeakyReLU) at 47x156 -> 376x1248 with the BN shift at +-60, so every
   mask is unambiguous.  Reference: float64 CPU autograd.  Forward, dcoarse, dgamma, dbeta: bounds as
   test_gpu_backward.test_refine_head_backward_exact_side_of_kink.  dW: the disparity channel (~90 on average) meets a dz that
@@ -623,9 +628,9 @@ def test_refine_head_backward_kitti(kitti_refine_inputs, training, bn_bias):
     bn.bias.fill_(bn_bias)
     if not training:
       bn.running_var.fill_(400.0)
-  gconv, gbn = copy.deepcopy(conv).to(DEV), copy.deepcopy(bn).to(DEV)
+  gconv0, gbn0 = copy.deepcopy(conv), copy.deepcopy(bn)
   conv, bn = conv.double(), bn.double()
-  bn.train(training); gbn.train(training)
+  bn.train(training)
   coarse = coarse0.double().requires_grad_()
   up = F.interpolate(coarse.unsqueeze(1), size=(H, W), mode="bilinear", align_corners=False) * (W / w)
   inp = torch.cat([up, rgb.double()], 1)
@@ -635,15 +640,22 @@ def test_refine_head_backward_kitti(kitti_refine_inputs, training, bn_bias):
   gy, gu = rnd(B, 32, H, W, seed=3), rnd(B, H, W, seed=4)
   ((y * gy.double()).sum() + (up.squeeze(1) * gu.double()).sum()).backward()
   dw_abs = torch.nn.grad.conv2d_weight(inp.detach().abs(), conv.weight.shape, z.grad.abs(), padding=1)
-  cg = coarse0.to(DEV).requires_grad_()
-  upg, yg = Fn.refine_head_autograd(cg, rgb.to(DEV), gconv, gbn, training)
-  ((yg * cl(gy)).sum() + (upg * gu.to(DEV)).sum()).backward()
+
+  def run():
+    gconv, gbn = copy.deepcopy(gconv0).to(DEV), copy.deepcopy(gbn0).to(DEV)
+    gbn.train(training)
+    cg = coarse0.to(DEV).requires_grad_()
+    upg, yg = Fn.refine_head_autograd(cg, rgb.to(DEV), gconv, gbn, training)
+    ((yg * cl(gy)).sum() + (upg * gu.to(DEV)).sum()).backward()
+    return yg.detach(), dict(dcoarse=cg.grad, dW=gconv.weight.grad, dbias=gconv.bias.grad, dgamma=gbn.weight.grad,
+                             dbeta=gbn.bias.grad)
+  yg, d = layer_grads(wgrad_side, run)
   what = f"RefineHead 376x1248 shift={bn_bias} train={training}"
-  close(uncl(yg.detach()), y.detach(), 1e-5, what + ": forward")
-  close(cg.grad.cpu(), coarse.grad, 3e-5, what + ": dcoarse")
-  bounded(gconv.weight.grad, conv.weight.grad, 5e-5 * dw_abs, what + ": dW")
-  close(gbn.weight.grad.cpu(), bn.weight.grad, 3e-5, what + ": dgamma")
-  close(gbn.bias.grad.cpu(), bn.bias.grad, 3e-5, what + ": dbeta")
+  close(uncl(yg), y.detach(), 1e-5, what + ": forward")
+  close(d["dcoarse"].cpu(), coarse.grad, 3e-5, what + ": dcoarse")
+  bounded(d["dW"], conv.weight.grad, 5e-5 * dw_abs, what + ": dW")
+  close(d["dgamma"].cpu(), bn.weight.grad, 3e-5, what + ": dgamma")
+  close(d["dbeta"].cpu(), bn.bias.grad, 3e-5, what + ": dbeta")
 
 
 def test_refine_tail_backward_kitti():
