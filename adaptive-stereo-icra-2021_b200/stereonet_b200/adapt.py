@@ -98,28 +98,58 @@ class AdaptStepper:
         averaged in place and the fused clip + Adam kernel applies 1 / world — no per-parameter pack / unpack;
       * `dp_params` (+ `dp_group`) with a torch optimizer: pack -> all-reduce -> unpack (round-1 path);
       * `sync_grads`: a callable run between backward and the update (eager path only).
-    With use_graph=True the step is graph(fwd + loss + bwd + gather) -> eager all-reduce -> graph(clip + Adam)."""
+    The update after backward has three parts, run back to back in the eager step: before the collective, the collective, after
+    it.  With use_graph=True the step is graph(fwd + loss + bwd + before) -> eager collective -> graph(after)."""
+    update = self._split_update(dp_params, dp_group, dp_bucket, sync_grads)
     if self.use_graph and sync_grads is None:
-      return self._step_graph(left, right, dp_params, dp_group, replay, dp_bucket)
-    if dp_params is not None and sync_grads is None and dp_bucket is None:
-      from . import parallel
-      sync_grads = lambda: parallel.allreduce_gradients(dp_params, dp_group)
-    out = self._fwd_bwd(left, right, replay)
+      key = (tuple(left.shape), str(left.device), None if dp_params is None else len(dp_params), dp_bucket is not None,
+             None if replay is None else tuple(tuple(t.shape) for t in replay), self.batched_replay)
+      return self._step_graph(key, left, right, replay, update)
+    return self._step_eager(left, right, replay, update)
+
+  def _split_update(self, dp_params, dp_group, dp_bucket, sync_grads):
+    """The update after backward as (before, collective, after).  before() returns the tensor that collective(flat) reduces and
+    after(flat) finishes from; without a collective (None) before() is the whole update.  The graph step captures before() and
+    after() in one graph each and runs the collective eagerly between them: a captured NCCL collective hung a two-GPU run."""
+    if dp_bucket is None and sync_grads is not None:
+      return (lambda: None), (lambda flat: sync_grads()), (lambda flat: self._update())
+    if dp_bucket is None and dp_params is None:
+      return self._update, None, None
+    import torch.distributed as dist
+    from . import parallel
+    world = dist.get_world_size(dp_group)
+    collective = lambda flat: dist.all_reduce(flat, op=dist.ReduceOp.SUM, group=dp_group)
     if dp_bucket is not None:
-      self.optimizer.pack()
-      self._update(grad_scale=dp_bucket.allreduce(dp_group), packed=True)
-      return out
-    if sync_grads is not None:
-      sync_grads()
-    self._update()
+      def before():
+        self.optimizer.pack()
+        return dp_bucket.flat
+      return before, collective, lambda flat: self._update(grad_scale=dp_bucket.average(world), packed=True)
+
+    def after(flat):
+      parallel.unpack_gradients(dp_params, flat, world)
+      self._update()
+    return (lambda: parallel.pack_gradients(dp_params)), collective, after
+
+  def _step_eager(self, left, right, replay, update):
+    before, collective, after = update
+    out = self._fwd_bwd(left, right, replay)
+    flat = before()
+    if collective is not None:
+      collective(flat)
+      after(flat)
     return out
 
   def _fwd_bwd(self, left, right, replay):
-    s = self.stereo_net.input_scale
     self.feature_net.train(); self.stereo_net.train()
     self._refresh_weights()
-    if replay is not None and self.batched_replay:
-      return self._fwd_bwd_batched(left, right, replay)
+    loss, outputs = (self._loss_batched if replay is not None and self.batched_replay else self._loss)(left, right, replay)
+    fcs = feature_contrast_mean(outputs["cost_volume_l/{}".format(self.stereo_net.input_scale + self.stereo_net.k)]).mean()
+    self.optimizer.zero_grad()
+    loss.backward()
+    return loss.detach(), fcs, outputs
+
+  def _loss(self, left, right, replay):
+    s = self.stereo_net.input_scale
     from .autograd import fused
     if self.two_streams and left.is_cuda:
       if self._wstream is None:
@@ -146,10 +176,7 @@ class AdaptStepper:
         loss = loss + self.er_loss_weight * join_replay(self._replay_loss, replay)
     finally:
       fused.WGRAD_STREAM = None
-    fcs = feature_contrast_mean(outputs["cost_volume_l/{}".format(s + self.stereo_net.k)]).mean()
-    self.optimizer.zero_grad()
-    loss.backward()
-    return loss.detach(), fcs, outputs
+    return loss, outputs
 
   def _replay_loss(self, replay):
     self._feature_fork = "replay side"      # the replay pass runs on a side stream already: its right feature pass needs another
@@ -167,9 +194,9 @@ class AdaptStepper:
       self._wprep = fused.WeightPrepBatch([self.feature_net, self.stereo_net])
     self._wprep.refresh()
 
-  def _fwd_bwd_batched(self, left, right, replay):
+  def _loss_batched(self, left, right, replay):
     """Row f3: one batch-(n+m) pass for the n stream frames and the m replay samples; Monodepth loss on the first n
-    predictions, Khamis robust loss on the rest (snb_khamis_loss), same 1 : er_loss_weight mix as adapt.py:383-388."""
+    predictions (the outputs returned), Khamis robust loss on the rest (snb_khamis_loss), 1 : er_loss_weight as adapt.py:383-388."""
     s = self.stereo_net.input_scale
     n = left.shape[0]
     outputs = self.predict(torch.cat([left, replay[0]], 0), torch.cat([right, replay[1]], 0))
@@ -177,10 +204,7 @@ class AdaptStepper:
     head = {k: v[:n] for k, v in outputs.items()}
     loss = monodepth_single_loss(left, right, head, s)
     loss = loss + self.er_loss_weight * khamis_robust_loss(outputs[key][n:], replay[2])
-    fcs = feature_contrast_mean(head["cost_volume_l/{}".format(s + self.stereo_net.k)]).mean()
-    self.optimizer.zero_grad()
-    loss.backward()
-    return loss.detach(), fcs, head
+    return loss, head
 
   def _update(self, grad_scale=1.0, packed=False):
     if self.fused_opt:
@@ -201,15 +225,14 @@ class AdaptStepper:
         ts += [v for v in st.values() if isinstance(v, torch.Tensor)]
     return ts
 
-  def _capture(self, left, right, dp_params, dp_group, replay=None, dp_bucket=None):
-    import torch.distributed as dist
-    from . import ops, parallel
+  def _capture(self, left, right, replay, update):
+    from . import ops
     from .autograd import fused
+    before, collective, after = update
     self.feature_net.train(); self.stereo_net.train()
     dev = left.device
     sl, sr = left.clone(), right.clone()
     srep = None if replay is None else tuple(t.clone() for t in replay)        # static replay buffers (left, right, gt)
-    world = dist.get_world_size(dp_group) if (dp_params is not None or dp_bucket is not None) else 1
     fresh = (not self.fused_opt) and len(self.optimizer.state) == 0
     snap = [(t, t.detach().clone()) for t in self._state_tensors()]
     cur = torch.cuda.current_stream(dev)
@@ -219,14 +242,7 @@ class AdaptStepper:
       # One eager warm-up step allocates the lazily-created state (Adam moments and step counters, derived-weight
       # caches, allocator pools); model and optimizer state are restored afterwards so that capturing does not advance
       # the adaptation.
-      self._fwd_bwd(sl, sr, srep)
-      if dp_bucket is not None:
-        self.optimizer.pack()
-        self._update(grad_scale=dp_bucket.allreduce(dp_group), packed=True)
-      else:
-        if dp_params is not None:
-          parallel.allreduce_gradients(dp_params, dp_group)
-        self._update()
+      self._step_eager(sl, sr, srep, update)
       self.optimizer.zero_grad(set_to_none=True)
       with torch.no_grad():
         for t, saved in snap:                 # in place: the graphs will hold these addresses
@@ -240,40 +256,22 @@ class AdaptStepper:
     fused.bump_epoch()
     n0 = ops.LAUNCHES
     g1 = torch.cuda.CUDAGraph()
-    flat = None
     with torch.cuda.graph(g1):
       out = self._fwd_bwd(sl, sr, srep)
-      if dp_bucket is not None:
-        self.optimizer.pack()
-      elif dp_params is not None:
-        flat = parallel.pack_gradients(dp_params)
-      else:
-        self._update()
+      flat = before()
     g2 = None
-    if dp_bucket is not None:
+    if collective is not None:
       g2 = torch.cuda.CUDAGraph()
       with torch.cuda.graph(g2, pool=g1.pool()):
-        with torch.no_grad():
-          dp_bucket.stats.mul_(1.0 / world)
-        self._update(grad_scale=1.0 / world, packed=True)
-      flat = dp_bucket.flat
-    elif dp_params is not None:
-      g2 = torch.cuda.CUDAGraph()
-      with torch.cuda.graph(g2, pool=g1.pool()):
-        with torch.no_grad():
-          parallel.unpack_gradients(dp_params, flat, world)
-        self._update()
+        after(flat)
     self.launches_per_step = ops.LAUNCHES - n0          # library kernels inside one replay
     return dict(g1=g1, g2=g2, flat=flat, left=sl, right=sr, replay=srep, out=out)
 
-  def _step_graph(self, left, right, dp_params, dp_group, replay=None, dp_bucket=None):
-    import torch.distributed as dist
+  def _step_graph(self, key, left, right, replay, update):
     from .autograd import fused
-    key = (tuple(left.shape), str(left.device), None if dp_params is None else len(dp_params), dp_bucket is not None,
-           None if replay is None else tuple(tuple(t.shape) for t in replay), self.batched_replay)
     e = self._graphs.get(key)
     if e is None:
-      e = self._graphs[key] = self._capture(left, right, dp_params, dp_group, replay, dp_bucket)
+      e = self._graphs[key] = self._capture(left, right, replay, update)
     e["left"].copy_(left, non_blocking=True)
     e["right"].copy_(right, non_blocking=True)
     if replay is not None:
@@ -281,7 +279,7 @@ class AdaptStepper:
         dst.copy_(src, non_blocking=True)
     e["g1"].replay()
     if e["g2"] is not None:
-      dist.all_reduce(e["flat"], op=dist.ReduceOp.SUM, group=dp_group)      # eager, between the two graphs
+      update[1](e["flat"])                  # the collective, eager between the two graphs
       e["g2"].replay()
     fused.bump_epoch()                      # the replay rewrote the parameters behind torch's version counters
     return e["out"]

@@ -66,6 +66,11 @@ class DPBucket:
     (grad_scale = 1 / world).  Returns 1 / world."""
     world = dist.get_world_size(group)
     dist.all_reduce(self.flat, op=dist.ReduceOp.SUM, group=group)
+    return self.average(world)
+
+  def average(self, world):
+    """What follows the SUM all-reduce of `flat` over `world` replicas: the statistics are averaged in place.  Returns 1 / world,
+    the grad_scale of the optimizer step that averages the gradients."""
     self.stats.mul_(1.0 / world)
     return 1.0 / world
 
